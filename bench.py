@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the uplink OFDM receiver hot path on B200.
 
-    python bench.py --gpus N --steps K --warmup W [--impl ours|reference] [--config c2]
+    python bench.py --gpus N --steps K --warmup W [--impl ours|reference] [--config c2] [--dump-outputs DIR]
 
 Metric (BASELINE.json): LS+MRC antenna-samples/s.  One antenna-sample = one complex64 time
 sample from one antenna, cyclic prefix included (A*S*(N+C) per frame).  A "step" is one pass
@@ -50,7 +50,12 @@ def parse_args():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the c5 latency and other-config legs")
     ap.add_argument("--no-scaling-c4", action="store_true", help="skip the config-4 block that every rank runs")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (seeded sample of frames) as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return args
 
 
 # frames per step per GPU: large enough that one step's input exceeds the 126 MB L2 many times over
@@ -587,6 +592,24 @@ def ring_stream_leg(m, n_frames=768, feeder_threads=None, config="c3", lanes=3, 
         shutil.rmtree(d, ignore_errors=True)
 
 
+def dump_outputs(out_dir, comb, bits, budget=48 << 20):
+    """What the timed call hands its caller, for a fixed, seeded sample of the batch's frames (at most `budget`
+    bytes), so that two builds can be compared output for output on the same inputs.  float32 .npy files:
+    combined [n, S-1, K, 2] (re, im), bits [n, S-1, row bytes] (the packed bytes, values 0..255), and
+    frames [n] (float64), the sampled frame indices."""
+    import numpy as np
+    import torch
+
+    F = comb.shape[0]
+    n = max(1, min(F, budget // (4 * (comb[0].numel() + bits[0].numel()))))
+    idx = np.sort(np.random.default_rng(0).choice(F, size=n, replace=False))
+    sel = torch.from_numpy(idx).to(comb.device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "combined.npy"), comb.index_select(0, sel).cpu().numpy())
+    np.save(os.path.join(out_dir, "bits.npy"), bits.index_select(0, sel).cpu().numpy().astype(np.float32))
+    np.save(os.path.join(out_dir, "frames.npy"), idx.astype(np.float64))
+
+
 def workload_config(cfg, frames, e2e_frames):
     return {"workload": f"{cfg.name}: {cfg.fft_size}-pt FFT, CP {cfg.cp_len}, {cfg.n_ant} antennas, 1 pilot + "
                         f"{cfg.n_sym - 1} data symbols, {1 << cfg.qam_bits}-QAM",
@@ -675,6 +698,8 @@ def main():
     p_ms, d_ms = rcv.kernel_ms_history(min(args.steps, 256))
     rcv.set_timing(False)
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, comb, bits)
     t = torch.tensor([ms], device=dev, dtype=torch.float64)
     if dist is not None:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
