@@ -73,6 +73,8 @@ ABI = {
     "lsmrc_llr_from_combined": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p]),
     "lsmrc_zf_create": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, POINTER(c_int)]),
     "lsmrc_zf_apply": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
+    "lsmrc_demod_frames_device_mu": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_float, c_void_p, c_void_p, c_void_p,
+                                             POINTER(c_int)]),
     "lsmrc_ring_copy_query": (c_int, [c_void_p, c_int]),
     "lsmrc_ring_submit_frames": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_int]),
     "lsmrc_set_timing": (c_int, [c_void_p, c_int]),
@@ -211,6 +213,19 @@ class LsMrcReceiver:
         bad = c_int()
         self._ck(self.lib.lsmrc_zf_create(self.h, _ptr(d_x), n_ant, n_sc, n_users, _ptr(d_hzf), byref(bad)))
         return bad.value
+
+    DETECTORS = {"zf": 0, "mmse": 1}
+
+    def demod_frames_device_mu(self, d_rx, n_frames, n_users, d_combined, d_bits=None, d_hconj=None, detector="zf",
+                               noise_var=0.0, count_singular=False):
+        """Multi-user frames (symbols 0..U-1 per-user pilots, U..S-1 data of all users): per-user LS channel and ZF or
+        MMSE detection.  d_combined [F,S-U,U,K], d_bits [F,S-U,U,row], d_hconj [F,U,A,K].  With count_singular the call
+        is synchronous and returns the number of (frame, subcarrier) pairs whose Gram matrix was singular."""
+        bad = c_int(0)
+        self._ck(self.lib.lsmrc_demod_frames_device_mu(self.h, _ptr(d_rx), n_frames, n_users, self.DETECTORS.get(detector, -1),
+                                                       float(noise_var), _ptr(d_hconj), _ptr(d_combined), _ptr(d_bits),
+                                                       byref(bad) if count_singular else None))
+        return bad.value if count_singular else None
 
     def zf_apply(self, d_hzf, d_xd, n_ant, n_sc, n_users, d_hx):
         self._ck(self.lib.lsmrc_zf_apply(self.h, _ptr(d_hzf), _ptr(d_xd), n_ant, n_sc, n_users, _ptr(d_hx)))

@@ -36,6 +36,10 @@ struct PlanOps {
     cudaError_t (*launch)(int mode, const KernelParams&, cudaStream_t, int max_data_ctas, unsigned* grid_out, long long* items_out);
     // shuffle-stage plans: pilot and data items of whole frames in ONE persistent launch (lsmrc_frames_sh); nullptr otherwise
     cudaError_t (*launch_fused)(const KernelParams&, cudaStream_t, int max_data_ctas);
+    // multi-user detection: users per pass of the data kernel, and the launch of the weight layout + data kernel
+    int mu_ug;
+    cudaError_t (*mu_prepare)(int* ctas_per_sm);
+    cudaError_t (*mu_launch)(const KernelParams&, const float2* hzf, float2* wd, int n_users, int max_ctas, int n_sms, cudaStream_t);
 };
 
 // The one-launch kernel (MODE_ONESHOT) of a plan.  Small FFT sizes have a dedicated latency plan:
@@ -358,6 +362,44 @@ PilotOps make_pilot_ops()
     return o;
 }
 
+// Multi-user data kernel (lsmrc_mu_data): users per pass.  Each thread keeps UG * P complex sums in registers next to the
+// FFT working set: the most that compiles without spills (-Xptxas -v) -- two users for the 32-point plans of 1024 and
+// 4096 points (128 registers of sums), one for 512 and 2048 (two spill there), four at 16 points, eight at 8.  Larger
+// U re-runs the row transforms once per group of UG users (DESIGN.md 8e).
+template <class PL>
+constexpr int mu_ug() { return PL::P >= 32 ? ((PL::N == 512 || PL::N == 2048) ? 1 : 2) : (PL::P >= 16 ? 4 : 8); }
+
+template <class PL>
+constexpr size_t mu_smem() { return sizeof(float2) * (size_t)(PL::TWN + PL::TEAMS * PL::TEAM_STRIDE); }
+
+template <class PL>
+cudaError_t mu_prepare_impl(int* ctas_per_sm)
+{
+    constexpr int UG = mu_ug<PL>();
+    cudaError_t e = cudaFuncSetAttribute(lsmrc_mu_data<PL, UG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mu_smem<PL>());
+    if (e != cudaSuccess) return e;
+    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas_per_sm, lsmrc_mu_data<PL, UG>, PL::THREADS, mu_smem<PL>());
+}
+
+// max_ctas: resident CTAs of lsmrc_mu_data on the whole GPU (mu_prepare_impl x SMs)
+template <class PL>
+cudaError_t mu_launch_impl(const KernelParams& p, const float2* hzf, float2* wd, int n_users, int max_ctas, int n_sms, cudaStream_t st)
+{
+    constexpr int UG = mu_ug<PL>();
+    const int groups = (n_users + UG - 1) / UG;
+    cudaError_t e;
+    const long long rows = (long long)p.n_frames * groups * UG * p.n_ant;
+    long long wblocks = (rows * PL::N + 255) / 256;
+    if (wblocks > (long long)n_sms * 16) wblocks = (long long)n_sms * 16;
+    k_mu_weights<PL><<<(unsigned)wblocks, 256, 0, st>>>(hzf, wd, p.n_ant, n_users, groups * UG, rows);
+    if ((e = cudaGetLastError()) != cudaSuccess) return e;
+    const long long items = (long long)p.n_frames * groups * p.n_sym_work;
+    long long grid = (items + PL::TEAMS - 1) / PL::TEAMS;
+    if (grid > max_ctas) grid = max_ctas;
+    lsmrc_mu_data<PL, UG><<<(unsigned)grid, PL::THREADS, mu_smem<PL>(), st>>>(p, wd, n_users, groups);
+    return cudaGetLastError();
+}
+
 template <class PL, int MINB>
 PlanOps make_ops()
 {
@@ -375,6 +417,9 @@ PlanOps make_ops()
     o.prepare = &prepare_impl<PL, MINB>;
     o.launch = &launch_impl<PL, MINB>;
     o.launch_fused = PL::SH > 1 ? &launch_fused_impl<PL, MINB> : nullptr;
+    o.mu_ug = mu_ug<PL>();
+    o.mu_prepare = &mu_prepare_impl<PL>;
+    o.mu_launch = &mu_launch_impl<PL>;
     return o;
 }
 
@@ -559,6 +604,14 @@ struct lsmrc_ctx {
     unsigned long long* d_hit = nullptr;  // frame-sync first-hit key
     float* d_noise_part = nullptr;        // [frames][S-1] row partials of the noise estimator
     size_t noise_part_rows = 0;
+    // multi-user path (lsmrc_demod_frames_device_mu): its own channel state and scratch, grown on demand
+    ChanState mu_ch;
+    float2* d_mu_hconj = nullptr;  // [U][F][A][K] conj(H) per user, as the pilot kernel writes it
+    float2* d_mu_hzf = nullptr;    // [F][K][U][A] conj(W)
+    float2* d_mu_wd = nullptr;     // [F][UP][A][N] W in the data kernel's slot layout
+    size_t mu_hconj_cap = 0, mu_hzf_cap = 0, mu_wd_cap = 0;  // bytes
+    int* d_mu_count = nullptr;     // singular (frame, subcarrier) pairs
+    int mu_max_ctas = 0;           // resident CTAs of the multi-user data kernel (0: not prepared yet)
     float* soft_llr = nullptr;            // set for the duration of a *_soft call
     float soft_inv_noise = 1.f;
     bool timing = false;
@@ -993,6 +1046,57 @@ int stage_symbol(lsmrc_ctx* h, const void* rx_sym, int on_device, const float2**
 
 }  // namespace
 
+namespace {
+
+// subcarriers per CTA of k_zf_create: kZfKT where its tile fits shared memory, else the largest power of two below that
+// does (0: not even one subcarrier fits)
+size_t zf_smem(int kt, int n_ant, int n_users)
+{
+    return sizeof(float2) * ((size_t)kt * n_ant * n_users + (size_t)kt * n_users * 2 * n_users);
+}
+
+int zf_tile(const lsmrc_ctx* h, int n_ant, int n_users)
+{
+    int kt = kZfKT;
+    while (kt >= 1 && zf_smem(kt, n_ant, n_users) + 1024 > h->smem_optin) kt /= 2;
+    return kt;
+}
+
+// The dynamic shared-memory limit of k_zf_create is a per-device, per-process attribute: lsmrc_create raises it once to the
+// largest tile zf_tile can pick (smem_optin - 1024), the same value for every handle, so no handle lowers it under
+// another and no call sets it (calls stay capturable).  Frames go on gridDim.y in chunks of at most 65535.
+int launch_zf_create(lsmrc_ctx* h, cudaStream_t st, const float2* x, float2* hzf, int n_ant, int n_sc, int n_users, int kt, float lambda,
+                     int n_frames, long long x_frame_stride, long long x_user_stride, long long hzf_frame_stride, int* d_count)
+{
+    const size_t smem = zf_smem(kt, n_ant, n_users);
+    constexpr int kMaxGridY = 65535;
+    for (int f0 = 0; f0 < n_frames; f0 += kMaxGridY) {
+        const int nf = n_frames - f0 < kMaxGridY ? n_frames - f0 : kMaxGridY;
+        const dim3 grid((unsigned)((n_sc + kt - 1) / kt), (unsigned)nf);
+        k_zf_create<<<grid, 128, smem, st>>>(x + f0 * x_frame_stride, hzf + f0 * hzf_frame_stride, n_ant, n_sc, n_users, kt, lambda,
+                                             x_frame_stride, x_user_stride, hzf_frame_stride, d_count);
+        h->launches++;
+        CK(h, cudaGetLastError());
+    }
+    return LSMRC_OK;
+}
+
+// device scratch that only grows (a call after one of the same size allocates nothing: CUDA-graph capturable)
+template <class T>
+int ensure_scratch(lsmrc_ctx* h, T*& ptr, size_t& cap, size_t bytes, cudaStream_t quiesce)
+{
+    if (cap >= bytes) return LSMRC_OK;
+    CK(h, cudaStreamSynchronize(quiesce));
+    cudaFree(ptr);
+    ptr = nullptr;
+    cap = 0;
+    CK(h, cudaMalloc(&ptr, bytes));
+    cap = bytes;
+    return LSMRC_OK;
+}
+
+}  // namespace
+
 extern "C" {
 
 int lsmrc_abi_version(void) { return LSMRC_ABI_VERSION; }
@@ -1138,6 +1242,11 @@ int lsmrc_create(const lsmrc_config* cfg, lsmrc_handle* out)
         if ((e = cudaMemcpy(h->d_one_tw, tw1.data(), tw1.size() * sizeof(float2), cudaMemcpyHostToDevice)) != cudaSuccess) { fail_cuda(h, e, "cudaMemcpy twiddles"); return bail(LSMRC_ERR_CUDA); }
     }
     if ((e = cudaMalloc(&h->d_pilot_bin, (size_t)h->K * sizeof(float2))) != cudaSuccess) { fail_cuda(h, e, "cudaMalloc pilot"); return bail(LSMRC_ERR_CUDA); }
+    // zero forcing: allow the largest tile once (see launch_zf_create)
+    if ((e = cudaFuncSetAttribute(k_zf_create, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(h->smem_optin - 1024))) != cudaSuccess) {
+        fail_cuda(h, e, "cudaFuncSetAttribute (zero forcing)");
+        return bail(LSMRC_ERR_CUDA);
+    }
     // the table uploads above are pageable-memory copies on the legacy stream (they return once staged); the kernels
     // run on non-blocking streams that do not order against it
     if ((e = cudaDeviceSynchronize()) != cudaSuccess) { fail_cuda(h, e, "cudaDeviceSynchronize"); return bail(LSMRC_ERR_CUDA); }
@@ -1159,6 +1268,11 @@ int lsmrc_destroy(lsmrc_handle h)
     cudaFree(h->d_pilot_bin);
     free_chan(h->dev_ch);
     free_chan(h->one_ch);
+    free_chan(h->mu_ch);
+    cudaFree(h->d_mu_hconj);
+    cudaFree(h->d_mu_hzf);
+    cudaFree(h->d_mu_wd);
+    cudaFree(h->d_mu_count);
     cudaFree(h->d_sym);
     cudaFree(h->d_one_hconj);
     cudaFree(h->d_one_comb);
@@ -1233,6 +1347,74 @@ int lsmrc_demod_frames_device(lsmrc_handle h, const void* d_rx, int n_frames, vo
     return launch_frames(h, compute_stream(h), static_cast<const float2*>(d_rx), n_frames, h->dev_ch,
                          static_cast<float2*>(d_hconj), static_cast<float*>(d_hsqrd), static_cast<float2*>(d_combined),
                          static_cast<uint8_t*>(d_bits), h->timing);
+}
+
+int lsmrc_demod_frames_device_mu(lsmrc_handle h, const void* d_rx, int n_frames, int n_users, int detector, float noise_var,
+                                 void* d_hconj, void* d_combined, void* d_bits, int* n_singular)
+{
+    if (!h || !d_rx || !d_combined) return fail(h, LSMRC_ERR_INVALID, "null argument");
+    if (n_frames < 0) return fail(h, LSMRC_ERR_INVALID, "n_frames < 0");
+    const int A = h->cfg.n_ant, S = h->cfg.n_sym, N = h->cfg.fft_size, K = h->K;
+    if (n_users < 1 || n_users > kZfMaxUsers || n_users > A || n_users >= S)
+        return fail(h, LSMRC_ERR_INVALID, "need 1 <= n_users <= 16, n_users <= n_ant and n_users < n_sym");
+    if (detector != LSMRC_DETECT_ZF && detector != LSMRC_DETECT_MMSE) return fail(h, LSMRC_ERR_INVALID, "unknown detector");
+    if (detector == LSMRC_DETECT_MMSE && !(std::isfinite(noise_var) && noise_var > 0.f))
+        return fail(h, LSMRC_ERR_INVALID, "MMSE needs a finite noise_var > 0");
+    if (!h->have_pilot) return fail(h, LSMRC_ERR_NO_PILOT, "set the pilot first");
+    if (n_frames == 0) {
+        if (n_singular) *n_singular = 0;
+        return LSMRC_OK;
+    }
+    const int kt = zf_tile(h, A, n_users);
+    if (kt < 1) return fail(h, LSMRC_ERR_UNSUPPORTED, "n_ant * n_users too large for one CTA's shared memory");
+    CK(h, cudaSetDevice(h->cfg.device));
+    cudaStream_t st = compute_stream(h);
+    const int U = n_users, UP = (U + h->ops->mu_ug - 1) / h->ops->mu_ug * h->ops->mu_ug;
+    const long long F = n_frames;
+    int rc;
+    if ((rc = ensure_chan(h, h->mu_ch, n_frames, st)) != LSMRC_OK) return rc;
+    if ((rc = ensure_scratch(h, h->d_mu_hconj, h->mu_hconj_cap, sizeof(float2) * (size_t)(U * F * A * K), st)) != LSMRC_OK) return rc;
+    if ((rc = ensure_scratch(h, h->d_mu_hzf, h->mu_hzf_cap, sizeof(float2) * (size_t)(F * K * U * A), st)) != LSMRC_OK) return rc;
+    if ((rc = ensure_scratch(h, h->d_mu_wd, h->mu_wd_cap, sizeof(float2) * (size_t)(F * UP * A * N), st)) != LSMRC_OK) return rc;
+    if (!h->d_mu_count) CK(h, cudaMalloc(&h->d_mu_count, sizeof(int)));
+    if (h->mu_max_ctas == 0) {
+        int per_sm = 0;
+        CK(h, h->ops->mu_prepare(&per_sm));
+        if (per_sm < 1) return fail(h, LSMRC_ERR_CUDA, "multi-user data kernel does not fit on an SM");
+        h->mu_max_ctas = per_sm * h->n_sms;
+    }
+    // 1. LS channel of every user from its own pilot symbol: the single-user pilot launch, once per pilot symbol
+    KernelParams p = base_params(h);
+    p.n_frames = n_frames;
+    const long long user_elems = F * A * K;
+    for (int u = 0; u < U; ++u) {
+        p.rx = static_cast<const float2*>(d_rx) + (long long)u * p.sym_stride;
+        if ((rc = launch_pilot(h, st, p, h->mu_ch, h->d_mu_hconj + u * user_elems, nullptr)) != LSMRC_OK) return rc;
+    }
+    // 2. detector per (frame, subcarrier): X = conj(H) [U][A][K] of the frame -> Hzf = conj(W)
+    if (n_singular) CK(h, cudaMemsetAsync(h->d_mu_count, 0, sizeof(int), st));
+    if ((rc = launch_zf_create(h, st, h->d_mu_hconj, h->d_mu_hzf, A, K, U, kt, detector == LSMRC_DETECT_MMSE ? noise_var : 0.f, n_frames,
+                               (long long)A * K, user_elems, (long long)K * U * A, n_singular ? h->d_mu_count : nullptr)) != LSMRC_OK)
+        return rc;
+    // 3. detection fused with the row FFT of every data symbol
+    p.rx = static_cast<const float2*>(d_rx);
+    p.first_sym = U;
+    p.n_sym_work = S - U;
+    p.combined = static_cast<float2*>(d_combined);
+    p.bits = static_cast<uint8_t*>(d_bits);
+    CK(h, h->ops->mu_launch(p, h->d_mu_hzf, h->d_mu_wd, U, h->mu_max_ctas, h->n_sms, st));
+    h->launches += 2;
+    if (d_hconj) {  // [U][F][A][K] -> [F][U][A][K]
+        const size_t row = sizeof(float2) * (size_t)A * K;
+        for (int u = 0; u < U; ++u)
+            CK(h, cudaMemcpy2DAsync(static_cast<float2*>(d_hconj) + (size_t)u * A * K, row * U, h->d_mu_hconj + u * user_elems, row, row,
+                                    (size_t)n_frames, cudaMemcpyDeviceToDevice, st));
+    }
+    if (n_singular) {
+        CK(h, cudaMemcpyAsync(n_singular, h->d_mu_count, sizeof(int), cudaMemcpyDeviceToHost, st));
+        CK(h, cudaStreamSynchronize(st));
+    }
+    return LSMRC_OK;
 }
 
 int lsmrc_demod_frames_device_soft(lsmrc_handle h, const void* d_rx, int n_frames, void* d_combined, void* d_bits,
@@ -1313,18 +1495,18 @@ int lsmrc_zf_create(lsmrc_handle h, const void* d_x, int n_ant, int n_sc, int n_
     if (!h || !d_x || !d_hzf) return fail(h, LSMRC_ERR_INVALID, "null argument");
     if (n_ant < 1 || n_sc < 1 || n_users < 1 || n_users > kZfMaxUsers) return fail(h, LSMRC_ERR_INVALID, "need n_ant, n_sc >= 1 and 1 <= n_users <= 16");
     if (n_users > n_ant) return fail(h, LSMRC_ERR_INVALID, "more users than antennas: X X^H would be singular");
-    const size_t smem = sizeof(float2) * ((size_t)kZfKT * n_ant * n_users + (size_t)kZfKT * n_users * 2 * n_users);
-    if (smem + 1024 > h->smem_optin) return fail(h, LSMRC_ERR_UNSUPPORTED, "n_ant * n_users too large for one CTA's shared memory");
+    const int kt = zf_tile(h, n_ant, n_users);
+    if (kt < 1) return fail(h, LSMRC_ERR_UNSUPPORTED, "n_ant * n_users too large for one CTA's shared memory");
     CK(h, cudaSetDevice(h->cfg.device));
     cudaStream_t st = compute_stream(h);
     if (!h->d_hit) CK(h, cudaMalloc(&h->d_hit, sizeof(unsigned long long)));
     int* d_count = reinterpret_cast<int*>(h->d_hit);
     CK(h, cudaMemsetAsync(d_count, 0, sizeof(int), st));
-    if (smem + 1024 > (48u << 10)) CK(h, cudaFuncSetAttribute(k_zf_create, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    k_zf_create<<<(unsigned)((n_sc + kZfKT - 1) / kZfKT), 128, smem, st>>>(static_cast<const float2*>(d_x), static_cast<float2*>(d_hzf), n_ant,
-                                                                              n_sc, n_users, d_count);
-    h->launches++;
-    CK(h, cudaGetLastError());
+    {
+        const int rc = launch_zf_create(h, st, static_cast<const float2*>(d_x), static_cast<float2*>(d_hzf), n_ant, n_sc, n_users, kt, 0.f, 1,
+                                        0, (long long)n_ant * n_sc, 0, d_count);
+        if (rc != LSMRC_OK) return rc;
+    }
     if (n_singular) {
         CK(h, cudaMemcpyAsync(n_singular, d_count, sizeof(int), cudaMemcpyDeviceToHost, st));
         CK(h, cudaStreamSynchronize(st));

@@ -2160,30 +2160,38 @@ __global__ void k_llr_rows(const float2* __restrict__ combined, const float* __r
 
 // ---- multi-user zero forcing (SURVEY 8f rank 4; cpuLS.hpp:400-463, uncalled in the reference) ---------------
 // createZeroForcingMatrix: per subcarrier k, with Xk = X[:, :, k] (U users x A antennas),
-//   Hk = Xk^H * inv(Xk * Xk^H)   (A x U, column-major, ld = A)  ->  Hzf[k][u][a].
-// A CTA takes KT consecutive subcarriers so that the gather from X [U][A][K] reads KT contiguous samples per
-// (user, antenna); Gram matrix, inverse (Gauss-Jordan with partial pivoting, one thread per subcarrier -- U is a
-// handful) and the A x U product all run out of shared memory.  Singular subcarriers (a pivot below 1e-6 of the
-// largest Gram entry) yield a zero block and are counted in *n_singular.
+//   Hk = Xk^H * inv(Xk * Xk^H + lambda*I)   (A x U, column-major, ld = A)  ->  Hzf[k][u][a].
+// A CTA takes KT (<= kZfKT, chosen by the launcher so that the tile fits shared memory) consecutive subcarriers so that
+// the gather from X [U][A][K] reads KT contiguous samples per (user, antenna); Gram matrix, inverse (Gauss-Jordan with
+// partial pivoting, one thread per subcarrier -- U is a handful) and the A x U product all run out of shared memory.
+// Singular subcarriers (a pivot below 1e-6 of the largest Gram entry) yield a zero block and are counted in *n_singular.
+// blockIdx.y is the frame: X and Hzf of frame f start at f * x_frame_stride / f * hzf_frame_stride; user u's rows of X
+// at u * x_user_stride.  Per subcarrier the result depends on neither KT nor the frame batch.
+// With X = conj(H) (H the A x U channel of subcarrier k), Hzf[k][u][a] = conj(W_k[u][a]) for the linear detector
+// W_k = inv(H^H H + lambda*I) H^H: ZF at lambda = 0, MMSE at lambda = noise variance (DESIGN.md 8e).
 constexpr int kZfKT = 8;
 constexpr int kZfMaxUsers = 16;
 
-__global__ void k_zf_create(const float2* __restrict__ X, float2* __restrict__ Hzf, int A, int K, int U, int* n_singular)
+__global__ void k_zf_create(const float2* __restrict__ X, float2* __restrict__ Hzf, int A, int K, int U, int KT, float lambda,
+                            long long x_frame_stride, long long x_user_stride, long long hzf_frame_stride, int* n_singular)
 {
     extern __shared__ __align__(16) float2 zsm[];
-    float2* s_x = zsm;                          // [KT][A][U]  (users x antennas, column-major per subcarrier)
-    float2* s_g = s_x + (size_t)kZfKT * A * U;  // [KT][U][2U] augmented rows for the inverse
+    float2* s_x = zsm;                      // [KT][A][U]  (users x antennas, column-major per subcarrier)
+    float2* s_g = s_x + (size_t)KT * A * U;  // [KT][U][2U] augmented rows for the inverse
     __shared__ int s_ok[kZfKT];
-    const int k0 = blockIdx.x * kZfKT;
-    const int nk = min(kZfKT, K - k0);
-    for (int idx = threadIdx.x; idx < U * A * kZfKT; idx += blockDim.x) {
-        const int kt = idx % kZfKT, ua = idx / kZfKT;  // ua = u*A + a, kt fastest: contiguous in X
+    X += (long long)blockIdx.y * x_frame_stride;
+    Hzf += (long long)blockIdx.y * hzf_frame_stride;
+    const int k0 = blockIdx.x * KT;
+    const int nk = min(KT, K - k0);
+    for (int idx = threadIdx.x; idx < U * A * KT; idx += blockDim.x) {
+        const int kt = idx % KT, ua = idx / KT;  // ua = u*A + a, kt fastest: contiguous in X
         const int u = ua / A, a = ua - u * A;
-        s_x[((size_t)kt * A + a) * U + u] = (kt < nk) ? X[(size_t)ua * K + k0 + kt] : make_float2(0.f, 0.f);
+        s_x[((size_t)kt * A + a) * U + u] = (kt < nk) ? X[(long long)u * x_user_stride + (long long)a * K + k0 + kt] : make_float2(0.f, 0.f);
     }
     __syncthreads();
-    // Gram matrix G[u][v] = sum_a x[u,a] * conj(x[v,a]) into the left half of the augmented rows, identity right
-    for (int idx = threadIdx.x; idx < kZfKT * U * U; idx += blockDim.x) {
+    // Gram matrix G[u][v] = sum_a x[u,a] * conj(x[v,a]) (+ lambda on the diagonal) into the left half of the augmented
+    // rows, identity right
+    for (int idx = threadIdx.x; idx < KT * U * U; idx += blockDim.x) {
         const int kt = idx / (U * U), r = idx % (U * U), u = r / U, v = r % U;
         const float2* xk = s_x + (size_t)kt * A * U;
         float2 acc = make_float2(0.f, 0.f);
@@ -2192,12 +2200,13 @@ __global__ void k_zf_create(const float2* __restrict__ X, float2* __restrict__ H
             acc.x += p.x * q.x + p.y * q.y;
             acc.y += p.y * q.x - p.x * q.y;
         }
+        if (u == v) acc.x += lambda;  // (a diagonal sum is >= +0: adding lambda = 0 leaves it bit for bit)
         float2* row = s_g + ((size_t)kt * U + u) * 2 * U;
         row[v] = acc;
         row[U + v] = make_float2(u == v ? 1.f : 0.f, 0.f);
     }
     __syncthreads();
-    if (threadIdx.x < kZfKT) {
+    if (threadIdx.x < KT) {
         const int kt = threadIdx.x;
         float2* w = s_g + (size_t)kt * U * 2 * U;
         bool ok = kt < nk;
@@ -2248,7 +2257,7 @@ __global__ void k_zf_create(const float2* __restrict__ X, float2* __restrict__ H
     }
     __syncthreads();
     // Hk[a][u] = sum_v conj(x[v,a]) * Ginv[v][u]; a fastest so the store is coalesced
-    for (int idx = threadIdx.x; idx < kZfKT * U * A; idx += blockDim.x) {
+    for (int idx = threadIdx.x; idx < KT * U * A; idx += blockDim.x) {
         const int kt = idx / (U * A), r = idx % (U * A), u = r / A, a = r % A;
         if (kt >= nk) continue;
         const float2* xk = s_x + (size_t)kt * A * U;
@@ -2278,6 +2287,127 @@ __global__ void k_zf_apply(const float2* __restrict__ Hzf, const float2* __restr
             acc.y += h.x * x.y + h.y * x.x;
         }
         HX[(size_t)a * K + k] = acc;
+    }
+}
+
+// ---- multi-user detection (DESIGN.md 8e) ----------------------------------------------------------------------
+// Frame [S][A][N+C] with U users: symbol u < U is user u's pilot (the others silent), symbols U..S-1 carry all users.
+// Per-user conj(H) comes from the pilot kernel run once per pilot symbol, the detector W_k (U x A per subcarrier) from
+// k_zf_create as conj(Hzf).  The data kernel never stores the FFT output: per (frame, data symbol, group of UG users) a
+// team transforms each antenna row and accumulates x^[u][k] += Wd[u][a][slot] * y'[slot] in registers.
+
+// Wd [F][UP][A][N]: W_k[u][a] in the plan's slot layout (Plan::hpos), times conj of the slot's unit factor (the sink
+// of row_fft sees y' = u * Y on the shuffle-stage plans, so Wd * y' = W * Y).  Users U..UP-1 (padding of the last
+// group) and bin 0 are zero.  Hzf [F][K][U][A] = conj(W).
+template <class PL>
+__global__ void k_mu_weights(const float2* __restrict__ hzf, float2* __restrict__ wd, int A, int U, int UP, long long rows)
+{
+    constexpr int N = PL::N, T = PL::T, K = N - 1;
+    const long long n = rows * N;
+    for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < n; idx += (long long)gridDim.x * blockDim.x) {
+        const int pos = (int)(idx % N);
+        const long long row = idx / N;  // (f * UP + u) * A + a
+        const int a = (int)(row % A);
+        const int u = (int)((row / A) % UP);
+        const long long f = row / ((long long)A * UP);
+        const int sl = pos / T, t = pos % T;
+        const int bin = (PL::SH == 1) ? pos : PL::bin_of(sl, t);
+        float2 w = make_float2(0.f, 0.f);
+        if (bin > 0 && u < U) {
+            const float2 c = hzf[((f * K + (bin - 1)) * U + u) * A + a];
+            w = make_float2(c.x, -c.y);
+            if constexpr (PL::SH > 1) w = PL::unfix(sl, t, w);
+        }
+        wd[idx] = w;
+    }
+}
+
+// Teams take items (frame f, user group g, data symbol s), consecutive items sharing (f, g) so that the teams working
+// at the same time read the same detector rows (L1/L2).  Outputs: combined [F][S-U][U][K] ascending frequency, bits
+// [F][S-U][U][row].  p.first_sym = U, p.n_sym_work = S-U; n_users = U, UP = groups * UG.
+template <class PL, int UG>
+__global__ void __launch_bounds__(PL::THREADS, 1) lsmrc_mu_data(const KernelParams p, const float2* __restrict__ wd, int n_users, int n_groups)
+{
+    constexpr int N = PL::N, P = PL::P, T = PL::T, K = N - 1;
+    extern __shared__ __align__(16) float2 smem[];
+    float2* s_tw1 = smem;
+    float2* s_tw2 = smem + PL::TW1;
+    float2* s_tiles = smem + PL::TWN;
+    const int team = threadIdx.x / T;
+    const int t = threadIdx.x % T;
+    float2* my_tiles = s_tiles + team * PL::TEAM_STRIDE;
+    for (int i = threadIdx.x; i < PL::TWN; i += PL::THREADS) smem[i] = p.twiddles[i];
+    __syncthreads();
+
+    const int U = n_users, UP = n_groups * UG, D = p.n_sym_work;
+    const long long n_items = (long long)p.n_frames * n_groups * D;
+    const long long n_rounds = (n_items + (long long)gridDim.x * PL::TEAMS - 1) / ((long long)gridDim.x * PL::TEAMS);
+    for (long long r = 0; r < n_rounds; ++r) {  // every team runs the same number of rounds: team_sync stays uniform
+        const long long raw = (r * gridDim.x + blockIdx.x) * PL::TEAMS + team;
+        const bool ok = raw < n_items;
+        const long long item = ok ? raw : n_items - 1;
+        const int s = (int)(item % D);
+        const long long fg = item / D;
+        const int g = (int)(fg % n_groups);
+        const long long f = fg / n_groups;
+        const float2* x0 = p.rx + f * p.frame_stride + (long long)(p.first_sym + s) * p.sym_stride + p.cp;
+        const float2* w0 = wd + (f * UP + (long long)g * UG) * p.n_ant * N;
+        const long long wstride = (long long)p.n_ant * N;  // between users
+        float2 acc[UG][P];
+#pragma unroll
+        for (int j = 0; j < UG; ++j)
+#pragma unroll
+            for (int sl = 0; sl < P; ++sl) acc[j][sl] = make_float2(0.f, 0.f);
+        for (int a = 0; a < p.n_ant; ++a) {
+            float2 v[P];
+            row_load<PL>(v, x0 + (long long)a * p.ant_stride, t);
+            float2* tile = my_tiles + (PL::NBUF == 2 ? (a & 1) * PL::TILE : 0);
+            const float2* wa = w0 + (long long)a * N;
+            row_fft<PL>(v, nullptr, tile, s_tw1, s_tw2, t, team, [&](int sl, int bin, float2 y) {
+                const int hp = PL::hpos(sl, t, bin);
+#pragma unroll
+                for (int j = 0; j < UG; ++j) acc[j][sl] = cmac(acc[j][sl], y, __ldg(wa + j * wstride + hp));
+            });
+        }
+        // epilogue per user: ascending-frequency store, hard demap into the team's tile (bytes), bit packing
+        uint8_t* s_idx = reinterpret_cast<uint8_t*>(my_tiles);
+        const int b = p.qam_bits;
+#pragma unroll
+        for (int j = 0; j < UG; ++j) {
+            // padding users of the last group: teams of whole warps skip them; narrower teams share a warp's __syncwarp
+            // with teams of other groups, so they run the epilogue without storing and every lane passes the same barriers
+            const int u = g * UG + j;
+            if constexpr (PL::T >= 32) {
+                if (u >= U) break;
+            }
+            const bool store = ok && u < U;
+            const long long orow = (f * D + s) * U + (u < U ? u : U - 1);
+            float2* out_row = p.combined + orow * K;
+            team_sync<PL>(team);  // the tile (last row's exchange buffer, or the previous user's bytes) is free
+#pragma unroll
+            for (int sl = 0; sl < P; ++sl) {
+                const int bin = PL::bin_of(sl, t);
+                if (bin > 0) {
+                    const int pos = (bin < N / 2) ? (bin - 1 + N / 2) : (bin - N / 2);
+                    if (store) out_row[pos] = acc[j][sl];
+                    s_idx[pos] = (uint8_t)demap_symbol(acc[j][sl].x, acc[j][sl].y, b);
+                }
+            }
+            if (p.bits != nullptr) {
+                team_sync<PL>(team);
+                uint8_t* bits_row = p.bits + orow * p.bits_row_bytes;
+                for (int byte = t; byte < p.bits_row_bytes; byte += T) {
+                    unsigned v8 = 0;
+                    for (int q = 0; q < 8; ++q) {
+                        const int pos = byte * 8 + q;
+                        const int sym = pos / b, bit = pos - sym * b;
+                        if (sym < K) v8 |= ((s_idx[sym] >> bit) & 1u) << q;
+                    }
+                    if (store) bits_row[byte] = (uint8_t)v8;
+                }
+            }
+        }
+        team_sync<PL>(team);  // the bytes alias the tile the next item's first row is exchanged through
     }
 }
 

@@ -130,6 +130,82 @@ def make_frames_torch(n_frames, cfg, device, seed=None, snr_db="cfg", chunk=64):
     return rx, pilot_asc, src
 
 
+def make_frames_mu(n_frames, n_ant, fft_size, cp_len, n_sym, qam_bits, n_users, snr_db=None, seed=0, h=None, pilot_asc=None):
+    """Multi-user uplink frames (include/ofdm_lsmrc.h, lsmrc_demod_frames_device_mu): symbol u < U carries user u's
+    pilot (the handle's pilot, the other users silent), symbols U..S-1 the data of all U users at once; i.i.d. Rayleigh
+    channel per user, antenna and subcarrier; AWGN at `snr_db` per user and antenna.  `h` [F,U,A,K] (bin order)
+    replaces the random channel.  With n_users=1 the random draws, their order and the arithmetic are those of
+    make_frames: rx is byte-identical.  Returns dict(rx [F,S,A,N+C] c64, pilot_asc [K] c64, src_idx [F,S-U,U,K] u8
+    (ascending frequency), h_true [F,U,A,K] c128 (bin order))."""
+    F, A, N, C, S, U = n_frames, n_ant, fft_size, cp_len, n_sym, n_users
+    K = N - 1
+    assert 1 <= U < S
+    rng = np.random.default_rng(seed)
+    pilot_asc = make_pilot(K, seed) if pilot_asc is None else np.asarray(pilot_asc, np.complex64)
+    src_idx = rng.integers(0, 1 << qam_bits, size=(F, S - U, U, K), dtype=np.uint8)
+    data_asc = qam_map_indices(src_idx, qam_bits)
+    tx_bin = np.zeros((F, S, U, N), np.complex128)
+    for u in range(U):
+        tx_bin[:, u, u, 1:] = asc_to_bin(pilot_asc.astype(np.complex128))
+    tx_bin[:, U:, :, 1:] = asc_to_bin(data_asc)
+    if h is None:
+        h = (rng.standard_normal((F, U, A, K)) + 1j * rng.standard_normal((F, U, A, K))) / np.sqrt(2.0)
+    else:
+        h = np.asarray(h, np.complex128)
+        assert h.shape == (F, U, A, K)
+    hfull = np.zeros((F, U, A, N), np.complex128)
+    hfull[..., 1:] = h
+    yf = tx_bin[:, :, 0, None, :] * hfull[:, None, 0, :, :]    # [F,S,A,N]
+    for u in range(1, U):
+        yf = yf + tx_bin[:, :, u, None, :] * hfull[:, None, u, :, :]
+    yt = np.fft.ifft(yf, axis=-1)
+    if snr_db is not None:
+        sig_pow = K / (N * N)
+        sigma = np.sqrt(sig_pow / (10.0 ** (snr_db / 10.0)) / 2.0)
+        yt = yt + sigma * (rng.standard_normal(yt.shape) + 1j * rng.standard_normal(yt.shape))
+    rx = np.concatenate([yt[..., N - C:], yt], axis=-1) if C > 0 else yt
+    return {"rx": np.ascontiguousarray(rx.astype(np.complex64)), "pilot_asc": pilot_asc,
+            "src_idx": src_idx, "h_true": h}
+
+
+def make_frames_mu_torch(n_frames, n_ant, fft_size, cp_len, n_sym, qam_bits, n_users, device, seed=0, snr_db=30.0,
+                         chunk=16):
+    """make_frames_mu built directly on `device` with torch, for full-size batches (same frame format, its own random
+    stream).  Returns (rx [F,S,A,N+C] complex64 tensor, pilot_asc numpy [K], src_idx [F,S-U,U,K] uint8 tensor)."""
+    import torch
+
+    A, N, C, S, U, b = n_ant, fft_size, cp_len, n_sym, n_users, qam_bits
+    K = N - 1
+    g = torch.Generator(device=device)
+    g.manual_seed(seed)
+    pilot_asc = make_pilot(K, seed)
+    pil_bin = torch.from_numpy(asc_to_bin(pilot_asc)).to(device)
+    lut = torch.from_numpy(qam_map_indices(np.arange(1 << b), b).astype(np.complex64)).to(device)
+    rx = torch.empty((n_frames, S, A, N + C), dtype=torch.complex64, device=device)
+    src = torch.empty((n_frames, S - U, U, K), dtype=torch.uint8, device=device)
+    shift = (K + 1) // 2
+    for f0 in range(0, n_frames, chunk):
+        nf = min(chunk, n_frames - f0)
+        idx = torch.randint(0, 1 << b, (nf, S - U, U, K), generator=g, device=device, dtype=torch.uint8)
+        src[f0:f0 + nf] = idx
+        tx = torch.zeros((nf, S, U, N), dtype=torch.complex64, device=device)
+        for u in range(U):
+            tx[:, u, u, 1:] = pil_bin
+        tx[:, U:, :, 1:] = torch.roll(lut[idx.long()], -shift, dims=-1)
+        h = torch.zeros((nf, U, A, N), dtype=torch.complex64, device=device)
+        h[..., 1:] = torch.view_as_complex(torch.randn((nf, U, A, K, 2), generator=g, device=device) * (0.5 ** 0.5))
+        yf = torch.einsum("fsun,fuan->fsan", tx, h)
+        yt = torch.fft.ifft(yf, dim=-1)
+        if snr_db is not None:
+            sigma = (K / (N * N) / (10.0 ** (snr_db / 10.0)) / 2.0) ** 0.5
+            yt = yt + sigma * torch.view_as_complex(torch.randn((*yt.shape, 2), generator=g, device=device))
+        rx[f0:f0 + nf, :, :, C:] = yt
+        if C > 0:
+            rx[f0:f0 + nf, :, :, :C] = yt[..., N - C:]
+        del tx, h, yf, yt, idx
+    return rx, pilot_asc, src
+
+
 def make_pn(length=255, seed=0x1D):
     """+-1 maximal-length sequence (8-bit LFSR x^8+x^6+x^5+x^4+1 -> period 255), as complex64.  Stands in for
     the reference's PNSeq_255_MaxLenSeq.dat (rx_and_corr.cpp:228), which is not shipped."""

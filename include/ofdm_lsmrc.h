@@ -236,6 +236,34 @@ int lsmrc_sync_assemble(lsmrc_handle h, const void *d_buf1, const void *d_buf2, 
 int lsmrc_zf_create(lsmrc_handle h, const void *d_x, int n_ant, int n_sc, int n_users, void *d_hzf, int *n_singular);
 int lsmrc_zf_apply(lsmrc_handle h, const void *d_hzf, const void *d_xd, int n_ant, int n_sc, int n_users, void *d_hx);
 
+/* ---- multi-user uplink: per-user LS channel estimates and linear detection fused with the row FFT (not in the
+ *      reference; DESIGN.md 8e).  Frame format: the usual rx [F][S][A][N+C] (N+C per antenna row, CP first), with
+ *      U = n_users:
+ *        symbols 0 .. U-1   time-orthogonal pilots: on symbol u user u sends the handle's pilot (lsmrc_set_pilot*),
+ *                           the other users are silent;
+ *        symbols U .. S-1   data of all U users on the same subcarriers at once.
+ *      With U = 1 this is the single-user frame.  Per frame f and subcarrier k (FFT-bin order):
+ *        H[u][a][k] = Z_u[a][k] / X[k]                       LS per user (Z_u: FFT of pilot symbol u)
+ *        G_k = H_k^H H_k + lambda I,  W_k = inv(G_k) H_k^H    H_k the A x U matrix; W_k is U x A
+ *        xhat[s][u][k] = sum_a W_k[u][a] Z_s[a][k]           every data symbol s
+ *      ZF: lambda = 0.  MMSE: lambda = noise_var, the noise variance per antenna and subcarrier after the FFT (same
+ *      convention as lsmrc_demod_frames_device_soft).  A subcarrier whose Gram matrix G_k is singular (a pivot below
+ *      1e-6 of its largest entry, the rule of lsmrc_zf_create) gets W_k = 0, so its outputs are zero.
+ *      With U = 1 and ZF, W = conj(H) / sum_a |H|^2: MRC.
+ *      Device pointers, complex64 unless noted; the handle's compute stream, as lsmrc_demod_frames_device:
+ *        d_hconj    [F][U][A][K]        conj(H) per user in the reference layout (bin k+1 at index k); may be NULL
+ *        d_combined [F][S-U][U][K]      xhat, ascending frequency
+ *        d_bits     [F][S-U][U][row]    hard-demapped xhat, row = lsmrc_bits_row_bytes(N, b); may be NULL
+ *        n_singular (host, may be NULL; non-NULL makes the call synchronous): (frame, subcarrier) pairs whose Gram
+ *                   matrix was singular.
+ *      Any FFT size the handle supports, A <= 256, 1 <= U <= 16, U <= A, U < S.  LSMRC_ERR_INVALID for a bad U, an
+ *      unknown detector, or MMSE with a noise_var that is not finite and > 0; LSMRC_ERR_NO_PILOT without a pilot.
+ *      Nothing is mirrored on the host: with n_singular == NULL the call can be captured into a CUDA graph after one
+ *      ordinary call of the same size (which allocates its scratch). */
+enum { LSMRC_DETECT_ZF = 0, LSMRC_DETECT_MMSE = 1 };
+int lsmrc_demod_frames_device_mu(lsmrc_handle h, const void *d_rx, int n_frames, int n_users, int detector,
+                                 float noise_var, void *d_hconj, void *d_combined, void *d_bits, int *n_singular);
+
 /* ---- memory and stream plumbing, so callers need no CUDA headers (replaces the raw
  *      cudaMalloc/cudaMemcpy/cudaFree calls of gpuLS_main.cu:73-91,135-139) ------------ */
 int lsmrc_dev_alloc(lsmrc_handle h, size_t bytes, void **d_ptr);

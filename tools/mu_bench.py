@@ -1,0 +1,144 @@
+"""Throughput of the multi-user receiver (lsmrc_demod_frames_device_mu) against single-user MRC
+(lsmrc_demod_frames_device) on the same device-resident input, alternating the two in one process.
+
+Inputs are built on the GPU (synth.make_frames_mu_torch) and are larger than twice the 126 MB L2, so every timed call
+streams its frames from HBM; the batches hold enough (frame, symbol) pairs to give every SM work (c2: 64 frames, c4: 32),
+since a smaller batch measures an idle GPU for either receiver.  Per call: CUDA events around the call, >= 5 warm-ups, >= 20 timed calls, median.
+One JSON line per (shape, users, detector) with the card name and power limit read in the same run.
+
+  python tools/mu_bench.py [--quick] [--out DIR]
+"""
+from __future__ import annotations
+
+import argparse
+import json
+import os
+import statistics
+import subprocess
+import sys
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+
+HBM_PEAK_GBS = 6555.2  # measured HBM read+write peak of the B200 (DESIGN.md)
+L2_BYTES = 126 << 20
+
+# (name, A, N, C, S, U, detector, frames).  c4 with 16 users needs more than 16 symbols (16 of them are pilots): S = 20.
+CASES = [
+    ("c2", 64, 1024, 64, 101, 1, "zf", 64),
+    ("c2", 64, 1024, 64, 101, 4, "zf", 64),
+    ("c2", 64, 1024, 64, 101, 4, "mmse", 64),
+    ("c2", 64, 1024, 64, 101, 8, "zf", 64),
+    ("c4", 256, 4096, 288, 14, 4, "zf", 32),
+    ("c4", 256, 4096, 288, 14, 4, "mmse", 32),
+    ("c4", 256, 4096, 288, 14, 8, "zf", 32),
+    ("c4_S20", 256, 4096, 288, 20, 16, "zf", 32),
+]
+
+
+def algorithmic_bytes(A, N, S, U, qam_bits):
+    """per frame: samples in (8*A*S*N, CP not counted) + per-user channel out (8*U*A*K) + detected symbols out
+    (8*(S-U)*U*K) + packed bits out"""
+    K = N - 1
+    bits = (S - U) * U * ((K * qam_bits + 7) // 8)
+    return 8 * A * S * N + 8 * U * A * K + 8 * (S - U) * U * K + bits
+
+
+def card():
+    import torch
+
+    name = torch.cuda.get_device_name(0)
+    try:
+        pl = subprocess.run(["nvidia-smi", "-i", "0", "--query-gpu=power.limit", "--format=csv,noheader"], capture_output=True,
+                            text=True, timeout=30).stdout.strip()
+    except Exception as e:  # (reported, not guessed)
+        pl = f"unknown ({e.__class__.__name__})"
+    return name, pl
+
+
+def time_calls(fn_a, fn_b, warmup, iters):
+    import torch
+
+    ev = [[torch.cuda.Event(enable_timing=True) for _ in range(2)] for _ in range(2)]
+    for _ in range(warmup):
+        fn_a()
+        fn_b()
+    torch.cuda.synchronize()
+    ta, tb = [], []
+    for _ in range(iters):
+        for fn, e, out in ((fn_a, ev[0], ta), (fn_b, ev[1], tb)):
+            e[0].record()
+            fn()
+            e[1].record()
+            e[1].synchronize()
+            out.append(e[0].elapsed_time(e[1]))
+    return statistics.median(ta), statistics.median(tb)
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--warmup", type=int, default=5)
+    ap.add_argument("--iters", type=int, default=20)
+    ap.add_argument("--quick", action="store_true", help="first two cases only, one frame each (rehearsal)")
+    ap.add_argument("--out", default=None, help="also append the JSON lines to DIR/mu_bench.jsonl")
+    args = ap.parse_args()
+    import torch
+
+    import ofdm_b200
+
+    if not torch.cuda.is_available():
+        raise SystemExit("mu_bench needs a CUDA GPU")
+    dev = torch.device("cuda:0")
+    name, power = card()
+    b = 4
+    lines = []
+    for (tag, A, N, C, S, U, det, F) in (CASES[:2] if args.quick else CASES):
+        K = N - 1
+        frame_bytes = 8 * S * A * (N + C)
+        if args.quick:
+            F = 1
+        else:
+            assert F * frame_bytes > 2 * L2_BYTES
+        rx, pilot, _ = ofdm_b200.synth.make_frames_mu_torch(F, A, N, C, S, b, U, dev, seed=1, snr_db=30.0, chunk=1)
+        comb_mu = torch.empty((F, S - U, U, K), dtype=torch.complex64, device=dev)
+        bits_mu = torch.empty((F, S - U, U, (K * b + 7) // 8), dtype=torch.uint8, device=dev)
+        hc_mu = torch.empty((F, U, A, K), dtype=torch.complex64, device=dev)
+        comb_su = torch.empty((F, S - 1, K), dtype=torch.complex64, device=dev)
+        bits_su = torch.empty((F, S - 1, (K * b + 7) // 8), dtype=torch.uint8, device=dev)
+        hc_su = torch.empty((F, A, K), dtype=torch.complex64, device=dev)
+        nv = 0.001 if det == "mmse" else 0.0
+        torch.cuda.synchronize()
+        st = torch.cuda.Stream(dev)  # (a stream of its own: handle 0 would select the receiver's internal stream)
+        with ofdm_b200.LsMrcReceiver(A, N, C, S, b) as r, torch.cuda.stream(st):
+            r.set_pilot(pilot)
+            r.set_stream(st.cuda_stream)
+
+            def mu():
+                r.demod_frames_device_mu(rx, F, U, comb_mu, bits_mu, hc_mu, detector=det, noise_var=nv)
+
+            def su():
+                r.demod_frames_device(rx, F, comb_su, bits_su, hc_su)
+
+            t_mu, t_su = time_calls(mu, su, args.warmup, args.iters)
+            r.set_stream(None)
+        byt = F * algorithmic_bytes(A, N, S, U, b)
+        rec = {"case": tag, "A": A, "N": N, "C": C, "S": S, "U": U, "detector": det, "qam_bits": b, "frames": F,
+               "input_MB": round(F * frame_bytes / 1e6, 1), "ms_mu": round(t_mu, 4), "ms_mrc": round(t_su, 4),
+               "antenna_samples_per_s": F * S * A * (N + C) / (t_mu * 1e-3),
+               "alg_GBps": round(byt / (t_mu * 1e-3) / 1e9, 1),
+               "hbm_fraction": round(byt / (t_mu * 1e-3) / 1e9 / HBM_PEAK_GBS, 4),
+               "ratio_to_mrc": round(t_su / t_mu, 4), "gpu": name, "power_limit": power,
+               "timing": f"median of {args.iters} CUDA-event timed calls after {args.warmup} warm-ups, alternating with MRC"}
+        print(json.dumps(rec), flush=True)
+        lines.append(rec)
+        del rx, comb_mu, bits_mu, hc_mu, comb_su, bits_su, hc_su
+        torch.cuda.empty_cache()
+    if args.out:
+        os.makedirs(args.out, exist_ok=True)
+        with open(os.path.join(args.out, "mu_bench.jsonl"), "a") as f:
+            for rec in lines:
+                f.write(json.dumps(rec) + "\n")
+
+
+if __name__ == "__main__":
+    main()
