@@ -75,6 +75,8 @@ ABI = {
     "lsmrc_zf_apply": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
     "lsmrc_demod_frames_device_mu": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_float, c_void_p, c_void_p, c_void_p,
                                              POINTER(c_int)]),
+    "lsmrc_demod_frames_device_mu_soft": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_float, c_void_p, c_void_p, c_void_p,
+                                                  c_void_p, c_void_p, POINTER(c_int)]),
     "lsmrc_ring_copy_query": (c_int, [c_void_p, c_int]),
     "lsmrc_ring_submit_frames": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_int]),
     "lsmrc_set_timing": (c_int, [c_void_p, c_int]),
@@ -225,6 +227,18 @@ class LsMrcReceiver:
         self._ck(self.lib.lsmrc_demod_frames_device_mu(self.h, _ptr(d_rx), n_frames, n_users, self.DETECTORS.get(detector, -1),
                                                        float(noise_var), _ptr(d_hconj), _ptr(d_combined), _ptr(d_bits),
                                                        byref(bad) if count_singular else None))
+        return bad.value if count_singular else None
+
+    def demod_frames_device_mu_soft(self, d_rx, n_frames, n_users, d_combined, d_llr, d_bits=None, d_hconj=None, d_sinr=None,
+                                    detector="zf", noise_var=1.0, count_singular=False):
+        """demod_frames_device_mu plus soft output: d_llr [F,S-U,U,K,b] float32 max-log LLRs (LLR > 0 <=> bit 0) and
+        d_sinr [F,U,K] float32 post-detection SINR, both ascending frequency.  noise_var (> 0, both detectors) is the
+        noise variance per antenna and subcarrier; MMSE uses it as its diagonal loading too.  d_combined and d_bits are
+        those of demod_frames_device_mu (for MMSE the biased estimate; the LLRs use the unbiased one)."""
+        bad = c_int(0)
+        self._ck(self.lib.lsmrc_demod_frames_device_mu_soft(self.h, _ptr(d_rx), n_frames, n_users, self.DETECTORS.get(detector, -1),
+                                                            float(noise_var), _ptr(d_hconj), _ptr(d_combined), _ptr(d_bits),
+                                                            _ptr(d_llr), _ptr(d_sinr), byref(bad) if count_singular else None))
         return bad.value if count_singular else None
 
     def zf_apply(self, d_hzf, d_xd, n_ant, n_sc, n_users, d_hx):

@@ -36,10 +36,15 @@ struct PlanOps {
     cudaError_t (*launch)(int mode, const KernelParams&, cudaStream_t, int max_data_ctas, unsigned* grid_out, long long* items_out);
     // shuffle-stage plans: pilot and data items of whole frames in ONE persistent launch (lsmrc_frames_sh); nullptr otherwise
     cudaError_t (*launch_fused)(const KernelParams&, cudaStream_t, int max_data_ctas);
-    // multi-user detection: users per pass of the data kernel, and the launch of the weight layout + data kernel
-    int mu_ug;
+    // multi-user detection: users per pass of the data kernel, and the launch of the weight layout + data kernel; the
+    // mu_soft_* twins run the kernel with the soft epilogue (soft_tab: k_mu_soft_scale's table; nullptr for the hard one)
+    int mu_ug, mu_soft_ug;
     cudaError_t (*mu_prepare)(int* ctas_per_sm);
-    cudaError_t (*mu_launch)(const KernelParams&, const float2* hzf, float2* wd, int n_users, int max_ctas, int n_sms, cudaStream_t);
+    cudaError_t (*mu_soft_prepare)(int* ctas_per_sm);
+    cudaError_t (*mu_launch)(const KernelParams&, const float2* hzf, float2* wd, const float2* soft_tab, int n_users, int max_ctas,
+                             int n_sms, cudaStream_t);
+    cudaError_t (*mu_soft_launch)(const KernelParams&, const float2* hzf, float2* wd, const float2* soft_tab, int n_users, int max_ctas,
+                                  int n_sms, cudaStream_t);
 };
 
 // The one-launch kernel (MODE_ONESHOT) of a plan.  Small FFT sizes have a dedicated latency plan:
@@ -365,27 +370,29 @@ PilotOps make_pilot_ops()
 // Multi-user data kernel (lsmrc_mu_data): users per pass.  Each thread keeps UG * P complex sums in registers next to the
 // FFT working set: the most that compiles without spills (-Xptxas -v) -- two users for the 32-point plans of 1024 and
 // 4096 points (128 registers of sums), one for 512 and 2048 (two spill there), four at 16 points, eight at 8.  Larger
-// U re-runs the row transforms once per group of UG users (DESIGN.md 8e).
-template <class PL>
+// U re-runs the row transforms once per group of UG users (DESIGN.md 8e).  The soft epilogue (SOFT) compiles without
+// spills at the same UG on every plan (DESIGN.md 8f).
+template <class PL, bool SOFT = false>
 constexpr int mu_ug() { return PL::P >= 32 ? ((PL::N == 512 || PL::N == 2048) ? 1 : 2) : (PL::P >= 16 ? 4 : 8); }
 
 template <class PL>
 constexpr size_t mu_smem() { return sizeof(float2) * (size_t)(PL::TWN + PL::TEAMS * PL::TEAM_STRIDE); }
 
-template <class PL>
+template <class PL, bool SOFT>
 cudaError_t mu_prepare_impl(int* ctas_per_sm)
 {
-    constexpr int UG = mu_ug<PL>();
-    cudaError_t e = cudaFuncSetAttribute(lsmrc_mu_data<PL, UG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mu_smem<PL>());
+    constexpr int UG = mu_ug<PL, SOFT>();
+    cudaError_t e = cudaFuncSetAttribute(lsmrc_mu_data<PL, UG, SOFT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mu_smem<PL>());
     if (e != cudaSuccess) return e;
-    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas_per_sm, lsmrc_mu_data<PL, UG>, PL::THREADS, mu_smem<PL>());
+    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas_per_sm, lsmrc_mu_data<PL, UG, SOFT>, PL::THREADS, mu_smem<PL>());
 }
 
 // max_ctas: resident CTAs of lsmrc_mu_data on the whole GPU (mu_prepare_impl x SMs)
-template <class PL>
-cudaError_t mu_launch_impl(const KernelParams& p, const float2* hzf, float2* wd, int n_users, int max_ctas, int n_sms, cudaStream_t st)
+template <class PL, bool SOFT>
+cudaError_t mu_launch_impl(const KernelParams& p, const float2* hzf, float2* wd, const float2* soft_tab, int n_users, int max_ctas, int n_sms,
+                           cudaStream_t st)
 {
-    constexpr int UG = mu_ug<PL>();
+    constexpr int UG = mu_ug<PL, SOFT>();
     const int groups = (n_users + UG - 1) / UG;
     cudaError_t e;
     const long long rows = (long long)p.n_frames * groups * UG * p.n_ant;
@@ -396,7 +403,7 @@ cudaError_t mu_launch_impl(const KernelParams& p, const float2* hzf, float2* wd,
     const long long items = (long long)p.n_frames * groups * p.n_sym_work;
     long long grid = (items + PL::TEAMS - 1) / PL::TEAMS;
     if (grid > max_ctas) grid = max_ctas;
-    lsmrc_mu_data<PL, UG><<<(unsigned)grid, PL::THREADS, mu_smem<PL>(), st>>>(p, wd, n_users, groups);
+    lsmrc_mu_data<PL, UG, SOFT><<<(unsigned)grid, PL::THREADS, mu_smem<PL>(), st>>>(p, wd, n_users, groups, soft_tab);
     return cudaGetLastError();
 }
 
@@ -417,9 +424,12 @@ PlanOps make_ops()
     o.prepare = &prepare_impl<PL, MINB>;
     o.launch = &launch_impl<PL, MINB>;
     o.launch_fused = PL::SH > 1 ? &launch_fused_impl<PL, MINB> : nullptr;
-    o.mu_ug = mu_ug<PL>();
-    o.mu_prepare = &mu_prepare_impl<PL>;
-    o.mu_launch = &mu_launch_impl<PL>;
+    o.mu_ug = mu_ug<PL, false>();
+    o.mu_soft_ug = mu_ug<PL, true>();
+    o.mu_prepare = &mu_prepare_impl<PL, false>;
+    o.mu_soft_prepare = &mu_prepare_impl<PL, true>;
+    o.mu_launch = &mu_launch_impl<PL, false>;
+    o.mu_soft_launch = &mu_launch_impl<PL, true>;
     return o;
 }
 
@@ -609,9 +619,11 @@ struct lsmrc_ctx {
     float2* d_mu_hconj = nullptr;  // [U][F][A][K] conj(H) per user, as the pilot kernel writes it
     float2* d_mu_hzf = nullptr;    // [F][K][U][A] conj(W)
     float2* d_mu_wd = nullptr;     // [F][UP][A][N] W in the data kernel's slot layout
-    size_t mu_hconj_cap = 0, mu_hzf_cap = 0, mu_wd_cap = 0;  // bytes
+    float* d_mu_soft = nullptr;    // soft output: ginv_diag [F][U][K] float, then the (rho, scale) table [F][U][K] float2
+    size_t mu_hconj_cap = 0, mu_hzf_cap = 0, mu_wd_cap = 0, mu_soft_cap = 0;  // bytes
     int* d_mu_count = nullptr;     // singular (frame, subcarrier) pairs
     int mu_max_ctas = 0;           // resident CTAs of the multi-user data kernel (0: not prepared yet)
+    int mu_soft_max_ctas = 0;      // the same for its soft instantiation
     float* soft_llr = nullptr;            // set for the duration of a *_soft call
     float soft_inv_noise = 1.f;
     bool timing = false;
@@ -1065,8 +1077,10 @@ int zf_tile(const lsmrc_ctx* h, int n_ant, int n_users)
 // The dynamic shared-memory limit of k_zf_create is a per-device, per-process attribute: lsmrc_create raises it once to the
 // largest tile zf_tile can pick (smem_optin - 1024), the same value for every handle, so no handle lowers it under
 // another and no call sets it (calls stay capturable).  Frames go on gridDim.y in chunks of at most 65535.
+// ginv_diag (may be nullptr): [F][U][K] diagonal of inv(G), frame stride U * K.
 int launch_zf_create(lsmrc_ctx* h, cudaStream_t st, const float2* x, float2* hzf, int n_ant, int n_sc, int n_users, int kt, float lambda,
-                     int n_frames, long long x_frame_stride, long long x_user_stride, long long hzf_frame_stride, int* d_count)
+                     int n_frames, long long x_frame_stride, long long x_user_stride, long long hzf_frame_stride, int* d_count,
+                     float* ginv_diag = nullptr)
 {
     const size_t smem = zf_smem(kt, n_ant, n_users);
     constexpr int kMaxGridY = 65535;
@@ -1074,7 +1088,8 @@ int launch_zf_create(lsmrc_ctx* h, cudaStream_t st, const float2* x, float2* hzf
         const int nf = n_frames - f0 < kMaxGridY ? n_frames - f0 : kMaxGridY;
         const dim3 grid((unsigned)((n_sc + kt - 1) / kt), (unsigned)nf);
         k_zf_create<<<grid, 128, smem, st>>>(x + f0 * x_frame_stride, hzf + f0 * hzf_frame_stride, n_ant, n_sc, n_users, kt, lambda,
-                                             x_frame_stride, x_user_stride, hzf_frame_stride, d_count);
+                                             x_frame_stride, x_user_stride, hzf_frame_stride, d_count,
+                                             ginv_diag ? ginv_diag + (long long)f0 * n_users * n_sc : nullptr);
         h->launches++;
         CK(h, cudaGetLastError());
     }
@@ -1272,6 +1287,7 @@ int lsmrc_destroy(lsmrc_handle h)
     cudaFree(h->d_mu_hconj);
     cudaFree(h->d_mu_hzf);
     cudaFree(h->d_mu_wd);
+    cudaFree(h->d_mu_soft);
     cudaFree(h->d_mu_count);
     cudaFree(h->d_sym);
     cudaFree(h->d_one_hconj);
@@ -1349,42 +1365,54 @@ int lsmrc_demod_frames_device(lsmrc_handle h, const void* d_rx, int n_frames, vo
                          static_cast<uint8_t*>(d_bits), h->timing);
 }
 
-int lsmrc_demod_frames_device_mu(lsmrc_handle h, const void* d_rx, int n_frames, int n_users, int detector, float noise_var,
-                                 void* d_hconj, void* d_combined, void* d_bits, int* n_singular)
+}  // extern "C"
+
+namespace {
+
+// The multi-user calls (lsmrc_demod_frames_device_mu and _mu_soft) share their argument checks (mu_check), phases 1-2
+// (mu_detect: scratch, per-user LS channel, detector build) and the hand-back (mu_finish); they differ in phase 3.
+int mu_check(lsmrc_ctx* h, const void* d_rx, const void* d_combined, int n_frames, int n_users, int detector, float noise_var)
 {
     if (!h || !d_rx || !d_combined) return fail(h, LSMRC_ERR_INVALID, "null argument");
     if (n_frames < 0) return fail(h, LSMRC_ERR_INVALID, "n_frames < 0");
-    const int A = h->cfg.n_ant, S = h->cfg.n_sym, N = h->cfg.fft_size, K = h->K;
+    const int A = h->cfg.n_ant, S = h->cfg.n_sym;
     if (n_users < 1 || n_users > kZfMaxUsers || n_users > A || n_users >= S)
         return fail(h, LSMRC_ERR_INVALID, "need 1 <= n_users <= 16, n_users <= n_ant and n_users < n_sym");
     if (detector != LSMRC_DETECT_ZF && detector != LSMRC_DETECT_MMSE) return fail(h, LSMRC_ERR_INVALID, "unknown detector");
     if (detector == LSMRC_DETECT_MMSE && !(std::isfinite(noise_var) && noise_var > 0.f))
         return fail(h, LSMRC_ERR_INVALID, "MMSE needs a finite noise_var > 0");
     if (!h->have_pilot) return fail(h, LSMRC_ERR_NO_PILOT, "set the pilot first");
-    if (n_frames == 0) {
-        if (n_singular) *n_singular = 0;
-        return LSMRC_OK;
-    }
+    return LSMRC_OK;
+}
+
+// Phases 1-2 on stream st for n_frames >= 1.  UG: users per pass of the data kernel that follows (Wd is sized for it);
+// ginv_diag (nullptr unless soft output is wanted) receives inv(G)'s diagonal [F][U][K].  On return p holds the data
+// kernel's parameters except its outputs.
+int mu_detect(lsmrc_ctx* h, cudaStream_t st, const void* d_rx, int n_frames, int n_users, int detector, float noise_var, int UG,
+              bool count, bool soft, KernelParams& p)
+{
+    const int A = h->cfg.n_ant, S = h->cfg.n_sym, N = h->cfg.fft_size, K = h->K;
     const int kt = zf_tile(h, A, n_users);
     if (kt < 1) return fail(h, LSMRC_ERR_UNSUPPORTED, "n_ant * n_users too large for one CTA's shared memory");
-    CK(h, cudaSetDevice(h->cfg.device));
-    cudaStream_t st = compute_stream(h);
-    const int U = n_users, UP = (U + h->ops->mu_ug - 1) / h->ops->mu_ug * h->ops->mu_ug;
+    const int U = n_users, UP = (U + UG - 1) / UG * UG;
     const long long F = n_frames;
     int rc;
     if ((rc = ensure_chan(h, h->mu_ch, n_frames, st)) != LSMRC_OK) return rc;
     if ((rc = ensure_scratch(h, h->d_mu_hconj, h->mu_hconj_cap, sizeof(float2) * (size_t)(U * F * A * K), st)) != LSMRC_OK) return rc;
     if ((rc = ensure_scratch(h, h->d_mu_hzf, h->mu_hzf_cap, sizeof(float2) * (size_t)(F * K * U * A), st)) != LSMRC_OK) return rc;
     if ((rc = ensure_scratch(h, h->d_mu_wd, h->mu_wd_cap, sizeof(float2) * (size_t)(F * UP * A * N), st)) != LSMRC_OK) return rc;
+    if (soft && (rc = ensure_scratch(h, h->d_mu_soft, h->mu_soft_cap, (sizeof(float2) + sizeof(float)) * (size_t)(F * U * K), st)) != LSMRC_OK)
+        return rc;
     if (!h->d_mu_count) CK(h, cudaMalloc(&h->d_mu_count, sizeof(int)));
-    if (h->mu_max_ctas == 0) {
+    int& max_ctas = soft ? h->mu_soft_max_ctas : h->mu_max_ctas;
+    if (max_ctas == 0) {
         int per_sm = 0;
-        CK(h, h->ops->mu_prepare(&per_sm));
+        CK(h, (soft ? h->ops->mu_soft_prepare : h->ops->mu_prepare)(&per_sm));
         if (per_sm < 1) return fail(h, LSMRC_ERR_CUDA, "multi-user data kernel does not fit on an SM");
-        h->mu_max_ctas = per_sm * h->n_sms;
+        max_ctas = per_sm * h->n_sms;
     }
     // 1. LS channel of every user from its own pilot symbol: the single-user pilot launch, once per pilot symbol
-    KernelParams p = base_params(h);
+    p = base_params(h);
     p.n_frames = n_frames;
     const long long user_elems = F * A * K;
     for (int u = 0; u < U; ++u) {
@@ -1392,18 +1420,22 @@ int lsmrc_demod_frames_device_mu(lsmrc_handle h, const void* d_rx, int n_frames,
         if ((rc = launch_pilot(h, st, p, h->mu_ch, h->d_mu_hconj + u * user_elems, nullptr)) != LSMRC_OK) return rc;
     }
     // 2. detector per (frame, subcarrier): X = conj(H) [U][A][K] of the frame -> Hzf = conj(W)
-    if (n_singular) CK(h, cudaMemsetAsync(h->d_mu_count, 0, sizeof(int), st));
+    if (count) CK(h, cudaMemsetAsync(h->d_mu_count, 0, sizeof(int), st));
     if ((rc = launch_zf_create(h, st, h->d_mu_hconj, h->d_mu_hzf, A, K, U, kt, detector == LSMRC_DETECT_MMSE ? noise_var : 0.f, n_frames,
-                               (long long)A * K, user_elems, (long long)K * U * A, n_singular ? h->d_mu_count : nullptr)) != LSMRC_OK)
+                               (long long)A * K, user_elems, (long long)K * U * A, count ? h->d_mu_count : nullptr,
+                               soft ? h->d_mu_soft + 2 * F * U * K : nullptr)) != LSMRC_OK)
         return rc;
-    // 3. detection fused with the row FFT of every data symbol
     p.rx = static_cast<const float2*>(d_rx);
     p.first_sym = U;
     p.n_sym_work = S - U;
-    p.combined = static_cast<float2*>(d_combined);
-    p.bits = static_cast<uint8_t*>(d_bits);
-    CK(h, h->ops->mu_launch(p, h->d_mu_hzf, h->d_mu_wd, U, h->mu_max_ctas, h->n_sms, st));
-    h->launches += 2;
+    return LSMRC_OK;
+}
+
+// after phase 3: conj(H) to the caller's layout, the singular count back to the host
+int mu_finish(lsmrc_ctx* h, cudaStream_t st, int n_frames, int n_users, void* d_hconj, int* n_singular)
+{
+    const int A = h->cfg.n_ant, K = h->K, U = n_users;
+    const long long user_elems = (long long)n_frames * A * K;
     if (d_hconj) {  // [U][F][A][K] -> [F][U][A][K]
         const size_t row = sizeof(float2) * (size_t)A * K;
         for (int u = 0; u < U; ++u)
@@ -1415,6 +1447,66 @@ int lsmrc_demod_frames_device_mu(lsmrc_handle h, const void* d_rx, int n_frames,
         CK(h, cudaStreamSynchronize(st));
     }
     return LSMRC_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int lsmrc_demod_frames_device_mu(lsmrc_handle h, const void* d_rx, int n_frames, int n_users, int detector, float noise_var,
+                                 void* d_hconj, void* d_combined, void* d_bits, int* n_singular)
+{
+    int rc;
+    if ((rc = mu_check(h, d_rx, d_combined, n_frames, n_users, detector, noise_var)) != LSMRC_OK) return rc;
+    if (n_frames == 0) {
+        if (n_singular) *n_singular = 0;
+        return LSMRC_OK;
+    }
+    CK(h, cudaSetDevice(h->cfg.device));
+    cudaStream_t st = compute_stream(h);
+    KernelParams p;
+    if ((rc = mu_detect(h, st, d_rx, n_frames, n_users, detector, noise_var, h->ops->mu_ug, n_singular != nullptr, false, p)) != LSMRC_OK)
+        return rc;
+    // 3. detection fused with the row FFT of every data symbol
+    p.combined = static_cast<float2*>(d_combined);
+    p.bits = static_cast<uint8_t*>(d_bits);
+    CK(h, h->ops->mu_launch(p, h->d_mu_hzf, h->d_mu_wd, nullptr, n_users, h->mu_max_ctas, h->n_sms, st));
+    h->launches += 2;
+    return mu_finish(h, st, n_frames, n_users, d_hconj, n_singular);
+}
+
+int lsmrc_demod_frames_device_mu_soft(lsmrc_handle h, const void* d_rx, int n_frames, int n_users, int detector, float noise_var,
+                                      void* d_hconj, void* d_combined, void* d_bits, void* d_llr, void* d_sinr, int* n_singular)
+{
+    if (!d_llr) return fail(h, LSMRC_ERR_INVALID, "null argument");
+    if (!(std::isfinite(noise_var) && noise_var > 0.f)) return fail(h, LSMRC_ERR_INVALID, "soft output needs a finite noise_var > 0");
+    int rc;
+    if ((rc = mu_check(h, d_rx, d_combined, n_frames, n_users, detector, noise_var)) != LSMRC_OK) return rc;
+    if (n_frames == 0) {
+        if (n_singular) *n_singular = 0;
+        return LSMRC_OK;
+    }
+    CK(h, cudaSetDevice(h->cfg.device));
+    cudaStream_t st = compute_stream(h);
+    KernelParams p;
+    if ((rc = mu_detect(h, st, d_rx, n_frames, n_users, detector, noise_var, h->ops->mu_soft_ug, n_singular != nullptr, true, p)) != LSMRC_OK)
+        return rc;
+    // 3a. (rho, scale) per (frame, user, subcarrier) from the diagonal of inv(G)
+    const long long n = (long long)n_frames * n_users * h->K;
+    float2* tab = reinterpret_cast<float2*>(h->d_mu_soft);
+    long long blocks = (n + 255) / 256;
+    if (blocks > (long long)h->n_sms * 16) blocks = (long long)h->n_sms * 16;
+    k_mu_soft_scale<<<(unsigned)blocks, 256, 0, st>>>(h->d_mu_soft + 2 * n, tab, static_cast<float*>(d_sinr), n, h->K,
+                                                      detector == LSMRC_DETECT_MMSE ? 1 : 0, noise_var, noise_var);
+    h->launches++;
+    CK(h, cudaGetLastError());
+    // 3b. detection fused with the row FFT, with the soft epilogue
+    p.combined = static_cast<float2*>(d_combined);
+    p.bits = static_cast<uint8_t*>(d_bits);
+    p.llr = static_cast<float*>(d_llr);
+    CK(h, h->ops->mu_soft_launch(p, h->d_mu_hzf, h->d_mu_wd, tab, n_users, h->mu_soft_max_ctas, h->n_sms, st));
+    h->launches += 2;
+    return mu_finish(h, st, n_frames, n_users, d_hconj, n_singular);
 }
 
 int lsmrc_demod_frames_device_soft(lsmrc_handle h, const void* d_rx, int n_frames, void* d_combined, void* d_bits,

@@ -2169,11 +2169,14 @@ __global__ void k_llr_rows(const float2* __restrict__ combined, const float* __r
 // at u * x_user_stride.  Per subcarrier the result depends on neither KT nor the frame batch.
 // With X = conj(H) (H the A x U channel of subcarrier k), Hzf[k][u][a] = conj(W_k[u][a]) for the linear detector
 // W_k = inv(H^H H + lambda*I) H^H: ZF at lambda = 0, MMSE at lambda = noise variance (DESIGN.md 8e).
+// ginv_diag (may be nullptr) [frame][U][K]: the real diagonal of M_k = inv(G_k), 0 on a singular subcarrier -- what the
+// soft output of the multi-user path needs (DESIGN.md 8f).
 constexpr int kZfKT = 8;
 constexpr int kZfMaxUsers = 16;
 
 __global__ void k_zf_create(const float2* __restrict__ X, float2* __restrict__ Hzf, int A, int K, int U, int KT, float lambda,
-                            long long x_frame_stride, long long x_user_stride, long long hzf_frame_stride, int* n_singular)
+                            long long x_frame_stride, long long x_user_stride, long long hzf_frame_stride, int* n_singular,
+                            float* __restrict__ ginv_diag)
 {
     extern __shared__ __align__(16) float2 zsm[];
     float2* s_x = zsm;                      // [KT][A][U]  (users x antennas, column-major per subcarrier)
@@ -2272,6 +2275,15 @@ __global__ void k_zf_create(const float2* __restrict__ X, float2* __restrict__ H
         }
         Hzf[(size_t)(k0 + kt) * A * U + (size_t)u * A + a] = acc;
     }
+    // the row swaps are row operations of [G | I] as well: the right half is inv(G) itself, no permutation to undo.
+    // (A loop of its own after the product, where few registers are live: the kernel keeps its register count.)
+    if (ginv_diag != nullptr) {
+        float* gd = ginv_diag + (long long)blockIdx.y * U * K + k0;
+        for (int idx = threadIdx.x; idx < U * nk; idx += blockDim.x) {
+            const int u = idx / nk, kt = idx - u * nk;  // kt fastest: contiguous in ginv_diag
+            gd[(long long)u * K + kt] = s_ok[kt] ? s_g[((size_t)kt * U + u) * 2 * U + U + u].x : 0.f;
+        }
+    }
 }
 
 // multiplyWithChannelInv: HX[a][k] = sum_u Hk[a + A*u] * Xd[u][k]
@@ -2322,11 +2334,45 @@ __global__ void k_mu_weights(const float2* __restrict__ hzf, float2* __restrict_
     }
 }
 
+// Soft output of the linear detector (DESIGN.md 8f): per (frame, user, subcarrier) from d = [inv(G_k)]_uu (k_zf_create's
+// ginv_diag, [F][U][K] bin order k = bin - 1) the pair (rho, scale) the data kernel's soft epilogue needs:
+//   ZF   (mmse = 0):  rho = 1 / (sigma2 d),              scale = 1
+//   MMSE (mmse = 1):  rho = 1 / (lambda d) - 1 (>= 0),   scale = 1 / beta,  beta = 1 - lambda d = [W H]_uu
+// (rho of MMSE straight from lambda d: 1 - beta cancels in fp32 at high SNR).  d = 0 (singular subcarrier) or rho <= 0
+// give (0, 0): every LLR of that subcarrier is 0.  sinr (may be nullptr) [F][U][K] gets rho in ascending frequency.
+__global__ void k_mu_soft_scale(const float* __restrict__ ginv_diag, float2* __restrict__ tab, float* __restrict__ sinr, long long n,
+                                int K, int mmse, float lambda, float sigma2)
+{
+    for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < n; idx += (long long)gridDim.x * blockDim.x) {
+        const float d = ginv_diag[idx];
+        float rho = 0.f, scale = 0.f;
+        if (d > 0.f) {
+            if (mmse) {
+                const float ld = lambda * d;
+                rho = 1.0f / ld - 1.0f;
+                if (rho > 0.f) scale = 1.0f / (1.0f - ld);
+                else rho = 0.f;
+            } else {
+                rho = 1.0f / (sigma2 * d);
+                scale = 1.0f;
+            }
+        }
+        tab[idx] = make_float2(rho, scale);
+        if (sinr != nullptr) {
+            const long long fu = idx / K;
+            const int bin = (int)(idx - fu * K) + 1, half = (K + 1) / 2;
+            sinr[fu * K + (bin < half ? bin - 1 + half : bin - half)] = rho;
+        }
+    }
+}
+
 // Teams take items (frame f, user group g, data symbol s), consecutive items sharing (f, g) so that the teams working
 // at the same time read the same detector rows (L1/L2).  Outputs: combined [F][S-U][U][K] ascending frequency, bits
 // [F][S-U][U][row].  p.first_sym = U, p.n_sym_work = S-U; n_users = U, UP = groups * UG.
-template <class PL, int UG>
-__global__ void __launch_bounds__(PL::THREADS, 1) lsmrc_mu_data(const KernelParams p, const float2* __restrict__ wd, int n_users, int n_groups)
+// SOFT: also p.llr [F][S-U][U][K][b] from soft_tab [F][U][K] (k_mu_soft_scale); the hard kernel ignores soft_tab.
+template <class PL, int UG, bool SOFT = false>
+__global__ void __launch_bounds__(PL::THREADS, 1) lsmrc_mu_data(const KernelParams p, const float2* __restrict__ wd, int n_users, int n_groups,
+                                                                const float2* __restrict__ soft_tab)
 {
     constexpr int N = PL::N, P = PL::P, T = PL::T, K = N - 1;
     extern __shared__ __align__(16) float2 smem[];
@@ -2369,43 +2415,67 @@ __global__ void __launch_bounds__(PL::THREADS, 1) lsmrc_mu_data(const KernelPara
                 for (int j = 0; j < UG; ++j) acc[j][sl] = cmac(acc[j][sl], y, __ldg(wa + j * wstride + hp));
             });
         }
-        // epilogue per user: ascending-frequency store, hard demap into the team's tile (bytes), bit packing
+        // epilogue per user: ascending-frequency store, hard demap into the team's tile (bytes), bit packing; SOFT: max-log
+        // LLRs of the user's symbol times scale, at rho (DESIGN.md 8f).  BC = bits per symbol, fixed at compile time for
+        // the soft epilogue (straight-line soft_symbol); 0 = p.qam_bits at run time (the hard kernel).
         uint8_t* s_idx = reinterpret_cast<uint8_t*>(my_tiles);
-        const int b = p.qam_bits;
+        auto epilogue = [&](auto bconst) {
+            constexpr int BC = decltype(bconst)::value;
+            const int b = BC > 0 ? BC : p.qam_bits;
 #pragma unroll
-        for (int j = 0; j < UG; ++j) {
-            // padding users of the last group: teams of whole warps skip them; narrower teams share a warp's __syncwarp
-            // with teams of other groups, so they run the epilogue without storing and every lane passes the same barriers
-            const int u = g * UG + j;
-            if constexpr (PL::T >= 32) {
-                if (u >= U) break;
-            }
-            const bool store = ok && u < U;
-            const long long orow = (f * D + s) * U + (u < U ? u : U - 1);
-            float2* out_row = p.combined + orow * K;
-            team_sync<PL>(team);  // the tile (last row's exchange buffer, or the previous user's bytes) is free
-#pragma unroll
-            for (int sl = 0; sl < P; ++sl) {
-                const int bin = PL::bin_of(sl, t);
-                if (bin > 0) {
-                    const int pos = (bin < N / 2) ? (bin - 1 + N / 2) : (bin - N / 2);
-                    if (store) out_row[pos] = acc[j][sl];
-                    s_idx[pos] = (uint8_t)demap_symbol(acc[j][sl].x, acc[j][sl].y, b);
+            for (int j = 0; j < UG; ++j) {
+                // padding users of the last group: teams of whole warps skip them; narrower teams share a warp's
+                // __syncwarp with teams of other groups, so they run the epilogue without storing and every lane passes
+                // the same barriers
+                const int u = g * UG + j;
+                if constexpr (PL::T >= 32) {
+                    if (u >= U) break;
                 }
-            }
-            if (p.bits != nullptr) {
-                team_sync<PL>(team);
-                uint8_t* bits_row = p.bits + orow * p.bits_row_bytes;
-                for (int byte = t; byte < p.bits_row_bytes; byte += T) {
-                    unsigned v8 = 0;
-                    for (int q = 0; q < 8; ++q) {
-                        const int pos = byte * 8 + q;
-                        const int sym = pos / b, bit = pos - sym * b;
-                        if (sym < K) v8 |= ((s_idx[sym] >> bit) & 1u) << q;
+                const bool store = ok && u < U;
+                const long long orow = (f * D + s) * U + (u < U ? u : U - 1);
+                float2* out_row = p.combined + orow * K;
+                [[maybe_unused]] const float2* tab_row = SOFT ? soft_tab + (f * U + u) * K - 1 : nullptr;  // indexed by bin
+                [[maybe_unused]] float* llr_row = SOFT ? p.llr + orow * K * BC : nullptr;
+                team_sync<PL>(team);  // the tile (last row's exchange buffer, or the previous user's bytes) is free
+#pragma unroll
+                for (int sl = 0; sl < P; ++sl) {
+                    const int bin = PL::bin_of(sl, t);
+                    if (bin > 0) {
+                        const int pos = (bin < N / 2) ? (bin - 1 + N / 2) : (bin - N / 2);
+                        if (store) out_row[pos] = acc[j][sl];
+                        s_idx[pos] = (uint8_t)demap_symbol(acc[j][sl].x, acc[j][sl].y, b);
+                        if constexpr (SOFT) {
+                            if (store) {
+                                const float2 rs = __ldg(tab_row + bin);  // (rho, scale)
+                                float l[BC];
+                                soft_symbol<BC>(__fmul_rn(acc[j][sl].x, rs.y), __fmul_rn(acc[j][sl].y, rs.y), rs.x, l);
+#pragma unroll
+                                for (int q = 0; q < BC; ++q) llr_row[pos * BC + q] = l[q];
+                            }
+                        }
                     }
-                    if (store) bits_row[byte] = (uint8_t)v8;
+                }
+                if (p.bits != nullptr) {
+                    team_sync<PL>(team);
+                    uint8_t* bits_row = p.bits + orow * p.bits_row_bytes;
+                    for (int byte = t; byte < p.bits_row_bytes; byte += T) {
+                        unsigned v8 = 0;
+                        for (int q = 0; q < 8; ++q) {
+                            const int pos = byte * 8 + q;
+                            const int sym = pos / b, bit = pos - sym * b;
+                            if (sym < K) v8 |= ((s_idx[sym] >> bit) & 1u) << q;
+                        }
+                        if (store) bits_row[byte] = (uint8_t)v8;
+                    }
                 }
             }
+        };
+        if constexpr (SOFT) {
+            if (p.qam_bits == 2) epilogue(std::integral_constant<int, 2>{});
+            else if (p.qam_bits == 4) epilogue(std::integral_constant<int, 4>{});
+            else epilogue(std::integral_constant<int, 6>{});
+        } else {
+            epilogue(std::integral_constant<int, 0>{});
         }
         team_sync<PL>(team);  // the bytes alias the tile the next item's first row is exchanged through
     }

@@ -264,6 +264,28 @@ enum { LSMRC_DETECT_ZF = 0, LSMRC_DETECT_MMSE = 1 };
 int lsmrc_demod_frames_device_mu(lsmrc_handle h, const void *d_rx, int n_frames, int n_users, int detector,
                                  float noise_var, void *d_hconj, void *d_combined, void *d_bits, int *n_singular);
 
+/* ---- multi-user uplink with soft output: lsmrc_demod_frames_device_mu plus per-user post-detection SINR and max-log
+ *      LLRs for a channel decoder (DESIGN.md 8f).  Per frame, subcarrier k and user u, with M_k = inv(G_k) (G_k as
+ *      above) and d = [M_k]_uu, sigma2 = noise_var:
+ *        ZF:    rho = 1 / (sigma2 d)                      LLRs of xhat
+ *        MMSE:  rho = 1 / (lambda d) - 1 (at least 0)     LLRs of xhat / beta, beta = 1 - lambda d = [W_k H_k]_uu
+ *                                                         (the MMSE output is biased: xhat = beta x + interference + noise)
+ *      rho is the post-detection SINR of user u on subcarrier k; the LLRs are those of lsmrc_demod_frames_device_soft
+ *      with sum|H|^2 / noise_var replaced by rho.  A singular subcarrier gets rho = 0 and all-zero LLRs.  With U = 1
+ *      both detectors give lsmrc_demod_frames_device_soft's LLRs for the same noise_var.
+ *        d_llr      [F][S-U][U][K][b] float, ascending frequency, bit order of the packed bits, LLR > 0 <=> bit 0
+ *        d_sinr     [F][U][K] float, ascending frequency: rho; may be NULL
+ *      Every other argument keeps its meaning and layout from lsmrc_demod_frames_device_mu, and d_combined and d_bits
+ *      are byte-identical to what that call writes for the same input.  For MMSE they therefore stay the biased xhat:
+ *      only the two sign bits of each symbol are guaranteed to agree with the hard bits, the amplitude bits of the LLRs
+ *      come from the unbiased xhat / beta.
+ *      noise_var must be finite and > 0 for both detectors (ZF scales its LLRs by it).  LSMRC_ERR_INVALID for a NULL
+ *      d_llr or such a noise_var, otherwise the errors of lsmrc_demod_frames_device_mu.  With n_singular == NULL the
+ *      call can be captured into a CUDA graph after one ordinary call of the same size. */
+int lsmrc_demod_frames_device_mu_soft(lsmrc_handle h, const void *d_rx, int n_frames, int n_users, int detector,
+                                      float noise_var, void *d_hconj, void *d_combined, void *d_bits,
+                                      void *d_llr, void *d_sinr, int *n_singular);
+
 /* ---- memory and stream plumbing, so callers need no CUDA headers (replaces the raw
  *      cudaMalloc/cudaMemcpy/cudaFree calls of gpuLS_main.cu:73-91,135-139) ------------ */
 int lsmrc_dev_alloc(lsmrc_handle h, size_t bytes, void **d_ptr);

@@ -6,7 +6,10 @@ streams its frames from HBM; the batches hold enough (frame, symbol) pairs to gi
 since a smaller batch measures an idle GPU for either receiver.  Per call: CUDA events around the call, >= 5 warm-ups, >= 20 timed calls, median.
 One JSON line per (shape, users, detector) with the card name and power limit read in the same run.
 
-  python tools/mu_bench.py [--quick] [--out DIR]
+With --soft the pair is lsmrc_demod_frames_device_mu_soft (LLRs and SINR) against lsmrc_demod_frames_device_mu on the
+same input: the cost of the soft output (DESIGN.md 8f).
+
+  python tools/mu_bench.py [--quick] [--soft] [--out DIR]
 """
 from __future__ import annotations
 
@@ -34,6 +37,7 @@ CASES = [
     ("c4", 256, 4096, 288, 14, 8, "zf", 32),
     ("c4_S20", 256, 4096, 288, 20, 16, "zf", 32),
 ]
+SOFT_CASES = [c for c in CASES if c[5] in (4, 8) and c[0] in ("c2", "c4")]
 
 
 def algorithmic_bytes(A, N, S, U, qam_bits):
@@ -42,6 +46,12 @@ def algorithmic_bytes(A, N, S, U, qam_bits):
     K = N - 1
     bits = (S - U) * U * ((K * qam_bits + 7) // 8)
     return 8 * A * S * N + 8 * U * A * K + 8 * (S - U) * U * K + bits
+
+
+def soft_extra_bytes(N, S, U, qam_bits):
+    """per frame, on top of algorithmic_bytes: the LLR store (4*b per user-symbol) and the SINR store (4*U*K)"""
+    K = N - 1
+    return 4 * qam_bits * (S - U) * U * K + 4 * U * K
 
 
 def card():
@@ -80,6 +90,7 @@ def main():
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--iters", type=int, default=20)
     ap.add_argument("--quick", action="store_true", help="first two cases only, one frame each (rehearsal)")
+    ap.add_argument("--soft", action="store_true", help="soft multi-user call against the hard one instead of MU against MRC")
     ap.add_argument("--out", default=None, help="also append the JSON lines to DIR/mu_bench.jsonl")
     args = ap.parse_args()
     import torch
@@ -92,7 +103,8 @@ def main():
     name, power = card()
     b = 4
     lines = []
-    for (tag, A, N, C, S, U, det, F) in (CASES[:2] if args.quick else CASES):
+    cases = SOFT_CASES if args.soft else CASES
+    for (tag, A, N, C, S, U, det, F) in (cases[:2] if args.quick else cases):
         K = N - 1
         frame_bytes = 8 * S * A * (N + C)
         if args.quick:
@@ -106,7 +118,10 @@ def main():
         comb_su = torch.empty((F, S - 1, K), dtype=torch.complex64, device=dev)
         bits_su = torch.empty((F, S - 1, (K * b + 7) // 8), dtype=torch.uint8, device=dev)
         hc_su = torch.empty((F, A, K), dtype=torch.complex64, device=dev)
-        nv = 0.001 if det == "mmse" else 0.0
+        nv = 0.001 if det == "mmse" or args.soft else 0.0
+        if args.soft:
+            llr = torch.empty((F, S - U, U, K, b), dtype=torch.float32, device=dev)
+            sinr = torch.empty((F, U, K), dtype=torch.float32, device=dev)
         torch.cuda.synchronize()
         st = torch.cuda.Stream(dev)  # (a stream of its own: handle 0 would select the receiver's internal stream)
         with ofdm_b200.LsMrcReceiver(A, N, C, S, b) as r, torch.cuda.stream(st):
@@ -119,9 +134,28 @@ def main():
             def su():
                 r.demod_frames_device(rx, F, comb_su, bits_su, hc_su)
 
-            t_mu, t_su = time_calls(mu, su, args.warmup, args.iters)
+            def soft():
+                r.demod_frames_device_mu_soft(rx, F, U, comb_mu, llr, bits_mu, hc_mu, sinr, detector=det, noise_var=nv)
+
+            if args.soft:
+                t_soft, t_mu = time_calls(soft, mu, args.warmup, args.iters)
+            else:
+                t_mu, t_su = time_calls(mu, su, args.warmup, args.iters)
             r.set_stream(None)
         byt = F * algorithmic_bytes(A, N, S, U, b)
+        if args.soft:
+            sbyt = byt + F * soft_extra_bytes(N, S, U, b)
+            rec = {"case": tag, "A": A, "N": N, "C": C, "S": S, "U": U, "detector": det, "qam_bits": b, "frames": F,
+                   "ms_soft": round(t_soft, 4), "ms_hard": round(t_mu, 4), "soft_over_hard": round(t_soft / t_mu, 4),
+                   "llr_bytes_over_input": round(soft_extra_bytes(N, S, U, b) / (8 * A * S * N), 4),
+                   "alg_GBps_soft": round(sbyt / (t_soft * 1e-3) / 1e9, 1),
+                   "hbm_fraction_soft": round(sbyt / (t_soft * 1e-3) / 1e9 / HBM_PEAK_GBS, 4), "gpu": name, "power_limit": power,
+                   "timing": f"median of {args.iters} CUDA-event timed calls after {args.warmup} warm-ups, soft and hard alternating"}
+            print(json.dumps(rec), flush=True)
+            lines.append(rec)
+            del rx, comb_mu, bits_mu, hc_mu, comb_su, bits_su, hc_su, llr, sinr
+            torch.cuda.empty_cache()
+            continue
         rec = {"case": tag, "A": A, "N": N, "C": C, "S": S, "U": U, "detector": det, "qam_bits": b, "frames": F,
                "input_MB": round(F * frame_bytes / 1e6, 1), "ms_mu": round(t_mu, 4), "ms_mrc": round(t_su, 4),
                "antenna_samples_per_s": F * S * A * (N + C) / (t_mu * 1e-3),
