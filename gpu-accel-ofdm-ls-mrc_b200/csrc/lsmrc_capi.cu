@@ -1513,7 +1513,9 @@ int lsmrc_demod_frames_device_soft(lsmrc_handle h, const void* d_rx, int n_frame
                                    void* d_llr, float noise_var)
 {
     if (!h || !d_rx || !d_combined || !d_llr) return fail(h, LSMRC_ERR_INVALID, "null argument");
-    if (!(noise_var > 0.f)) return fail(h, LSMRC_ERR_INVALID, "noise_var must be positive");
+    // the epilogue scales by 1/noise_var: +inf, and subnormals whose reciprocal overflows, would give +-inf or NaN LLRs
+    if (!(std::isfinite(noise_var) && noise_var > 0.f && std::isfinite(1.0f / noise_var)))
+        return fail(h, LSMRC_ERR_INVALID, "soft output needs a finite noise_var > 0 with a finite reciprocal");
     if (n_frames < 0) return fail(h, LSMRC_ERR_INVALID, "n_frames < 0");
     if (!h->have_pilot) return fail(h, LSMRC_ERR_NO_PILOT, "set the pilot first");
     if (n_frames == 0) return LSMRC_OK;

@@ -109,7 +109,9 @@ int lsmrc_demod_frames_device(lsmrc_handle h, const void *d_rx, int n_frames, vo
 /* Same as lsmrc_demod_frames_device plus soft output (SURVEY 8f, rank 2 -- not in the reference):
  * d_llr [F][S-1][K][b] float, ascending frequency, bit order as in the packed bits, LLR > 0 <=> bit 0.
  * Max-log piecewise-linear LLRs scaled by the post-MRC SNR sum|H|^2 / noise_var (noise_var: noise variance
- * per antenna and subcarrier after the FFT, supplied by the caller).  d_bits may be NULL. */
+ * per antenna and subcarrier after the FFT, supplied by the caller).  d_bits may be NULL.
+ * noise_var must be finite and > 0 with a finite float reciprocal (>= 1/FLT_MAX, about 2.9e-39): anything else
+ * (0, negative, NaN, +inf, smaller subnormals) is LSMRC_ERR_INVALID and nothing is launched. */
 int lsmrc_demod_frames_device_soft(lsmrc_handle h, const void *d_rx, int n_frames, void *d_combined,
                                    void *d_bits, void *d_llr, float noise_var);
 
