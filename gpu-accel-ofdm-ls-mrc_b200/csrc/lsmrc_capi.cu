@@ -33,18 +33,15 @@ struct PlanOps {
     size_t smem;
     void (*fill_twiddles)(float2*);
     cudaError_t (*prepare)(int* data_ctas_per_sm, int* pilot_ctas_per_sm);
-    cudaError_t (*launch)(int mode, const KernelParams&, cudaStream_t, int max_data_ctas, unsigned* grid_out, long long* items_out);
+    cudaError_t (*launch)(int mode, const KernelParams&, cudaStream_t, int max_data_ctas);
     // shuffle-stage plans: pilot and data items of whole frames in ONE persistent launch (lsmrc_frames_sh); nullptr otherwise
     cudaError_t (*launch_fused)(const KernelParams&, cudaStream_t, int max_data_ctas);
-    // multi-user detection: users per pass of the data kernel, and the launch of the weight layout + data kernel; the
-    // mu_soft_* twins run the kernel with the soft epilogue (soft_tab: k_mu_soft_scale's table; nullptr for the hard one)
-    int mu_ug, mu_soft_ug;
-    cudaError_t (*mu_prepare)(int* ctas_per_sm);
-    cudaError_t (*mu_soft_prepare)(int* ctas_per_sm);
-    cudaError_t (*mu_launch)(const KernelParams&, const float2* hzf, float2* wd, const float2* soft_tab, int n_users, int max_ctas,
+    // multi-user detection: users per pass of the data kernel, and the launch of the weight layout + data kernel; `soft`
+    // selects the kernel with the soft epilogue (soft_tab: k_mu_soft_scale's table; nullptr for the hard one)
+    int mu_ug;
+    cudaError_t (*mu_prepare)(bool soft, int* ctas_per_sm);
+    cudaError_t (*mu_launch)(bool soft, const KernelParams&, const float2* hzf, float2* wd, const float2* soft_tab, int n_users, int max_ctas,
                              int n_sms, cudaStream_t);
-    cudaError_t (*mu_soft_launch)(const KernelParams&, const float2* hzf, float2* wd, const float2* soft_tab, int n_users, int max_ctas,
-                                  int n_sms, cudaStream_t);
 };
 
 // The one-launch kernel (MODE_ONESHOT) of a plan.  Small FFT sizes have a dedicated latency plan:
@@ -56,16 +53,6 @@ struct OneshotOps {
     cudaError_t (*prepare)(int smem_optin);
     // antenna split to use for this batch, 0 when the mode does not apply
     int (*split)(int n_frames, int n_sym_work, int n_ant, int n_sms, size_t smem_optin);
-    cudaError_t (*launch)(const KernelParams&, cudaStream_t);
-};
-
-// The pilot kernel of a plan.  2048 and 4096 points run it with their own plan (16 points per thread, twice the
-// threads per row): measured 15 % faster than the data kernel's 32-point plan there, while the data kernel prefers 32.
-struct PilotOps {
-    int N, P, R2, R3, teams, threads, twn;
-    size_t smem;
-    void (*fill_twiddles)(float2*);
-    cudaError_t (*prepare)(int* ctas_per_sm);
     cudaError_t (*launch)(const KernelParams&, cudaStream_t);
 };
 
@@ -226,7 +213,7 @@ cudaError_t prepare_impl(int* data_ctas_per_sm, int* pilot_ctas_per_sm)
     // (tensor-memory columns per CTA: 2P for the stage-1 twiddles, power of two >= 32)
     e = occupancy_with_tmem(data_ctas_per_sm, lsmrc_kernel<PL, MODE_DATA, MINB>, PL::THREADS, PL::SMEM_BYTES, PL::TW_TMEM ? 2 * PL::P : 0);
     if (e != cudaSuccess) return e;
-    if constexpr (PL::X_TMA && PL::H_RING) {  // the bulk-copy instantiation of the data kernel shares the persistent grid size
+    if constexpr (PL::X_TMA) {  // the bulk-copy instantiation of the data kernel shares the persistent grid size
         e = cudaFuncSetAttribute(lsmrc_kernel<PL, MODE_DATA, MINB, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PL::SMEM_BYTES);
         if (e != cudaSuccess) return e;
         int xt = 0;
@@ -274,8 +261,7 @@ cudaError_t launch_fused_impl(const KernelParams& p, cudaStream_t st, int max_da
 }
 
 template <class PL, int MINB>
-cudaError_t launch_impl(int mode, const KernelParams& p, cudaStream_t st, int max_data_ctas, unsigned* grid_out,
-                        long long* items_out)
+cudaError_t launch_impl(int mode, const KernelParams& p, cudaStream_t st, int max_data_ctas)
 {
     if (mode == MODE_FFT) {
         const long long groups = ((long long)p.n_frames + PL::TEAMS - 1) / PL::TEAMS;
@@ -285,14 +271,12 @@ cudaError_t launch_impl(int mode, const KernelParams& p, cudaStream_t st, int ma
         const long long n_virtual = (long long)((p.n_frames + p.frames_per_cta - 1) / p.frames_per_cta) * p.n_groups;
         const long long cap = p.pilot_grid_cap > 0 ? p.pilot_grid_cap : n_virtual;
         const unsigned grid = (unsigned)(n_virtual < cap ? n_virtual : cap);  // CTAs stride over the virtual CTAs
-#ifndef LSMRC_NO_PILOT_SH
         if constexpr (PL::SH > 1) {
             if (p.frames_per_cta == 1) {
                 lsmrc_pilot_sh<PL, MINB><<<grid, PL::THREADS, pilot_sh_smem<PL>(), st>>>(p);
                 return cudaGetLastError();
             }
         }
-#endif
         lsmrc_kernel<PL, MODE_PILOT, pilot_minb<PL, MINB>()><<<grid, PL::THREADS, PL::SMEM_BYTES, st>>>(p);
     } else {
         long long items;
@@ -313,15 +297,13 @@ cudaError_t launch_impl(int mode, const KernelParams& p, cudaStream_t st, int ma
             items = (n_work + slots - 1) / slots;
         }
         const unsigned grid = (unsigned)(items < max_data_ctas ? items : max_data_ctas);  // persistent CTAs
-        if (grid_out) *grid_out = grid;
-        if (items_out) *items_out = items;
         if constexpr (PL::SH > 1) {
             if (q.ant_split == 1) {
                 lsmrc_data_sh<PL, MINB><<<grid, PL::THREADS, data_sh_smem<PL>(), st>>>(q);
                 return cudaGetLastError();
             }
         }
-        if constexpr (PL::X_TMA && PL::H_RING) {
+        if constexpr (PL::X_TMA) {
             if (q.x_tma) {  // rows 16-byte aligned: the instantiation that brings them in by bulk copy
                 lsmrc_kernel<PL, MODE_DATA, MINB, true><<<grid, PL::THREADS, PL::SMEM_BYTES, st>>>(q);
                 return cudaGetLastError();
@@ -332,67 +314,33 @@ cudaError_t launch_impl(int mode, const KernelParams& p, cudaStream_t st, int ma
     return cudaGetLastError();
 }
 
-template <class PL, int MINB>
-cudaError_t pilot_prepare_impl(int* ctas_per_sm)
-{
-    cudaError_t e = cudaFuncSetAttribute(lsmrc_kernel<PL, MODE_PILOT, MINB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PL::SMEM_BYTES);
-    if (e != cudaSuccess) return e;
-    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas_per_sm, lsmrc_kernel<PL, MODE_PILOT, MINB>, PL::THREADS, PL::SMEM_BYTES);
-}
-
-template <class PL, int MINB>
-cudaError_t pilot_launch_impl(const KernelParams& p, cudaStream_t st)
-{
-    const long long n_virtual = (long long)((p.n_frames + p.frames_per_cta - 1) / p.frames_per_cta) * p.n_groups;
-    const long long cap = p.pilot_grid_cap > 0 ? p.pilot_grid_cap : n_virtual;
-    lsmrc_kernel<PL, MODE_PILOT, MINB><<<(unsigned)(n_virtual < cap ? n_virtual : cap), PL::THREADS, PL::SMEM_BYTES, st>>>(p);
-    return cudaGetLastError();
-}
-
-template <class PL, int MINB>
-PilotOps make_pilot_ops()
-{
-    PilotOps o;
-    o.N = PL::N;
-    o.P = PL::P;
-    o.R2 = PL::R2;
-    o.R3 = PL::R3;
-    o.teams = PL::TEAMS;
-    o.threads = PL::THREADS;
-    o.twn = PL::TWN;
-    o.smem = PL::SMEM_BYTES;
-    o.fill_twiddles = &fill_twiddles_impl<PL>;
-    o.prepare = &pilot_prepare_impl<PL, MINB>;
-    o.launch = &pilot_launch_impl<PL, MINB>;
-    return o;
-}
-
 // Multi-user data kernel (lsmrc_mu_data): users per pass.  Each thread keeps UG * P complex sums in registers next to the
 // FFT working set: the most that compiles without spills (-Xptxas -v) -- two users for the 32-point plans of 1024 and
 // 4096 points (128 registers of sums), one for 512 and 2048 (two spill there), four at 16 points, eight at 8.  Larger
 // U re-runs the row transforms once per group of UG users (DESIGN.md 8e).  The soft epilogue (SOFT) compiles without
 // spills at the same UG on every plan (DESIGN.md 8f).
-template <class PL, bool SOFT = false>
+template <class PL>
 constexpr int mu_ug() { return PL::P >= 32 ? ((PL::N == 512 || PL::N == 2048) ? 1 : 2) : (PL::P >= 16 ? 4 : 8); }
 
 template <class PL>
 constexpr size_t mu_smem() { return sizeof(float2) * (size_t)(PL::TWN + PL::TEAMS * PL::TEAM_STRIDE); }
 
-template <class PL, bool SOFT>
-cudaError_t mu_prepare_impl(int* ctas_per_sm)
+template <class PL>
+cudaError_t mu_prepare_impl(bool soft, int* ctas_per_sm)
 {
-    constexpr int UG = mu_ug<PL, SOFT>();
-    cudaError_t e = cudaFuncSetAttribute(lsmrc_mu_data<PL, UG, SOFT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mu_smem<PL>());
+    constexpr int UG = mu_ug<PL>();
+    const auto kernel = soft ? lsmrc_mu_data<PL, UG, true> : lsmrc_mu_data<PL, UG, false>;
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mu_smem<PL>());
     if (e != cudaSuccess) return e;
-    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas_per_sm, lsmrc_mu_data<PL, UG, SOFT>, PL::THREADS, mu_smem<PL>());
+    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas_per_sm, kernel, PL::THREADS, mu_smem<PL>());
 }
 
-// max_ctas: resident CTAs of lsmrc_mu_data on the whole GPU (mu_prepare_impl x SMs)
-template <class PL, bool SOFT>
-cudaError_t mu_launch_impl(const KernelParams& p, const float2* hzf, float2* wd, const float2* soft_tab, int n_users, int max_ctas, int n_sms,
-                           cudaStream_t st)
+// max_ctas: resident CTAs of the (hard or soft) lsmrc_mu_data on the whole GPU (mu_prepare_impl x SMs)
+template <class PL>
+cudaError_t mu_launch_impl(bool soft, const KernelParams& p, const float2* hzf, float2* wd, const float2* soft_tab, int n_users, int max_ctas,
+                           int n_sms, cudaStream_t st)
 {
-    constexpr int UG = mu_ug<PL, SOFT>();
+    constexpr int UG = mu_ug<PL>();
     const int groups = (n_users + UG - 1) / UG;
     cudaError_t e;
     const long long rows = (long long)p.n_frames * groups * UG * p.n_ant;
@@ -403,7 +351,8 @@ cudaError_t mu_launch_impl(const KernelParams& p, const float2* hzf, float2* wd,
     const long long items = (long long)p.n_frames * groups * p.n_sym_work;
     long long grid = (items + PL::TEAMS - 1) / PL::TEAMS;
     if (grid > max_ctas) grid = max_ctas;
-    lsmrc_mu_data<PL, UG, SOFT><<<(unsigned)grid, PL::THREADS, mu_smem<PL>(), st>>>(p, wd, n_users, groups, soft_tab);
+    if (soft) lsmrc_mu_data<PL, UG, true><<<(unsigned)grid, PL::THREADS, mu_smem<PL>(), st>>>(p, wd, n_users, groups, soft_tab);
+    else lsmrc_mu_data<PL, UG, false><<<(unsigned)grid, PL::THREADS, mu_smem<PL>(), st>>>(p, wd, n_users, groups, soft_tab);
     return cudaGetLastError();
 }
 
@@ -424,17 +373,14 @@ PlanOps make_ops()
     o.prepare = &prepare_impl<PL, MINB>;
     o.launch = &launch_impl<PL, MINB>;
     o.launch_fused = PL::SH > 1 ? &launch_fused_impl<PL, MINB> : nullptr;
-    o.mu_ug = mu_ug<PL, false>();
-    o.mu_soft_ug = mu_ug<PL, true>();
-    o.mu_prepare = &mu_prepare_impl<PL, false>;
-    o.mu_soft_prepare = &mu_prepare_impl<PL, true>;
-    o.mu_launch = &mu_launch_impl<PL, false>;
-    o.mu_soft_launch = &mu_launch_impl<PL, true>;
+    o.mu_ug = mu_ug<PL>();
+    o.mu_prepare = &mu_prepare_impl<PL>;
+    o.mu_launch = &mu_launch_impl<PL>;
     return o;
 }
 
 // ---- the plans.  Template arguments: N, P (points per thread), R2, R3, teams per CTA, tile buffers per team, rows of
-// x prefetched to L2, rows of Hconj prefetched to L1, register prefetch of the next row, x through L1, Hconj ring,
+// x prefetched to L2, rows of Hconj prefetched to L1, register prefetch of the next row, Hconj ring,
 // x rows by bulk copy, stage-1 twiddles in tensor memory, lanes of the shuffle stage.  Each setting is the measured
 // winner of its A/B (DESIGN.md section 3 keeps the log, including the variants that lost and were deleted).
 // (64 points: 8 threads x 8 points per row.  16 x 4 -- teams of 4 threads reading 32 contiguous bytes per load, 8 lines per
@@ -444,9 +390,9 @@ using Plan64 = Plan<64, 8, 8, 1, 8, 2, 1, 1, 0>;  // (next sample row prefetched
 using Plan128 = Plan<128, 16, 8, 1, 16, 2, 0, 0, 1>;  // (8 x 4 x 4, three stages with 128-byte team loads: 25-30 % slower; L2/L1 prefetches: -1..-9 %)
 using Plan256 = Plan<256, 16, 16, 1, 8, 2, 1, 1, 1>;  // (+ L2 prefetch of the sample row after next: +7 %)
 using Plan512 = Plan<512, 32, 16, 1, 8, 1, 1, 1>;  // (tensor-memory twiddles measured 10 % slower here: teams of 16 threads)
-using Plan1024 = Plan<1024, 32, 32, 1, 4, 1, 0, 1, 0, false, true, true, true>;
-using Plan2048 = Plan<2048, 32, 32, 1, 2, 1, 1, 0, 0, false, false, false, true, 2>;
-using Plan4096 = Plan<4096, 32, 32, 1, 1, 1, 1, 0, 0, false, false, false, true, 4>;
+using Plan1024 = Plan<1024, 32, 32, 1, 4, 1, 0, 1, 0, true, true, true>;
+using Plan2048 = Plan<2048, 32, 32, 1, 2, 1, 1, 0, 0, false, false, true, 2>;
+using Plan4096 = Plan<4096, 32, 32, 1, 1, 1, 1, 0, 0, false, false, true, 4>;
 constexpr int kMinBlocks = 3;  // 3 CTAs (12 warps) per SM at 168 registers: measured best for every size
 
 // LSMRC_ONLY_N=<size> (development): instantiate the kernels of one FFT size only -- a full build takes 85 s
@@ -484,14 +430,6 @@ const PlanOps* find_plan(int N)
     };
     for (const PlanOps& o : plans)
         if (o.N == N) return &o;
-    return nullptr;
-}
-
-// Dedicated pilot plans (sizes not listed use the main plan's MODE_PILOT instantiation).  Only for plans whose
-// channel rows are in bin order: the shuffle-stage plans need the pilot kernel to share their slot layout.
-const PilotOps* find_pilot_plan(int N)
-{
-    (void)N;  // (none at present: the plans whose pilot kernel had its own are now shuffle-stage plans)
     return nullptr;
 }
 
@@ -575,9 +513,6 @@ struct lsmrc_ctx {
     const PlanOps* ops = nullptr;
     const OneshotOps* one_ops = nullptr;  // one-launch kernel (own plan, own twiddle table)
     float2* d_one_tw = nullptr;
-    const PilotOps* pilot_ops = nullptr;  // dedicated pilot plan (own twiddle table) or nullptr: use ops
-    float2* d_pilot_tw = nullptr;
-    int pilot_teams = 1;                  // teams per CTA of whichever plan runs the pilot kernel
     int max_data_ctas = 1;  // persistent data-kernel grid: resident CTAs per SM x SM count
     int pilot_wave = 1;     // pilot-kernel CTAs resident at once on the whole GPU
     int n_sms = 1;
@@ -725,7 +660,7 @@ void free_chan(ChanState& c)
 // amortised -- unless the launch is tiny (latency configs), where every antenna gets its own team
 int pilot_groups(const lsmrc_ctx* h, int n_frames)
 {
-    const int teams = h->pilot_teams;
+    const int teams = h->ops->teams;
     const int max_g = (h->cfg.n_ant + teams - 1) / teams;
     const int min_rows = ((long long)n_frames * 4 >= h->pilot_wave) ? 16 : 1;
     int g_rows = h->cfg.n_ant / (teams * min_rows);
@@ -736,6 +671,13 @@ int pilot_groups(const lsmrc_ctx* h, int n_frames)
     if ((long long)g * n_frames > (long long)n_frames + kPilotCtaTarget) g = (int)(((long long)n_frames + kPilotCtaTarget) / n_frames);
     if (g < 1) g = 1;
     return g;
+}
+
+// bulk async copies of antenna rows need 16-byte aligned rows: even strides and prefix, aligned base
+int rows_16b_aligned(const KernelParams& p)
+{
+    return (reinterpret_cast<uintptr_t>(p.rx) % 16 == 0) && p.cp % 2 == 0 && p.ant_stride % 2 == 0 && p.sym_stride % 2 == 0 &&
+           p.frame_stride % 2 == 0;
 }
 
 int launch_pilot(lsmrc_ctx* h, cudaStream_t st, KernelParams p, ChanState& ch, float2* d_hconj, float* d_hsqrd)
@@ -750,29 +692,22 @@ int launch_pilot(lsmrc_ctx* h, cudaStream_t st, KernelParams p, ChanState& ch, f
     // packed grid still fills the GPU
     p.frames_per_cta = 1;
     if (p.n_groups == 1) {
-        int fpc = h->pilot_teams / h->cfg.n_ant;
+        int fpc = h->ops->teams / h->cfg.n_ant;
         while (fpc > 1 && (p.n_frames + fpc - 1) / fpc < h->pilot_wave) --fpc;
         if (fpc > 1) p.frames_per_cta = fpc;
     }
     p.epart = ch.epart;
     p.counters = ch.counters;
-    // bulk async copies of antenna rows need 16-byte aligned rows: even strides and prefix, aligned base
-    p.x_tma = (reinterpret_cast<uintptr_t>(p.rx) % 16 == 0) && p.cp % 2 == 0 && p.ant_stride % 2 == 0 && p.sym_stride % 2 == 0 &&
-              p.frame_stride % 2 == 0;
+    p.x_tma = rows_16b_aligned(p);
     {
         // tiny virtual CTAs (a round or two of row FFTs per team: few antennas, small N) amortise the per-CTA setup by
         // striding one resident wave of CTAs over them; larger ones are left to the hardware scheduler, which
         // balances them better than a static stride
-        const int tpf = h->pilot_teams / p.frames_per_cta;
+        const int tpf = h->ops->teams / p.frames_per_cta;
         const int rounds = (h->cfg.n_ant + p.n_groups * tpf - 1) / (p.n_groups * tpf);
         p.pilot_grid_cap = rounds <= 2 ? h->pilot_wave : 0;
     }
-    if (h->pilot_ops) {
-        p.twiddles = h->d_pilot_tw;
-        CK(h, h->pilot_ops->launch(p, st));
-    } else {
-        CK(h, h->ops->launch(MODE_PILOT, p, st, h->max_data_ctas, nullptr, nullptr));
-    }
+    CK(h, h->ops->launch(MODE_PILOT, p, st, h->max_data_ctas));
     h->launches++;
     return LSMRC_OK;
 }
@@ -784,11 +719,9 @@ int launch_data(lsmrc_ctx* h, cudaStream_t st, KernelParams p, ChanState& ch, fl
     p.hwork = ch.hwork;
     p.hsqrd = d_hsqrd ? d_hsqrd : ch.hsqrd;
     p.n_groups = 1;
-    // bulk async copies of antenna rows (X_TMA plans) need 16-byte aligned rows: even strides and prefix, aligned base
-    p.x_tma = (reinterpret_cast<uintptr_t>(p.rx) % 16 == 0) && p.cp % 2 == 0 && p.ant_stride % 2 == 0 && p.sym_stride % 2 == 0 &&
-              p.frame_stride % 2 == 0;
+    p.x_tma = rows_16b_aligned(p);
     p.ticket = ch.ticket;
-    CK(h, h->ops->launch(MODE_DATA, p, st, h->max_data_ctas, nullptr, nullptr));
+    CK(h, h->ops->launch(MODE_DATA, p, st, h->max_data_ctas));
     h->launches++;
     return LSMRC_OK;
 }
@@ -798,12 +731,12 @@ int launch_data(lsmrc_ctx* h, cudaStream_t st, KernelParams p, ChanState& ch, fl
 int launch_fused(lsmrc_ctx* h, cudaStream_t st, KernelParams p, ChanState& ch, float2* d_hconj, float* d_hsqrd, cudaEvent_t ev_before)
 {
     const lsmrc_config& c = h->cfg;
-    if (!h->ops->launch_fused || !h->one_launch_frames || h->pilot_ops || c.n_sym < 2) return 0;
+    if (!h->ops->launch_fused || !h->one_launch_frames || c.n_sym < 2) return 0;
     const int teams = h->ops->teams;
     const long long n_work = (long long)p.n_frames * (c.n_sym - 1);
     if ((n_work + teams - 1) / teams < (long long)h->max_data_ctas) return 0;  // (smaller batches: antenna split / wider pilot grid)
     p.n_groups = pilot_groups(h, p.n_frames);
-    if (p.n_groups == 1 && h->pilot_teams / c.n_ant > 1) return 0;             // (few antennas: the pilot kernel packs frames)
+    if (p.n_groups == 1 && teams / c.n_ant > 1) return 0;                        // (few antennas: the pilot kernel packs frames)
     p.first_sym = 1;
     p.n_sym_work = c.n_sym - 1;
     p.hwork = ch.hwork;
@@ -816,8 +749,7 @@ int launch_fused(lsmrc_ctx* h, cudaStream_t st, KernelParams p, ChanState& ch, f
     p.ticket = ch.ticket;
     p.ready = ch.ready;
     p.ant_split = 1;
-    p.x_tma = (reinterpret_cast<uintptr_t>(p.rx) % 16 == 0) && p.cp % 2 == 0 && p.ant_stride % 2 == 0 && p.sym_stride % 2 == 0 &&
-              p.frame_stride % 2 == 0;
+    p.x_tma = rows_16b_aligned(p);
     if (ev_before) CK(h, cudaEventRecord(ev_before, st));  // (no separate pilot phase: the split reported is 0 / whole)
     CK(h, h->ops->launch_fused(p, st, h->max_data_ctas));
     h->launches++;
@@ -877,28 +809,19 @@ int launch_frames(lsmrc_ctx* h, cudaStream_t st, const float2* d_rx, int n_frame
         CK(h, h->one_ops->launch(p, st));
         h->launches++;
         h->oneshot_calls++;
-        if (timed) {
-            CK(h, cudaEventRecord(ev[2], st));
-            h->ev_calls++;
+    } else {
+        if (lay) return fail(h, LSMRC_ERR_STATE, "in-place ring layout without the one-launch kernel");
+        int rc = launch_fused(h, st, p, ch, d_hconj, d_hsqrd, timed ? ev[1] : nullptr);
+        if (rc < 0) return rc;
+        if (rc == 0) {  // (1: channel estimate and data symbols of the whole batch went out as one persistent launch)
+            rc = launch_pilot(h, st, p, ch, d_hconj, d_hsqrd);
+            if (rc != LSMRC_OK) return rc;
+            if (timed) CK(h, cudaEventRecord(ev[1], st));
+            if (h->cfg.n_sym > 1) {
+                rc = launch_data(h, st, p, ch, d_hsqrd, 1, h->cfg.n_sym - 1);
+                if (rc != LSMRC_OK) return rc;
+            }
         }
-        return LSMRC_OK;
-    }
-    if (lay) return fail(h, LSMRC_ERR_STATE, "in-place ring layout without the one-launch kernel");
-    int rc = launch_fused(h, st, p, ch, d_hconj, d_hsqrd, timed ? ev[1] : nullptr);
-    if (rc < 0) return rc;
-    if (rc == 1) {  // channel estimate and data symbols of the whole batch went out as one persistent launch
-        if (timed) {
-            CK(h, cudaEventRecord(ev[2], st));
-            h->ev_calls++;
-        }
-        return LSMRC_OK;
-    }
-    rc = launch_pilot(h, st, p, ch, d_hconj, d_hsqrd);
-    if (rc != LSMRC_OK) return rc;
-    if (timed) CK(h, cudaEventRecord(ev[1], st));
-    if (h->cfg.n_sym > 1) {
-        rc = launch_data(h, st, p, ch, d_hsqrd, 1, h->cfg.n_sym - 1);
-        if (rc != LSMRC_OK) return rc;
     }
     if (timed) {
         CK(h, cudaEventRecord(ev[2], st));
@@ -1110,6 +1033,17 @@ int ensure_scratch(lsmrc_ctx* h, T*& ptr, size_t& cap, size_t bytes, cudaStream_
     return LSMRC_OK;
 }
 
+// a plan's twiddle table (twn entries, written by fill) into a new device buffer
+int upload_twiddles(lsmrc_ctx* h, void (*fill)(float2*), int twn, float2** d_tw)
+{
+    std::vector<float2> tw((size_t)twn);
+    fill(tw.data());
+    cudaError_t e;
+    if ((e = cudaMalloc(d_tw, tw.size() * sizeof(float2))) != cudaSuccess) return fail_cuda(h, e, "cudaMalloc twiddles");
+    if ((e = cudaMemcpy(*d_tw, tw.data(), tw.size() * sizeof(float2), cudaMemcpyHostToDevice)) != cudaSuccess) return fail_cuda(h, e, "cudaMemcpy twiddles");
+    return LSMRC_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1220,18 +1154,6 @@ int lsmrc_create(const lsmrc_config* cfg, lsmrc_handle* out)
         if (per_sm < 1 || pilot_per_sm < 1) { h->err = "kernel does not fit on an SM"; return bail(LSMRC_ERR_CUDA); }
         h->max_data_ctas = per_sm * prop.multiProcessorCount;
         h->pilot_wave = pilot_per_sm * prop.multiProcessorCount;
-        h->pilot_teams = ops->teams;
-        if ((h->pilot_ops = find_pilot_plan(cfg->fft_size)) != nullptr) {
-            int pp = 0;
-            if ((e = h->pilot_ops->prepare(&pp)) != cudaSuccess) { fail_cuda(h, e, "cudaFuncSetAttribute (pilot plan)"); return bail(LSMRC_ERR_CUDA); }
-            if (pp < 1) { h->err = "pilot kernel does not fit on an SM"; return bail(LSMRC_ERR_CUDA); }
-            h->pilot_wave = pp * prop.multiProcessorCount;
-            h->pilot_teams = h->pilot_ops->teams;
-            std::vector<float2> twp((size_t)h->pilot_ops->twn);
-            h->pilot_ops->fill_twiddles(twp.data());
-            if ((e = cudaMalloc(&h->d_pilot_tw, twp.size() * sizeof(float2))) != cudaSuccess) { fail_cuda(h, e, "cudaMalloc twiddles"); return bail(LSMRC_ERR_CUDA); }
-            if ((e = cudaMemcpy(h->d_pilot_tw, twp.data(), twp.size() * sizeof(float2), cudaMemcpyHostToDevice)) != cudaSuccess) { fail_cuda(h, e, "cudaMemcpy twiddles"); return bail(LSMRC_ERR_CUDA); }
-        }
         h->n_sms = prop.multiProcessorCount;
         h->smem_optin = prop.sharedMemPerBlockOptin;
     }
@@ -1239,10 +1161,7 @@ int lsmrc_create(const lsmrc_config* cfg, lsmrc_handle* out)
     for (int i = 0; i < lsmrc_ctx::kEvRing; ++i)
         for (int j = 0; j < 3; ++j)
             if ((e = cudaEventCreate(&h->ev[i][j])) != cudaSuccess) { fail_cuda(h, e, "cudaEventCreate"); return bail(LSMRC_ERR_CUDA); }
-    std::vector<float2> tw((size_t)ops->twn);
-    ops->fill_twiddles(tw.data());
-    if ((e = cudaMalloc(&h->d_tw, tw.size() * sizeof(float2))) != cudaSuccess) { fail_cuda(h, e, "cudaMalloc twiddles"); return bail(LSMRC_ERR_CUDA); }
-    if ((e = cudaMemcpy(h->d_tw, tw.data(), tw.size() * sizeof(float2), cudaMemcpyHostToDevice)) != cudaSuccess) { fail_cuda(h, e, "cudaMemcpy twiddles"); return bail(LSMRC_ERR_CUDA); }
+    if (upload_twiddles(h, ops->fill_twiddles, ops->twn, &h->d_tw) != LSMRC_OK) return bail(LSMRC_ERR_CUDA);
     if (const char* ev = std::getenv("LSMRC_H2D_STRIP_MIN_ROW")) {  // tuning/A-B knob
         const long v = std::atol(ev);
         h->h2d_strip_cp = v > 0;
@@ -1251,10 +1170,7 @@ int lsmrc_create(const lsmrc_config* cfg, lsmrc_handle* out)
     if ((h->one_ops = find_oneshot_plan(cfg->fft_size)) != nullptr) {
         const OneshotOps* oo = h->one_ops;
         if ((e = oo->prepare((int)prop.sharedMemPerBlockOptin)) != cudaSuccess) { fail_cuda(h, e, "cudaFuncSetAttribute (one-launch kernel)"); return bail(LSMRC_ERR_CUDA); }
-        std::vector<float2> tw1((size_t)oo->twn);
-        oo->fill_twiddles(tw1.data());
-        if ((e = cudaMalloc(&h->d_one_tw, tw1.size() * sizeof(float2))) != cudaSuccess) { fail_cuda(h, e, "cudaMalloc twiddles"); return bail(LSMRC_ERR_CUDA); }
-        if ((e = cudaMemcpy(h->d_one_tw, tw1.data(), tw1.size() * sizeof(float2), cudaMemcpyHostToDevice)) != cudaSuccess) { fail_cuda(h, e, "cudaMemcpy twiddles"); return bail(LSMRC_ERR_CUDA); }
+        if (upload_twiddles(h, oo->fill_twiddles, oo->twn, &h->d_one_tw) != LSMRC_OK) return bail(LSMRC_ERR_CUDA);
     }
     if ((e = cudaMalloc(&h->d_pilot_bin, (size_t)h->K * sizeof(float2))) != cudaSuccess) { fail_cuda(h, e, "cudaMalloc pilot"); return bail(LSMRC_ERR_CUDA); }
     // zero forcing: allow the largest tile once (see launch_zf_create)
@@ -1277,7 +1193,6 @@ int lsmrc_destroy(lsmrc_handle h)
     for (Lane& L : h->lanes) free_lane(L);
     cudaFree(h->d_tw);
     cudaFree(h->d_one_tw);
-    cudaFree(h->d_pilot_tw);
     cudaFree(h->d_noise_part);
     cudaFree(h->d_hit);
     cudaFree(h->d_pilot_bin);
@@ -1385,16 +1300,16 @@ int mu_check(lsmrc_ctx* h, const void* d_rx, const void* d_combined, int n_frame
     return LSMRC_OK;
 }
 
-// Phases 1-2 on stream st for n_frames >= 1.  UG: users per pass of the data kernel that follows (Wd is sized for it);
-// ginv_diag (nullptr unless soft output is wanted) receives inv(G)'s diagonal [F][U][K].  On return p holds the data
-// kernel's parameters except its outputs.
-int mu_detect(lsmrc_ctx* h, cudaStream_t st, const void* d_rx, int n_frames, int n_users, int detector, float noise_var, int UG,
-              bool count, bool soft, KernelParams& p)
+// Phases 1-2 on stream st for n_frames >= 1.  Wd is sized for the plan's users per pass of the data kernel (mu_ug);
+// with `soft`, ginv_diag receives inv(G)'s diagonal [F][U][K].  On return p holds the data kernel's parameters except
+// its outputs.
+int mu_detect(lsmrc_ctx* h, cudaStream_t st, const void* d_rx, int n_frames, int n_users, int detector, float noise_var, bool count,
+              bool soft, KernelParams& p)
 {
     const int A = h->cfg.n_ant, S = h->cfg.n_sym, N = h->cfg.fft_size, K = h->K;
     const int kt = zf_tile(h, A, n_users);
     if (kt < 1) return fail(h, LSMRC_ERR_UNSUPPORTED, "n_ant * n_users too large for one CTA's shared memory");
-    const int U = n_users, UP = (U + UG - 1) / UG * UG;
+    const int U = n_users, UG = h->ops->mu_ug, UP = (U + UG - 1) / UG * UG;
     const long long F = n_frames;
     int rc;
     if ((rc = ensure_chan(h, h->mu_ch, n_frames, st)) != LSMRC_OK) return rc;
@@ -1407,7 +1322,7 @@ int mu_detect(lsmrc_ctx* h, cudaStream_t st, const void* d_rx, int n_frames, int
     int& max_ctas = soft ? h->mu_soft_max_ctas : h->mu_max_ctas;
     if (max_ctas == 0) {
         int per_sm = 0;
-        CK(h, (soft ? h->ops->mu_soft_prepare : h->ops->mu_prepare)(&per_sm));
+        CK(h, h->ops->mu_prepare(soft, &per_sm));
         if (per_sm < 1) return fail(h, LSMRC_ERR_CUDA, "multi-user data kernel does not fit on an SM");
         max_ctas = per_sm * h->n_sms;
     }
@@ -1465,12 +1380,12 @@ int lsmrc_demod_frames_device_mu(lsmrc_handle h, const void* d_rx, int n_frames,
     CK(h, cudaSetDevice(h->cfg.device));
     cudaStream_t st = compute_stream(h);
     KernelParams p;
-    if ((rc = mu_detect(h, st, d_rx, n_frames, n_users, detector, noise_var, h->ops->mu_ug, n_singular != nullptr, false, p)) != LSMRC_OK)
+    if ((rc = mu_detect(h, st, d_rx, n_frames, n_users, detector, noise_var, n_singular != nullptr, false, p)) != LSMRC_OK)
         return rc;
     // 3. detection fused with the row FFT of every data symbol
     p.combined = static_cast<float2*>(d_combined);
     p.bits = static_cast<uint8_t*>(d_bits);
-    CK(h, h->ops->mu_launch(p, h->d_mu_hzf, h->d_mu_wd, nullptr, n_users, h->mu_max_ctas, h->n_sms, st));
+    CK(h, h->ops->mu_launch(false, p, h->d_mu_hzf, h->d_mu_wd, nullptr, n_users, h->mu_max_ctas, h->n_sms, st));
     h->launches += 2;
     return mu_finish(h, st, n_frames, n_users, d_hconj, n_singular);
 }
@@ -1489,7 +1404,7 @@ int lsmrc_demod_frames_device_mu_soft(lsmrc_handle h, const void* d_rx, int n_fr
     CK(h, cudaSetDevice(h->cfg.device));
     cudaStream_t st = compute_stream(h);
     KernelParams p;
-    if ((rc = mu_detect(h, st, d_rx, n_frames, n_users, detector, noise_var, h->ops->mu_soft_ug, n_singular != nullptr, true, p)) != LSMRC_OK)
+    if ((rc = mu_detect(h, st, d_rx, n_frames, n_users, detector, noise_var, n_singular != nullptr, true, p)) != LSMRC_OK)
         return rc;
     // 3a. (rho, scale) per (frame, user, subcarrier) from the diagonal of inv(G)
     const long long n = (long long)n_frames * n_users * h->K;
@@ -1504,7 +1419,7 @@ int lsmrc_demod_frames_device_mu_soft(lsmrc_handle h, const void* d_rx, int n_fr
     p.combined = static_cast<float2*>(d_combined);
     p.bits = static_cast<uint8_t*>(d_bits);
     p.llr = static_cast<float*>(d_llr);
-    CK(h, h->ops->mu_soft_launch(p, h->d_mu_hzf, h->d_mu_wd, tab, n_users, h->mu_soft_max_ctas, h->n_sms, st));
+    CK(h, h->ops->mu_launch(true, p, h->d_mu_hzf, h->d_mu_wd, tab, n_users, h->mu_soft_max_ctas, h->n_sms, st));
     h->launches += 2;
     return mu_finish(h, st, n_frames, n_users, d_hconj, n_singular);
 }
@@ -2045,7 +1960,7 @@ int lsmrc_stage_fft(lsmrc_handle h, void* d_rows, long long rows)
     p.ant_stride = h->cfg.fft_size;
     p.cp = 0;
     p.n_frames = (int)rows;
-    CK(h, h->ops->launch(MODE_FFT, p, compute_stream(h), h->max_data_ctas, nullptr, nullptr));
+    CK(h, h->ops->launch(MODE_FFT, p, compute_stream(h), h->max_data_ctas));
     h->launches++;
     return LSMRC_OK;
 }

@@ -60,7 +60,7 @@ struct KernelParams {
     // the ring).  split_sym = INT_MAX: ordinary addressing through frame_stride.
     const float2* rx2;
     int split_sym;
-    int x_tma;      // data kernel, X_TMA plans: antenna rows are 16-byte aligned, bulk copies allowed
+    int x_tma;      // antenna rows are 16-byte aligned: bulk copies allowed
     int rx_align4;  // one-launch kernel only: samples are only 4-byte aligned (slots behind the ring's 12-byte header)
     long long frame_stride;
     long long sym_stride;
@@ -107,7 +107,7 @@ struct KernelParams {
     const float2* twiddles;  // plan table: tw1 [(P-1)][T] then tw2 [(R2-1)][R3]
 };
 
-template <int N_, int P_, int R2_, int R3_, int TEAMS_, int NBUF_ = 2, int PF_X_ = 0, int PF_H_ = 0, int REG_PF_ = 0, bool X_L1_ = false, bool H_RING_ = false,
+template <int N_, int P_, int R2_, int R3_, int TEAMS_, int NBUF_ = 2, int PF_X_ = 0, int PF_H_ = 0, int REG_PF_ = 0, bool H_RING_ = false,
           bool X_TMA_ = false, bool TW_TMEM_ = false, int SH_ = 1>
 struct Plan {
     // SH > 1 (2 or 4; N = 32 * 32 * SH, teams of SH warps): the LAST radix-SH stage runs across the SH adjacent lanes
@@ -136,8 +136,6 @@ struct Plan {
     // REG_PF: data kernel loads row a+1 into registers right after stage 1 of row a (0 = off, 1 = on).  Pays for the
     // 16-points-per-thread plans; the 32-point plans would need a 255-register budget.
     static constexpr int REG_PF = REG_PF_;
-    // X_L1: prefetch the antenna-samples into L1 (and load them with L1 allocation) instead of L2
-    static constexpr bool X_L1 = X_L1_;
     // H_RING: the TEAMS teams of a CTA work on TEAMS data symbols of ONE frame and share each
     // Hconj row through a shared-memory ring filled by bulk async copies (TMA) on mbarriers
     static constexpr bool H_RING = H_RING_;
@@ -161,6 +159,7 @@ struct Plan {
     static __device__ __forceinline__ int at(int r, int c) { return r * ROW + (c ^ swz(r)); }
     static_assert(!X_TMA_ || (NBUF_ == 1 && N_ / P_ >= 16), "X_TMA: one tile per team, teams of at least half a warp");
     static_assert(!X_TMA_ || ((P_ * (N_ / P_ + 1)) % 2 == 0), "X_TMA: team tiles must stay 16-byte aligned");
+    static_assert(!X_TMA_ || H_RING_, "X_TMA: the data kernel sets up the row barriers with the Hconj ring's");
     static constexpr int NB2 = P / R2;     // stage-2 butterflies per thread
     static constexpr int NB3 = P / R3;     // stage-3 butterflies per thread (R3 > 1)
     static constexpr int RL = (R3 > 1) ? R3 : R2;  // radix of the last shared-memory stage
@@ -442,7 +441,7 @@ __device__ __forceinline__ void row_load(float2 (&v)[PL::P], const float2* __res
 {
 #pragma unroll
     for (int n1 = 0; n1 < PL::P; ++n1) {
-        v[n1] = PL::X_L1 ? __ldg(x + n1 * PL::T + t) : ld_stream(x + n1 * PL::T + t);
+        v[n1] = ld_stream(x + n1 * PL::T + t);
     }
 }
 
@@ -800,6 +799,24 @@ __device__ __forceinline__ void row_fft(float2 (&v)[PL::P], const float2* __rest
     if constexpr (PL::NBUF == 1) team_sync<PL>(team);
 }
 
+// Bit packing of one row by a team: the K demapped symbols in s_idx, b bits each, as one bit stream (bit j of the row =
+// bit j % b of symbol j / b) into bit j % 8 of byte j / 8.  Nothing is stored unless `store`.
+template <class PL>
+__device__ __forceinline__ void pack_bits(const uint8_t* s_idx, uint8_t* bits_row, int row_bytes, int b, bool store, int t)
+{
+    constexpr int K = PL::N - 1;
+    for (int byte = t; byte < row_bytes; byte += PL::T) {
+        unsigned v8 = 0;
+#pragma unroll
+        for (int q = 0; q < 8; ++q) {
+            const int pos = byte * 8 + q;
+            const int sym = pos / b, bit = pos - sym * b;
+            if (sym < K) v8 |= ((s_idx[sym] >> bit) & 1u) << q;
+        }
+        if (store) bits_row[byte] = (uint8_t)v8;
+    }
+}
+
 // Epilogue of one (frame, data symbol) held by a team: normalise (cpuLS.hpp:364-367), reorder to
 // ascending frequency (cpuLS.hpp:135-149), demap, pack, optional LLRs.  acc[sl] is the MRC sum of
 // the bin the thread owns in slot sl; e_row[bin - 1] = sum_a |H|^2 (global, or shared when
@@ -809,7 +826,7 @@ template <class PL, bool E_SHARED, bool E_CG = false>
 __device__ __forceinline__ void mrc_finish(const KernelParams& p, const float2 (&acc)[PL::P], const float* __restrict__ e_row,
                                            int f, int s, uint8_t* s_idx, bool valid, int t, int team)
 {
-    constexpr int N = PL::N, P = PL::P, T = PL::T, K = N - 1;
+    constexpr int N = PL::N, P = PL::P, K = N - 1;
     float2* out_row = p.combined + ((long long)f * p.n_sym_work + s) * K;
     uint8_t* bits_row = p.bits ? p.bits + ((long long)f * p.n_sym_work + s) * p.bits_row_bytes : nullptr;
     float* llr_row = p.llr ? p.llr + ((long long)f * p.n_sym_work + s) * K * p.qam_bits : nullptr;
@@ -844,22 +861,35 @@ __device__ __forceinline__ void mrc_finish(const KernelParams& p, const float2 (
         }
         if (bits_row != nullptr) {
             team_sync<PL>(team);
-            for (int byte = t; byte < p.bits_row_bytes; byte += T) {
-                unsigned v8 = 0;
-#pragma unroll
-                for (int q = 0; q < 8; ++q) {
-                    const int pos = byte * 8 + q;
-                    const int sym = pos / b, bit = pos - sym * b;
-                    if (sym < K) v8 |= ((s_idx[sym] >> bit) & 1u) << q;
-                }
-                if (valid) bits_row[byte] = (uint8_t)v8;
-            }
+            pack_bits<PL>(s_idx, bits_row, p.bits_row_bytes, b, valid, t);
         }
     };
     if (p.qam_bits == 2) finish(std::integral_constant<int, 2>{});
     else if (p.qam_bits == 4) finish(std::integral_constant<int, 4>{});
     else finish(std::integral_constant<int, 6>{});
 }
+
+// LS divide of the generic pilot paths (pilot kernel, one-launch kernel), per slot of the thread: the pilot value of
+// the slot's bin (load) and 1/|X|^2 (recip), hoisted out of the per-element divide of cpuLS.hpp:240-241 (<= 1 ulp apart).
+template <class PL>
+struct LsDivide {
+    float2 xp[PL::P];
+    float xden[PL::P];
+    __device__ __forceinline__ void load(const KernelParams& p, int sl, int t)
+    {
+        const int bin = PL::bin_of(sl, t);
+        xp[sl] = p.pilot_bin[bin > 0 ? bin - 1 : 0];
+    }
+    __device__ __forceinline__ void recip(int sl) { xden[sl] = 1.0f / (xp[sl].x * xp[sl].x + xp[sl].y * xp[sl].y); }
+    // the LS estimate H = Z / X of slot sl from its FFT output z (cpuLS.hpp:233-244); conj(H) is what gets stored
+    // (:303-307), |H|^2 = energy(H) what gets summed (cpuLS.hpp:211-228)
+    __device__ __forceinline__ float2 divide(int sl, float2 z) const
+    {
+        const float2 X = xp[sl];
+        return make_float2((z.x * X.x + z.y * X.y) * xden[sl], (z.y * X.x - z.x * X.y) * xden[sl]);
+    }
+    static __device__ __forceinline__ float energy(float2 h) { return h.x * h.x + h.y * h.y; }
+};
 
 // XT (data mode of X_TMA plans): antenna rows come in by bulk copy.  A compile-time switch, not a test of p.x_tma inside the
 // row loop: with both paths in one loop body ptxas schedules the common one 2 % slower (c2: 2.42 -> 2.36 ms per 256 frames).
@@ -910,13 +940,11 @@ __global__ void __launch_bounds__(PL::THREADS, MINB) lsmrc_kernel(const KernelPa
         const int fpc = p.frames_per_cta;
         const int tpf = PL::TEAMS / fpc;
         const int lf = team / tpf, tj = team % tpf;
-        float2 xp[P];   // pilot value per owned bin
-        float xden[P];  // 1/|X|^2, hoisted: cpuLS.hpp:240-241 divides by |X|^2 per element (<= 1 ulp apart)
+        LsDivide<PL> ls;
 #pragma unroll
         for (int sl = 0; sl < P; ++sl) {
-            const int bin = PL::bin_of(sl, t);
-            xp[sl] = p.pilot_bin[bin > 0 ? bin - 1 : 0];
-            xden[sl] = 1.0f / (xp[sl].x * xp[sl].x + xp[sl].y * xp[sl].y);
+            ls.load(p, sl, t);
+            ls.recip(sl);
         }
         const int n_virtual = ((p.n_frames + fpc - 1) / fpc) * p.n_groups;
         for (int vb = blockIdx.x; vb < n_virtual; vb += gridDim.x) {
@@ -945,18 +973,15 @@ __global__ void __launch_bounds__(PL::THREADS, MINB) lsmrc_kernel(const KernelPa
                 prefetch_row<T, false>(x0 + (long long)(a_raw + per_iter) * p.ant_stride, N, t);
             row_fft<PL>(v, nullptr, tile, s_tw1, s_tw2, t, team,
                         [&](int sl, int bin, float2 z) {
-                            // LS estimate, complex division of cpuLS.hpp:233-244, then conj (:303-307)
-                            const float2 X = xp[sl];
-                            const float re = (z.x * X.x + z.y * X.y) * xden[sl];
-                            const float im = (z.y * X.x - z.x * X.y) * xden[sl];
+                            const float2 H = ls.divide(sl, z);
                             if (a_ok) {
                                 // (shuffle-stage plans: z carries the unit factor of its slot, and so does the hc the
                                 // data kernel will multiply its equally factored outputs with; the exported copy is exact)
-                                const float2 hc = (bin > 0) ? make_float2(re, -im) : make_float2(0.f, 0.f);
+                                const float2 hc = (bin > 0) ? make_float2(H.x, -H.y) : make_float2(0.f, 0.f);
                                 hw_row[PL::hpos(sl, t, bin)] = hc;
                                 if (bin > 0) {
                                     if (hc_row) hc_row[bin - 1] = PL::refix(sl, t, hc);
-                                    e[sl] += re * re + im * im;  // cpuLS.hpp:211-228
+                                    e[sl] += ls.energy(H);
                                 }
                             }
                         });
@@ -1050,17 +1075,15 @@ __global__ void __launch_bounds__(PL::THREADS, MINB) lsmrc_kernel(const KernelPa
             else prefetch_row<T, false>(xd + (long long)ad * p.ant_stride, N, t);
         }
         float e[P];
-        float2 xp[P];
-        float xden[P];
+        LsDivide<PL> ls;
 #pragma unroll
         for (int sl = 0; sl < P; ++sl) {
-            const int bin = PL::bin_of(sl, t);
             e[sl] = 0.f;
-            xp[sl] = p.pilot_bin[bin > 0 ? bin - 1 : 0];
+            ls.load(p, sl, t);
         }
         for (int i = threadIdx.x; i < PL::TWN; i += PL::THREADS) smem[i] = p.twiddles[i];
 #pragma unroll
-        for (int sl = 0; sl < P; ++sl) xden[sl] = 1.0f / (xp[sl].x * xp[sl].x + xp[sl].y * xp[sl].y);
+        for (int sl = 0; sl < P; ++sl) ls.recip(sl);
         __syncthreads();
 
         // ---- channel estimate (same arithmetic as MODE_PILOT with one antenna group) ----
@@ -1077,17 +1100,15 @@ __global__ void __launch_bounds__(PL::THREADS, MINB) lsmrc_kernel(const KernelPa
             float2* hw_row = hw_frame + (long long)a * N;
             float2* hc_row = hc_frame ? hc_frame + (long long)a * K : nullptr;
             row_fft<PL>(v, nullptr, tile, s_tw1, s_tw2, t, team, [&](int sl, int bin, float2 z) {
-                const float2 X = xp[sl];
-                const float re = (z.x * X.x + z.y * X.y) * xden[sl];
-                const float im = (z.y * X.x - z.x * X.y) * xden[sl];
+                const float2 H = ls.divide(sl, z);
                 if (a_ok) {
-                    const float2 hc = (bin > 0) ? make_float2(re, -im) : make_float2(0.f, 0.f);
+                    const float2 hc = (bin > 0) ? make_float2(H.x, -H.y) : make_float2(0.f, 0.f);
                     sh_row[bin] = hc;  // (read back below by the same thread for the same slot: unit factors cancel)
                     if (writer) {
                         hw_row[PL::hpos(sl, t, bin)] = hc;
                         if (bin > 0 && hc_row) hc_row[bin - 1] = PL::refix(sl, t, hc);
                     }
-                    if (bin > 0) e[sl] += re * re + im * im;
+                    if (bin > 0) e[sl] += ls.energy(H);
                 }
             });
         }
@@ -1206,13 +1227,6 @@ __global__ void __launch_bounds__(PL::THREADS, MINB) lsmrc_kernel(const KernelPa
             }
             __syncthreads();
         }
-        if constexpr (PL::X_TMA && !PL::H_RING) {
-            if (threadIdx.x == 0) {
-                for (int i = 0; i < PL::TEAMS; ++i) mbar_init(&bar_x[i], 1);
-                mbar_fence_init();
-            }
-            __syncthreads();
-        }
         const int groups = (p.n_sym_work + PL::TEAMS - 1) / PL::TEAMS;
         const long long n_work = (long long)p.n_frames * p.n_sym_work;
         const int AS = PL::H_RING ? 1 : p.ant_split;     // teams sharing one (frame, symbol)
@@ -1284,11 +1298,10 @@ __global__ void __launch_bounds__(PL::THREADS, MINB) lsmrc_kernel(const KernelPa
 
         float2 v[P];
         if (PL::REG_PF != 0) row_load<PL>(v, x0 + (long long)(aj < p.n_ant ? aj : p.n_ant - 1) * p.ant_stride, t);  // this team's first antenna
-        // X_TMA: row a of this team's symbol arrives in the team's tile by bulk copy; row 0 is requested here,
-        // row a+1 from inside row a (see the hook below).  x_tma is off when rows are not 16-byte aligned.
-        static_assert(!XT || (PL::X_TMA && PL::H_RING), "bulk-copied rows: X_TMA plans whose teams never split a pair's antennas");
-        constexpr bool x_tma = XT;  // (the launcher picks the instantiation: rows 16-byte aligned or not)
-        if (PL::X_TMA && x_tma && t == 0) {
+        // XT: row a of this team's symbol arrives in the team's tile by bulk copy; row 0 is requested here,
+        // row a+1 from inside row a (see the hook below).  (The launcher picks XT only when rows are 16-byte aligned.)
+        static_assert(!XT || PL::X_TMA, "bulk-copied rows: X_TMA plans (whose teams never split a pair's antennas)");
+        if (XT && t == 0) {
             fence_proxy_async();  // the tile doubled as the previous item's demap byte buffer
             mbar_expect_tx(&bar_x[team], ROW_BYTES);
             bulk_g2s(my_tiles, x0, ROW_BYTES, &bar_x[team]);
@@ -1310,7 +1323,7 @@ __global__ void __launch_bounds__(PL::THREADS, MINB) lsmrc_kernel(const KernelPa
             if (PL::REG_PF != 0) {
                 if (a + AS < p.n_ant) x_next = x0 + (long long)(a + AS) * p.ant_stride;
             }
-            if (PL::X_TMA && x_tma) {
+            if (XT) {
                 mbar_wait(&bar_x[team], x_phase);
                 x_phase ^= 1u;
 #pragma unroll
@@ -1321,9 +1334,9 @@ __global__ void __launch_bounds__(PL::THREADS, MINB) lsmrc_kernel(const KernelPa
             }
             // L2 prefetch: one row ahead of the demand loads, or one row ahead of the next bulk copy
             // (X_TMA plans whose rows are not 16-byte aligned fall back to demand loads and always prefetch one row)
-            const int pf_rows = (PL::X_TMA && x_tma) ? (PF_X > 0 ? PF_X + 1 : 0) : (PL::X_TMA ? 1 : PF_X);
+            const int pf_rows = XT ? (PF_X > 0 ? PF_X + 1 : 0) : (PL::X_TMA ? 1 : PF_X);
             if (pf_rows > 0 && a + pf_rows * AS < p.n_ant)
-                prefetch_row<T, PL::X_L1>(x0 + (long long)(a + pf_rows * AS) * p.ant_stride, N, t);
+                prefetch_row<T, false>(x0 + (long long)(a + pf_rows * AS) * p.ant_stride, N, t);
             if (!PL::H_RING && PF_H > 0 && a + PF_H * AS < p.n_ant)
                 prefetch_row<T, true>(hw_row + (long long)PF_H * AS * N, N, t);
             const int R = rows_done + a;
@@ -1346,10 +1359,10 @@ __global__ void __launch_bounds__(PL::THREADS, MINB) lsmrc_kernel(const KernelPa
                         },
                         tmem,
                         [&]() {
-                            if constexpr (PL::X_TMA) {
+                            if constexpr (XT) {
                                 // the tile has been read for the last time in this row: fetch the next row
                                 // into it while the last-stage butterflies and the MRC run
-                                if (x_tma && a + 1 < p.n_ant) {
+                                if (a + 1 < p.n_ant) {
                                     team_sync<PL>(team);
                                     if (t == 0) {
                                         fence_proxy_async();
@@ -1594,15 +1607,14 @@ __device__ __forceinline__ void sh_setup(const KernelParams& p, ShRow<PL>& row, 
 }
 
 // draws the next ticket of a persistent kernel (thread 0) and hands it to the whole CTA; -1 when the launch has run out
-// of its n_tickets.  The last CTA to find the counter exhausted re-arms it for the next launch (and, when `epoch` is
-// given, advances the launch number that the fused kernel's ready flags carry).
-template <class F>
-__device__ __forceinline__ long long draw_ticket(const KernelParams& p, long long n_tickets, long long* s_ticket, bool with_epoch, F&& decode)
+// of its n_tickets.  The last CTA to find the counter exhausted re-arms it for the next launch (and, with `with_epoch`,
+// advances the launch number that the fused kernel's ready flags carry).
+template <class TK>
+__device__ __forceinline__ TK draw_ticket(const KernelParams& p, TK n_tickets, TK* s_ticket, bool with_epoch)
 {
     if (threadIdx.x == 0) {
         const unsigned long long tk = atomicAdd(p.ticket, 1ULL);
-        *s_ticket = tk < (unsigned long long)n_tickets ? (long long)tk : -1;
-        if (*s_ticket >= 0) decode((long long)tk);  // (thread 0 only: whatever the CTA needs to know about the ticket, via shared memory)
+        *s_ticket = tk < (unsigned long long)n_tickets ? (TK)tk : -1;
         if (*s_ticket < 0) {
             __threadfence();
             if (atomicAdd(p.ticket + 1, 1ULL) == (unsigned long long)gridDim.x - 1ULL) {
@@ -1613,7 +1625,7 @@ __device__ __forceinline__ long long draw_ticket(const KernelParams& p, long lon
         }
     }
     __syncthreads();
-    const long long tk = *s_ticket;
+    const TK tk = *s_ticket;
     __syncthreads();  // s_ticket is rewritten by thread 0 at the top of the next round
     return tk;
 }
@@ -1638,7 +1650,7 @@ __global__ void __launch_bounds__(PL::THREADS, MINB) lsmrc_data_sh(const KernelP
     const long long n_items = (n_work + TEAMS - 1) / TEAMS;
     uint32_t h_phase = 0;
     for (;;) {
-        const long long item = draw_ticket(p, n_items, &s_ticket, false, [](long long) {});
+        const long long item = draw_ticket(p, n_items, &s_ticket, false);
         if (item < 0) break;
         sh_data_item<PL, false>(p, row, s_h + row.team * N, &bar_h[row.team], h_phase, (int)item);
     }
@@ -1854,7 +1866,7 @@ __global__ void __launch_bounds__(PL::THREADS, MINB) lsmrc_frames_sh(const Kerne
     bool g_valid = false;  // the LS-divide table sits where data items keep their channel rows
     uint32_t h_phase = 0;
     for (;;) {
-        const long long tk = draw_ticket(p, n_tickets, &s_ticket, true, [](long long) {});
+        const long long tk = draw_ticket(p, n_tickets, &s_ticket, true);
         if (tk < 0) break;
         const long long pilot = tk < np ? tk : -1, data = tk - np;
         if (pilot >= 0) {
@@ -2457,16 +2469,7 @@ __global__ void __launch_bounds__(PL::THREADS, 1) lsmrc_mu_data(const KernelPara
                 }
                 if (p.bits != nullptr) {
                     team_sync<PL>(team);
-                    uint8_t* bits_row = p.bits + orow * p.bits_row_bytes;
-                    for (int byte = t; byte < p.bits_row_bytes; byte += T) {
-                        unsigned v8 = 0;
-                        for (int q = 0; q < 8; ++q) {
-                            const int pos = byte * 8 + q;
-                            const int sym = pos / b, bit = pos - sym * b;
-                            if (sym < K) v8 |= ((s_idx[sym] >> bit) & 1u) << q;
-                        }
-                        if (store) bits_row[byte] = (uint8_t)v8;
-                    }
+                    pack_bits<PL>(s_idx, p.bits + orow * p.bits_row_bytes, p.bits_row_bytes, b, store, t);
                 }
             }
         };
