@@ -77,6 +77,8 @@ ABI = {
                                              POINTER(c_int)]),
     "lsmrc_demod_frames_device_mu_soft": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_float, c_void_p, c_void_p, c_void_p,
                                                   c_void_p, c_void_p, POINTER(c_int)]),
+    "lsmrc_precode_frames_device": (c_int, [c_void_p, c_void_p, c_int, c_int, c_float, c_void_p, c_int, c_void_p, c_void_p,
+                                            POINTER(c_int)]),
     "lsmrc_ring_copy_query": (c_int, [c_void_p, c_int]),
     "lsmrc_ring_submit_frames": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_int]),
     "lsmrc_set_timing": (c_int, [c_void_p, c_int]),
@@ -239,6 +241,17 @@ class LsMrcReceiver:
         self._ck(self.lib.lsmrc_demod_frames_device_mu_soft(self.h, _ptr(d_rx), n_frames, n_users, self.DETECTORS.get(detector, -1),
                                                             float(noise_var), _ptr(d_hconj), _ptr(d_combined), _ptr(d_bits),
                                                             _ptr(d_llr), _ptr(d_sinr), byref(bad) if count_singular else None))
+        return bad.value if count_singular else None
+
+    def precode_frames_device(self, d_hconj, n_frames, n_users, d_sym, n_sym_dl, d_tx, d_gain=None, reg=0.0,
+                              count_singular=False):
+        """Multi-user downlink: ZF (reg = 0) or regularised-ZF precoding from the uplink estimate d_hconj [F,U,A,K] (as
+        demod_frames_device_mu exports it), inverse FFT and cyclic prefix.  d_sym [F,Sd,U,K] complex64 ascending
+        frequency -> d_tx [F,Sd,A,N+C] complex64, d_gain [F] float32 per-frame power gain.  With count_singular the call
+        is synchronous and returns the number of (frame, subcarrier) pairs whose Gram matrix was singular."""
+        bad = c_int(0)
+        self._ck(self.lib.lsmrc_precode_frames_device(self.h, _ptr(d_hconj), n_frames, n_users, float(reg), _ptr(d_sym), n_sym_dl,
+                                                      _ptr(d_tx), _ptr(d_gain), byref(bad) if count_singular else None))
         return bad.value if count_singular else None
 
     def zf_apply(self, d_hzf, d_xd, n_ant, n_sc, n_users, d_hx):

@@ -42,6 +42,10 @@ struct PlanOps {
     cudaError_t (*mu_prepare)(bool soft, int* ctas_per_sm);
     cudaError_t (*mu_launch)(bool soft, const KernelParams&, const float2* hzf, float2* wd, const float2* soft_tab, int n_users, int max_ctas,
                              int n_sms, cudaStream_t);
+    // multi-user downlink: resident CTAs of the precode kernel, and the launch of the bin-order precoder layout + that kernel
+    cudaError_t (*dl_prepare)(int* ctas_per_sm);
+    cudaError_t (*dl_launch)(const float2* hzf, float2* pd, const float2* sym, const float* gain, float2* tx, const float2* twiddles,
+                             int n_frames, int n_sym, int n_ant, int n_users, int cp, int max_ctas, int n_sms, cudaStream_t);
 };
 
 // The one-launch kernel (MODE_ONESHOT) of a plan.  Small FFT sizes have a dedicated latency plan:
@@ -356,6 +360,34 @@ cudaError_t mu_launch_impl(bool soft, const KernelParams& p, const float2* hzf, 
     return cudaGetLastError();
 }
 
+// the precode kernel (lsmrc_dl_precode) has the multi-user data kernel's shared-memory layout: twiddles and team tiles
+template <class PL>
+cudaError_t dl_prepare_impl(int* ctas_per_sm)
+{
+    cudaError_t e = cudaFuncSetAttribute(lsmrc_dl_precode<PL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mu_smem<PL>());
+    if (e != cudaSuccess) return e;
+    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas_per_sm, lsmrc_dl_precode<PL>, PL::THREADS, mu_smem<PL>());
+}
+
+// max_ctas: resident CTAs of lsmrc_dl_precode on the whole GPU (dl_prepare_impl x SMs)
+template <class PL>
+cudaError_t dl_launch_impl(const float2* hzf, float2* pd, const float2* sym, const float* gain, float2* tx, const float2* twiddles,
+                           int n_frames, int n_sym, int n_ant, int n_users, int cp, int max_ctas, int n_sms, cudaStream_t st)
+{
+    const long long rows = (long long)n_frames * n_users * n_ant;
+    long long wblocks = (rows * PL::N + 255) / 256;
+    if (wblocks > (long long)n_sms * 16) wblocks = (long long)n_sms * 16;
+    // (plans without a shuffle stage: their slot layout is bin order, the uplink's instantiation serves)
+    k_mu_weights<PL, (PL::SH > 1)><<<(unsigned)wblocks, 256, 0, st>>>(hzf, pd, n_ant, n_users, n_users, rows);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    const long long items = (long long)n_frames * n_sym * n_ant;
+    long long grid = (items + PL::TEAMS - 1) / PL::TEAMS;
+    if (grid > max_ctas) grid = max_ctas;
+    lsmrc_dl_precode<PL><<<(unsigned)grid, PL::THREADS, mu_smem<PL>(), st>>>(pd, sym, gain, tx, twiddles, n_frames, n_sym, n_ant, n_users, cp);
+    return cudaGetLastError();
+}
+
 template <class PL, int MINB>
 PlanOps make_ops()
 {
@@ -376,6 +408,8 @@ PlanOps make_ops()
     o.mu_ug = mu_ug<PL>();
     o.mu_prepare = &mu_prepare_impl<PL>;
     o.mu_launch = &mu_launch_impl<PL>;
+    o.dl_prepare = &dl_prepare_impl<PL>;
+    o.dl_launch = &dl_launch_impl<PL>;
     return o;
 }
 
@@ -559,6 +593,13 @@ struct lsmrc_ctx {
     int* d_mu_count = nullptr;     // singular (frame, subcarrier) pairs
     int mu_max_ctas = 0;           // resident CTAs of the multi-user data kernel (0: not prepared yet)
     int mu_soft_max_ctas = 0;      // the same for its soft instantiation
+    // multi-user downlink (lsmrc_precode_frames_device): scratch of its own, so that it never regrows buffers a captured
+    // uplink call uses
+    float2* d_dl_hzf = nullptr;    // [F][K][U][A] conj(P)
+    float2* d_dl_pd = nullptr;     // [F][U][A][N] P in bin order
+    float* d_dl_part = nullptr;    // power partials [F][chunks], then the gain [F] when the caller passes none
+    size_t dl_hzf_cap = 0, dl_pd_cap = 0, dl_part_cap = 0;  // bytes
+    int dl_max_ctas = 0;           // resident CTAs of the precode kernel
     float* soft_llr = nullptr;            // set for the duration of a *_soft call
     float soft_inv_noise = 1.f;
     bool timing = false;
@@ -1178,6 +1219,12 @@ int lsmrc_create(const lsmrc_config* cfg, lsmrc_handle* out)
         fail_cuda(h, e, "cudaFuncSetAttribute (zero forcing)");
         return bail(LSMRC_ERR_CUDA);
     }
+    {  // downlink precode kernel: its shared-memory attribute once here, so that no call sets one (calls stay capturable)
+        int per_sm = 0;
+        if ((e = ops->dl_prepare(&per_sm)) != cudaSuccess) { fail_cuda(h, e, "cudaFuncSetAttribute (precode kernel)"); return bail(LSMRC_ERR_CUDA); }
+        if (per_sm < 1) { h->err = "precode kernel does not fit on an SM"; return bail(LSMRC_ERR_CUDA); }
+        h->dl_max_ctas = per_sm * h->n_sms;
+    }
     // the table uploads above are pageable-memory copies on the legacy stream (they return once staged); the kernels
     // run on non-blocking streams that do not order against it
     if ((e = cudaDeviceSynchronize()) != cudaSuccess) { fail_cuda(h, e, "cudaDeviceSynchronize"); return bail(LSMRC_ERR_CUDA); }
@@ -1204,6 +1251,9 @@ int lsmrc_destroy(lsmrc_handle h)
     cudaFree(h->d_mu_wd);
     cudaFree(h->d_mu_soft);
     cudaFree(h->d_mu_count);
+    cudaFree(h->d_dl_hzf);
+    cudaFree(h->d_dl_pd);
+    cudaFree(h->d_dl_part);
     cudaFree(h->d_sym);
     cudaFree(h->d_one_hconj);
     cudaFree(h->d_one_comb);
@@ -1422,6 +1472,63 @@ int lsmrc_demod_frames_device_mu_soft(lsmrc_handle h, const void* d_rx, int n_fr
     CK(h, h->ops->mu_launch(true, p, h->d_mu_hzf, h->d_mu_wd, tab, n_users, h->mu_soft_max_ctas, h->n_sms, st));
     h->launches += 2;
     return mu_finish(h, st, n_frames, n_users, d_hconj, n_singular);
+}
+
+int lsmrc_precode_frames_device(lsmrc_handle h, const void* d_hconj, int n_frames, int n_users, float reg, const void* d_sym,
+                                int n_sym_dl, void* d_tx, void* d_gain, int* n_singular)
+{
+    if (!h || !d_hconj || !d_sym || !d_tx) return fail(h, LSMRC_ERR_INVALID, "null argument");
+    if (n_frames < 0) return fail(h, LSMRC_ERR_INVALID, "n_frames < 0");
+    const int A = h->cfg.n_ant, N = h->cfg.fft_size, C = h->cfg.cp_len, K = h->K, U = n_users;
+    if (U < 1 || U > kZfMaxUsers || U > A) return fail(h, LSMRC_ERR_INVALID, "need 1 <= n_users <= 16 and n_users <= n_ant");
+    if (n_sym_dl < 1) return fail(h, LSMRC_ERR_INVALID, "n_sym_dl must be >= 1");
+    if (!(std::isfinite(reg) && reg >= 0.f)) return fail(h, LSMRC_ERR_INVALID, "reg must be finite and >= 0");
+    if (C > N) return fail(h, LSMRC_ERR_INVALID, "a cyclic prefix longer than the symbol cannot be transmitted");
+    const int kt = zf_tile(h, A, U);
+    if (kt < 1) return fail(h, LSMRC_ERR_UNSUPPORTED, "n_ant * n_users too large for one CTA's shared memory");
+    if (n_frames == 0) {
+        if (n_singular) *n_singular = 0;
+        return LSMRC_OK;
+    }
+    CK(h, cudaSetDevice(h->cfg.device));
+    cudaStream_t st = compute_stream(h);
+    const long long F = n_frames;
+    const long long frame_elems = (long long)K * U * A;  // one frame's precoder block
+    constexpr int kChunk = 4096;                         // elements per power partial
+    const int n_chunks = (int)((frame_elems + kChunk - 1) / kChunk);
+    int rc;
+    if ((rc = ensure_scratch(h, h->d_dl_hzf, h->dl_hzf_cap, sizeof(float2) * (size_t)(F * frame_elems), st)) != LSMRC_OK) return rc;
+    if ((rc = ensure_scratch(h, h->d_dl_pd, h->dl_pd_cap, sizeof(float2) * (size_t)(F * U * A * N), st)) != LSMRC_OK) return rc;
+    if ((rc = ensure_scratch(h, h->d_dl_part, h->dl_part_cap, sizeof(float) * (size_t)(F * n_chunks + F), st)) != LSMRC_OK) return rc;
+    if (!h->d_mu_count) CK(h, cudaMalloc(&h->d_mu_count, sizeof(int)));
+    // lsmrc_set_timing: the two phases on the handle's event ring (lsmrc_last_kernel_ms: precoder build, precode)
+    cudaEvent_t* ev = h->timing ? h->ev[h->ev_calls % lsmrc_ctx::kEvRing] : nullptr;
+    if (ev) CK(h, cudaEventRecord(ev[0], st));
+    // 1. precoder per (frame, subcarrier): X = conj(H) [U][A][K] of the frame, as the caller has it -> Hzf = conj(P)
+    if (n_singular) CK(h, cudaMemsetAsync(h->d_mu_count, 0, sizeof(int), st));
+    if ((rc = launch_zf_create(h, st, static_cast<const float2*>(d_hconj), h->d_dl_hzf, A, K, U, kt, reg, n_frames, frame_elems,
+                               (long long)A * K, frame_elems, n_singular ? h->d_mu_count : nullptr)) != LSMRC_OK)
+        return rc;
+    // 2. per-frame gain from the sum of |P|^2 in a fixed order
+    float* gain = d_gain ? static_cast<float*>(d_gain) : h->d_dl_part + F * n_chunks;
+    k_sq_norm_chunks<<<(unsigned)(F * n_chunks), 256, 0, st>>>(h->d_dl_hzf, frame_elems, kChunk, n_chunks, h->d_dl_part);
+    k_dl_gain<<<(unsigned)((F + 7) / 8), 256, 0, st>>>(h->d_dl_part, n_chunks, n_frames, (float)U * (float)K, gain);
+    h->launches += 2;
+    CK(h, cudaGetLastError());
+    if (ev) CK(h, cudaEventRecord(ev[1], st));
+    // 3. bin-order precoder, then precoding fused with the inverse row FFT and the cyclic prefix
+    CK(h, h->ops->dl_launch(h->d_dl_hzf, h->d_dl_pd, static_cast<const float2*>(d_sym), gain, static_cast<float2*>(d_tx), h->d_tw,
+                            n_frames, n_sym_dl, A, U, C, h->dl_max_ctas, h->n_sms, st));
+    h->launches += 2;
+    if (ev) {
+        CK(h, cudaEventRecord(ev[2], st));
+        h->ev_calls++;
+    }
+    if (n_singular) {
+        CK(h, cudaMemcpyAsync(n_singular, h->d_mu_count, sizeof(int), cudaMemcpyDeviceToHost, st));
+        CK(h, cudaStreamSynchronize(st));
+    }
+    return LSMRC_OK;
 }
 
 int lsmrc_demod_frames_device_soft(lsmrc_handle h, const void* d_rx, int n_frames, void* d_combined, void* d_bits,

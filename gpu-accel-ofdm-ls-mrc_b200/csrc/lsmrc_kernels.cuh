@@ -2323,10 +2323,14 @@ __global__ void k_zf_apply(const float2* __restrict__ Hzf, const float2* __restr
 // Wd [F][UP][A][N]: W_k[u][a] in the plan's slot layout (Plan::hpos), times conj of the slot's unit factor (the sink
 // of row_fft sees y' = u * Y on the shuffle-stage plans, so Wd * y' = W * Y).  Users U..UP-1 (padding of the last
 // group) and bin 0 are zero.  Hzf [F][K][U][A] = conj(W).
-template <class PL>
+// BIN_ORDER: plain bin order instead of the slot layout, no unit factor -- the downlink precoder (DESIGN.md 8g) feeds W
+// to the FFT's input, which is natural order on every plan.  (On plans without a shuffle stage the two layouts are the
+// same, so those only need the default instantiation.)
+template <class PL, bool BIN_ORDER = false>
 __global__ void k_mu_weights(const float2* __restrict__ hzf, float2* __restrict__ wd, int A, int U, int UP, long long rows)
 {
     constexpr int N = PL::N, T = PL::T, K = N - 1;
+    constexpr bool SLOTS = PL::SH > 1 && !BIN_ORDER;
     const long long n = rows * N;
     for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < n; idx += (long long)gridDim.x * blockDim.x) {
         const int pos = (int)(idx % N);
@@ -2335,12 +2339,12 @@ __global__ void k_mu_weights(const float2* __restrict__ hzf, float2* __restrict_
         const int u = (int)((row / A) % UP);
         const long long f = row / ((long long)A * UP);
         const int sl = pos / T, t = pos % T;
-        const int bin = (PL::SH == 1) ? pos : PL::bin_of(sl, t);
+        const int bin = SLOTS ? PL::bin_of(sl, t) : pos;
         float2 w = make_float2(0.f, 0.f);
         if (bin > 0 && u < U) {
             const float2 c = hzf[((f * K + (bin - 1)) * U + u) * A + a];
             w = make_float2(c.x, -c.y);
-            if constexpr (PL::SH > 1) w = PL::unfix(sl, t, w);
+            if constexpr (SLOTS) w = PL::unfix(sl, t, w);
         }
         wd[idx] = w;
     }
@@ -2481,6 +2485,116 @@ __global__ void __launch_bounds__(PL::THREADS, 1) lsmrc_mu_data(const KernelPara
             epilogue(std::integral_constant<int, 0>{});
         }
         team_sync<PL>(team);  // the bytes alias the tile the next item's first row is exchanged through
+    }
+}
+
+// ---- multi-user downlink (DESIGN.md 8g) ------------------------------------------------------------------------
+// Reciprocal ZF / regularised-ZF precoder from the uplink estimate: P_k[a][u] = W_k[u][a] = conj(Hzf[k][u][a])
+// (k_zf_create on X = conj(H) with lambda = reg), laid out by k_mu_weights<PL, true> in plain bin order [F][U][A][N].
+// One common gain per frame, g_f = sqrt(U*K / sum_k |P_k|_F^2), |P_k|_F = |Hzf_k|_F.
+
+// Power, step 1: part[f * n_chunks + c] = sum of |x|^2 over elements [c*chunk, (c+1)*chunk) of frame f's block of
+// frame_elems.  Fixed reduction order (per-thread strided sums, warp shuffles, warps in order): deterministic.
+__global__ void k_sq_norm_chunks(const float2* __restrict__ x, long long frame_elems, int chunk, int n_chunks, float* __restrict__ part)
+{
+    const long long f = blockIdx.x / n_chunks;
+    const long long i0 = (long long)(blockIdx.x - f * n_chunks) * chunk;
+    const int n = (int)min((long long)chunk, frame_elems - i0);
+    const float2* p = x + f * frame_elems + i0;
+    float acc = 0.f;
+    for (int i = threadIdx.x; i < n; i += blockDim.x) {
+        const float2 v = p[i];
+        acc += v.x * v.x + v.y * v.y;
+    }
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, off);
+    __shared__ float s_w[32];
+    if ((threadIdx.x & 31) == 0) s_w[threadIdx.x >> 5] = acc;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        float t = 0.f;
+        for (int w = 0; w < (int)(blockDim.x + 31) / 32; ++w) t += s_w[w];
+        part[blockIdx.x] = t;
+    }
+}
+
+// Power, step 2: gain[f] = sqrt(target / sum_c part[f][c]), one warp per frame, fixed order.  A frame whose precoder is
+// zero on every subcarrier (all singular) gets gain 0.
+__global__ void k_dl_gain(const float* __restrict__ part, int n_chunks, int n_frames, float target, float* __restrict__ gain)
+{
+    const int f = blockIdx.x * (blockDim.x / 32) + (threadIdx.x >> 5);
+    if (f >= n_frames) return;
+    const int lane = threadIdx.x & 31;
+    float acc = 0.f;
+    for (int c = lane; c < n_chunks; c += 32) acc += part[(long long)f * n_chunks + c];
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, off);
+    if (lane == 0) gain[f] = acc > 0.f ? sqrtf(target / acc) : 0.f;
+}
+
+// Precoding, inverse FFT and cyclic prefix, fused.  Teams take items (frame f, downlink symbol d, antenna a), a fastest,
+// so that the teams running at the same time share (f, d) and read the same symbol rows out of L1/L2.  Per item the
+// team forms the transform's input in registers -- slot n1 of thread t holds bin n = n1*T + t, row_load's natural order:
+//   v = conj(z[n]),  z[n] = sum_u P[u][a][n] * s[u][asc(n)],  z[0] = 0
+// -- runs the FORWARD row transform, IDFT(z) = conj(DFT(conj z)) / N, and the sink writes g/N * conj(Y) for time index
+// n = bin_of(sl, t) at C + n, and again at n - (N - C) when n >= N - C (the cyclic prefix).  On the shuffle-stage plans
+// the sink sees y' = u * Y, slots out of order: Y = Plan::unfix(y'), and bin_of gives the index (DESIGN.md 8g).
+// pd [F][U][A][N] bin order; sym [F][Sd][U][K] ascending frequency; gain [F]; tx [F][Sd][A][N+C], CP first.
+constexpr int kDlMinBlocks = 3;  // resident CTAs per SM the precode kernel is compiled for (168 registers at four warps)
+
+template <class PL>
+__global__ void __launch_bounds__(PL::THREADS, kDlMinBlocks) lsmrc_dl_precode(const float2* __restrict__ pd, const float2* __restrict__ sym,
+                                                                   const float* __restrict__ gain, float2* __restrict__ tx,
+                                                                   const float2* __restrict__ twiddles, int n_frames, int n_sym,
+                                                                   int A, int U, int cp)
+{
+    constexpr int N = PL::N, P = PL::P, T = PL::T, K = N - 1;
+    extern __shared__ __align__(16) float2 smem[];
+    float2* s_tw1 = smem;
+    float2* s_tw2 = smem + PL::TW1;
+    float2* s_tiles = smem + PL::TWN;
+    const int team = threadIdx.x / T;
+    const int t = threadIdx.x % T;
+    float2* my_tiles = s_tiles + team * PL::TEAM_STRIDE;
+    for (int i = threadIdx.x; i < PL::TWN; i += PL::THREADS) smem[i] = twiddles[i];
+    __syncthreads();
+
+    const long long n_items = (long long)n_frames * n_sym * A;
+    const long long n_rounds = (n_items + (long long)gridDim.x * PL::TEAMS - 1) / ((long long)gridDim.x * PL::TEAMS);
+    for (long long r = 0; r < n_rounds; ++r) {  // every team runs the same number of rounds: team_sync stays uniform
+        const long long raw = (r * gridDim.x + blockIdx.x) * PL::TEAMS + team;
+        const bool ok = raw < n_items;
+        const long long item = ok ? raw : n_items - 1;
+        const int a = (int)(item % A);
+        const long long fd = item / A;  // f * Sd + d
+        const long long f = fd / n_sym;
+        const float2* s_row = sym + fd * U * K;
+        const float2* p_row = pd + (f * U * A + a) * N;
+        float2 v[P];
+#pragma unroll
+        for (int n1 = 0; n1 < P; ++n1) v[n1] = make_float2(0.f, 0.f);
+        for (int u = 0; u < U; ++u) {
+            const float2* pu = p_row + (long long)u * A * N;
+            const float2* su = s_row + (long long)u * K;
+#pragma unroll
+            for (int n1 = 0; n1 < P; ++n1) {
+                const int n = n1 * T + t;
+                if (n > 0) v[n1] = cmac(v[n1], __ldg(pu + n), __ldg(su + (n < N / 2 ? n - 1 + N / 2 : n - N / 2)));
+            }
+        }
+#pragma unroll
+        for (int n1 = 0; n1 < P; ++n1) v[n1].y = -v[n1].y;
+        const float sc = __ldg(gain + f) * (1.0f / N);  // (exact: N is a power of two)
+        float2* out = tx + (fd * A + a) * (N + cp);
+        float2* tile = my_tiles + (PL::NBUF == 2 ? (int)(r & 1) * PL::TILE : 0);
+        row_fft<PL>(v, nullptr, tile, s_tw1, s_tw2, t, team, [&](int sl, int n, float2 y) {
+            const float2 Y = PL::unfix(sl, t, y);
+            const float2 o = make_float2(sc * Y.x, -sc * Y.y);
+            if (ok) {
+                out[cp + n] = o;
+                if (n >= N - cp) out[n - (N - cp)] = o;
+            }
+        });
     }
 }
 

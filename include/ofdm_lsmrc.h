@@ -288,6 +288,34 @@ int lsmrc_demod_frames_device_mu_soft(lsmrc_handle h, const void *d_rx, int n_fr
                                       float noise_var, void *d_hconj, void *d_combined, void *d_bits,
                                       void *d_llr, void *d_sinr, int *n_singular);
 
+/* ---- multi-user downlink: zero-forcing precoding from the uplink channel estimates, fused with the inverse row FFT
+ *      and cyclic-prefix insertion (DESIGN.md 8g; replaces createZeroForcingMatrix -> multiplyWithChannelInv ->
+ *      modOneSymbol -> addPrefix, cpuLS.hpp:391-529, uncalled in the reference).  Channel reciprocity (TDD): the
+ *      downlink channel from the antennas to user u is row u of H_k^T, H_k the A x U uplink channel of subcarrier k.
+ *      Per frame f and subcarrier k (FFT-bin order):
+ *        P_k = conj(H_k) inv(H_k^T conj(H_k) + reg I)        A x U precoder; P_k[a][u] = W_k[u][a], the uplink detector
+ *        z[d][a][k] = sum_u P_k[a][u] s[d][u][k]             bin 0 is 0
+ *        g_f = sqrt(U K / sum_k |P_k|_F^2)                   one gain per frame: unit-energy symbols give a mean transmit
+ *                                                            energy of U per used subcarrier
+ *        tx[d][a][C + n] = g_f IDFT(z[d][a])[n]              with the 1/N of numpy.fft.ifft; tx[d][a][0..C) = tx[d][a][N..N+C)
+ *      reg = 0 is ZF (H_k^T P_k = I: user u receives g_f s_u), reg > 0 regularised ZF.  A subcarrier whose Gram matrix is
+ *      singular (the rule of lsmrc_demod_frames_device_mu) gets P_k = 0 and adds nothing to the power sum; a frame with
+ *      no regular subcarrier gets g_f = 0.  The receiver's FFT of a tx row (CP dropped) gives back g_f z.
+ *      Device pointers, complex64 unless noted; the handle's compute stream, as lsmrc_demod_frames_device:
+ *        d_hconj    [F][U][A][K]          conj(H) per user in the reference layout, as lsmrc_demod_frames_device_mu writes
+ *                                         it (the handle keeps no channel state: the caller passes it back)
+ *        d_sym      [F][Sd][U][K]         user symbols, ascending frequency (the layout of that call's d_combined)
+ *        d_tx       [F][Sd][A][N+C]       time-domain antenna samples, CP first (the receiver's input layout)
+ *        d_gain     [F] float             g_f; may be NULL
+ *        n_singular (host, may be NULL; non-NULL makes the call synchronous): (frame, subcarrier) pairs whose Gram
+ *                   matrix was singular.
+ *      A, N and C come from the handle; any FFT size the handle supports, C <= N, A <= 256, 1 <= U <= 16, U <= A,
+ *      Sd = n_sym_dl >= 1.  No pilot is needed.  LSMRC_ERR_INVALID for a bad U or Sd, a reg that is not finite and >= 0,
+ *      or a NULL d_hconj / d_sym / d_tx; nothing is launched then.  With n_singular == NULL the call can be captured
+ *      into a CUDA graph after one ordinary call of the same size (which allocates its scratch). */
+int lsmrc_precode_frames_device(lsmrc_handle h, const void *d_hconj, int n_frames, int n_users, float reg,
+                                const void *d_sym, int n_sym_dl, void *d_tx, void *d_gain, int *n_singular);
+
 /* ---- memory and stream plumbing, so callers need no CUDA headers (replaces the raw
  *      cudaMalloc/cudaMemcpy/cudaFree calls of gpuLS_main.cu:73-91,135-139) ------------ */
 int lsmrc_dev_alloc(lsmrc_handle h, size_t bytes, void **d_ptr);
@@ -319,7 +347,9 @@ long long lsmrc_one_launch_frames_count(lsmrc_handle h);
 
 /* ---- instrumentation (replaces the clock() timers of ShMemSymBuff_gpu.hpp:113-257) --- */
 /* CUDA-event time of the pilot and data kernels of the most recent lsmrc_demod_frames_device
- * call (waits for them).  Enable with lsmrc_set_timing(h, 1); off by default. */
+ * call (waits for them).  Enable with lsmrc_set_timing(h, 1); off by default.  A timed
+ * lsmrc_precode_frames_device call reports its two phases in the same places: the precoder build
+ * (inverse and gain) as the pilot time, the precode phase (layout pass and precode kernel) as the data time. */
 int lsmrc_set_timing(lsmrc_handle h, int enabled);
 int lsmrc_last_kernel_ms(lsmrc_handle h, float *pilot_ms, float *data_ms);
 /* the same for the most recent min(max_n, 256) timed calls, oldest first; waits for them.  Lets a
