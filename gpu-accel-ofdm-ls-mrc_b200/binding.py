@@ -77,6 +77,7 @@ ABI = {
                                              POINTER(c_int)]),
     "lsmrc_demod_frames_device_mu_soft": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_float, c_void_p, c_void_p, c_void_p,
                                                   c_void_p, c_void_p, POINTER(c_int)]),
+    "lsmrc_set_mu_pilots": (c_int, [c_void_p, c_int]),
     "lsmrc_precode_frames_device": (c_int, [c_void_p, c_void_p, c_int, c_int, c_float, c_void_p, c_int, c_void_p, c_void_p,
                                             POINTER(c_int)]),
     "lsmrc_ring_copy_query": (c_int, [c_void_p, c_int]),
@@ -219,12 +220,21 @@ class LsMrcReceiver:
         return bad.value
 
     DETECTORS = {"zf": 0, "mmse": 1}
+    MU_PILOTS = {"time": 0, "comb": 1}
+
+    def set_mu_pilots(self, layout="time"):
+        """Pilot layout of the multi-user calls on this handle: "time" (default; symbols 0..U-1 carry one user's pilot
+        each) or "comb" (symbol 0 carries every user's pilot, user u on the ascending-frequency indices i = u mod U;
+        each user's channel is interpolated across its own subcarriers).  Read when a call is enqueued."""
+        self._ck(self.lib.lsmrc_set_mu_pilots(self.h, self.MU_PILOTS.get(layout, -1)))
 
     def demod_frames_device_mu(self, d_rx, n_frames, n_users, d_combined, d_bits=None, d_hconj=None, detector="zf",
                                noise_var=0.0, count_singular=False):
-        """Multi-user frames (symbols 0..U-1 per-user pilots, U..S-1 data of all users): per-user LS channel and ZF or
-        MMSE detection.  d_combined [F,S-U,U,K], d_bits [F,S-U,U,row], d_hconj [F,U,A,K].  With count_singular the call
-        is synchronous and returns the number of (frame, subcarrier) pairs whose Gram matrix was singular."""
+        """Multi-user frames: P pilot symbols, then symbols P..S-1 with the data of all users; per-user LS channel and ZF
+        or MMSE detection.  Time pilots (P = U): d_combined [F,S-U,U,K], d_bits [F,S-U,U,row].  Comb pilots (P = 1,
+        set_mu_pilots("comb")): d_combined [F,S-1,U,K], d_bits [F,S-1,U,row].  d_hconj [F,U,A,K] in both.  With
+        count_singular the call is synchronous and returns the number of (frame, subcarrier) pairs whose Gram matrix
+        was singular."""
         bad = c_int(0)
         self._ck(self.lib.lsmrc_demod_frames_device_mu(self.h, _ptr(d_rx), n_frames, n_users, self.DETECTORS.get(detector, -1),
                                                        float(noise_var), _ptr(d_hconj), _ptr(d_combined), _ptr(d_bits),
@@ -233,8 +243,9 @@ class LsMrcReceiver:
 
     def demod_frames_device_mu_soft(self, d_rx, n_frames, n_users, d_combined, d_llr, d_bits=None, d_hconj=None, d_sinr=None,
                                     detector="zf", noise_var=1.0, count_singular=False):
-        """demod_frames_device_mu plus soft output: d_llr [F,S-U,U,K,b] float32 max-log LLRs (LLR > 0 <=> bit 0) and
-        d_sinr [F,U,K] float32 post-detection SINR, both ascending frequency.  noise_var (> 0, both detectors) is the
+        """demod_frames_device_mu plus soft output: d_llr float32 max-log LLRs (LLR > 0 <=> bit 0), [F,S-U,U,K,b] with
+        time pilots and [F,S-1,U,K,b] with comb pilots, and d_sinr [F,U,K] float32 post-detection SINR, both ascending
+        frequency.  noise_var (> 0, both detectors) is the
         noise variance per antenna and subcarrier; MMSE uses it as its diagonal loading too.  d_combined and d_bits are
         those of demod_frames_device_mu (for MMSE the biased estimate; the LLRs use the unbiased one)."""
         bad = c_int(0)

@@ -586,10 +586,12 @@ struct lsmrc_ctx {
     // multi-user path (lsmrc_demod_frames_device_mu): its own channel state and scratch, grown on demand
     ChanState mu_ch;
     float2* d_mu_hconj = nullptr;  // [U][F][A][K] conj(H) per user, as the pilot kernel writes it
+    float2* d_mu_ls = nullptr;     // comb pilots: [F][A][K] LS estimate of pilot symbol 0, input of k_mu_comb_interp
     float2* d_mu_hzf = nullptr;    // [F][K][U][A] conj(W)
     float2* d_mu_wd = nullptr;     // [F][UP][A][N] W in the data kernel's slot layout
     float* d_mu_soft = nullptr;    // soft output: ginv_diag [F][U][K] float, then the (rho, scale) table [F][U][K] float2
-    size_t mu_hconj_cap = 0, mu_hzf_cap = 0, mu_wd_cap = 0, mu_soft_cap = 0;  // bytes
+    size_t mu_hconj_cap = 0, mu_ls_cap = 0, mu_hzf_cap = 0, mu_wd_cap = 0, mu_soft_cap = 0;  // bytes
+    int mu_pilots = LSMRC_MU_PILOTS_TIME;  // frame format of the multi-user calls (lsmrc_set_mu_pilots)
     int* d_mu_count = nullptr;     // singular (frame, subcarrier) pairs
     int mu_max_ctas = 0;           // resident CTAs of the multi-user data kernel (0: not prepared yet)
     int mu_soft_max_ctas = 0;      // the same for its soft instantiation
@@ -1247,6 +1249,7 @@ int lsmrc_destroy(lsmrc_handle h)
     free_chan(h->one_ch);
     free_chan(h->mu_ch);
     cudaFree(h->d_mu_hconj);
+    cudaFree(h->d_mu_ls);
     cudaFree(h->d_mu_hzf);
     cudaFree(h->d_mu_wd);
     cudaFree(h->d_mu_soft);
@@ -1336,13 +1339,18 @@ namespace {
 
 // The multi-user calls (lsmrc_demod_frames_device_mu and _mu_soft) share their argument checks (mu_check), phases 1-2
 // (mu_detect: scratch, per-user LS channel, detector build) and the hand-back (mu_finish); they differ in phase 3.
+// Both read the handle's pilot layout (h->mu_pilots) when they enqueue: a captured graph keeps the one it saw.
 int mu_check(lsmrc_ctx* h, const void* d_rx, const void* d_combined, int n_frames, int n_users, int detector, float noise_var)
 {
     if (!h || !d_rx || !d_combined) return fail(h, LSMRC_ERR_INVALID, "null argument");
     if (n_frames < 0) return fail(h, LSMRC_ERR_INVALID, "n_frames < 0");
     const int A = h->cfg.n_ant, S = h->cfg.n_sym;
-    if (n_users < 1 || n_users > kZfMaxUsers || n_users > A || n_users >= S)
+    if (h->mu_pilots == LSMRC_MU_PILOTS_COMB) {
+        if (n_users < 1 || n_users > kZfMaxUsers || n_users > A || S < 2)
+            return fail(h, LSMRC_ERR_INVALID, "comb pilots need 1 <= n_users <= 16, n_users <= n_ant and n_sym >= 2");
+    } else if (n_users < 1 || n_users > kZfMaxUsers || n_users > A || n_users >= S) {
         return fail(h, LSMRC_ERR_INVALID, "need 1 <= n_users <= 16, n_users <= n_ant and n_users < n_sym");
+    }
     if (detector != LSMRC_DETECT_ZF && detector != LSMRC_DETECT_MMSE) return fail(h, LSMRC_ERR_INVALID, "unknown detector");
     if (detector == LSMRC_DETECT_MMSE && !(std::isfinite(noise_var) && noise_var > 0.f))
         return fail(h, LSMRC_ERR_INVALID, "MMSE needs a finite noise_var > 0");
@@ -1363,7 +1371,9 @@ int mu_detect(lsmrc_ctx* h, cudaStream_t st, const void* d_rx, int n_frames, int
     const long long F = n_frames;
     int rc;
     if ((rc = ensure_chan(h, h->mu_ch, n_frames, st)) != LSMRC_OK) return rc;
+    const bool comb = h->mu_pilots == LSMRC_MU_PILOTS_COMB;
     if ((rc = ensure_scratch(h, h->d_mu_hconj, h->mu_hconj_cap, sizeof(float2) * (size_t)(U * F * A * K), st)) != LSMRC_OK) return rc;
+    if (comb && (rc = ensure_scratch(h, h->d_mu_ls, h->mu_ls_cap, sizeof(float2) * (size_t)(F * A * K), st)) != LSMRC_OK) return rc;
     if ((rc = ensure_scratch(h, h->d_mu_hzf, h->mu_hzf_cap, sizeof(float2) * (size_t)(F * K * U * A), st)) != LSMRC_OK) return rc;
     if ((rc = ensure_scratch(h, h->d_mu_wd, h->mu_wd_cap, sizeof(float2) * (size_t)(F * UP * A * N), st)) != LSMRC_OK) return rc;
     if (soft && (rc = ensure_scratch(h, h->d_mu_soft, h->mu_soft_cap, (sizeof(float2) + sizeof(float)) * (size_t)(F * U * K), st)) != LSMRC_OK)
@@ -1376,13 +1386,25 @@ int mu_detect(lsmrc_ctx* h, cudaStream_t st, const void* d_rx, int n_frames, int
         if (per_sm < 1) return fail(h, LSMRC_ERR_CUDA, "multi-user data kernel does not fit on an SM");
         max_ctas = per_sm * h->n_sms;
     }
-    // 1. LS channel of every user from its own pilot symbol: the single-user pilot launch, once per pilot symbol
+    // 1. LS channel of every user: the single-user pilot launch, once per pilot symbol (time-orthogonal pilots), or
+    //    once on the comb symbol 0 followed by each user's interpolation across its own subcarriers (comb pilots)
     p = base_params(h);
     p.n_frames = n_frames;
     const long long user_elems = F * A * K;
-    for (int u = 0; u < U; ++u) {
-        p.rx = static_cast<const float2*>(d_rx) + (long long)u * p.sym_stride;
-        if ((rc = launch_pilot(h, st, p, h->mu_ch, h->d_mu_hconj + u * user_elems, nullptr)) != LSMRC_OK) return rc;
+    const int n_pilot_sym = comb ? 1 : U;
+    if (comb) {
+        p.rx = static_cast<const float2*>(d_rx);
+        if ((rc = launch_pilot(h, st, p, h->mu_ch, h->d_mu_ls, nullptr)) != LSMRC_OK) return rc;
+        const long long rows = F * A, cap = (long long)h->n_sms * 16;
+        k_mu_comb_interp<<<(unsigned)(rows < cap ? rows : cap), 256, sizeof(float2) * (size_t)K, st>>>(h->d_mu_ls, h->d_mu_hconj, N, U,
+                                                                                                      rows, user_elems);
+        h->launches++;
+        CK(h, cudaGetLastError());
+    } else {
+        for (int u = 0; u < U; ++u) {
+            p.rx = static_cast<const float2*>(d_rx) + (long long)u * p.sym_stride;
+            if ((rc = launch_pilot(h, st, p, h->mu_ch, h->d_mu_hconj + u * user_elems, nullptr)) != LSMRC_OK) return rc;
+        }
     }
     // 2. detector per (frame, subcarrier): X = conj(H) [U][A][K] of the frame -> Hzf = conj(W)
     if (count) CK(h, cudaMemsetAsync(h->d_mu_count, 0, sizeof(int), st));
@@ -1391,8 +1413,8 @@ int mu_detect(lsmrc_ctx* h, cudaStream_t st, const void* d_rx, int n_frames, int
                                soft ? h->d_mu_soft + 2 * F * U * K : nullptr)) != LSMRC_OK)
         return rc;
     p.rx = static_cast<const float2*>(d_rx);
-    p.first_sym = U;
-    p.n_sym_work = S - U;
+    p.first_sym = n_pilot_sym;
+    p.n_sym_work = S - n_pilot_sym;
     return LSMRC_OK;
 }
 
@@ -2294,6 +2316,14 @@ int lsmrc_set_one_launch_frames(lsmrc_handle h, int enabled)
 }
 
 long long lsmrc_one_launch_frames_count(lsmrc_handle h) { return h ? h->fused_calls : -1; }
+
+int lsmrc_set_mu_pilots(lsmrc_handle h, int layout)
+{
+    if (!h) return LSMRC_ERR_INVALID;
+    if (layout != LSMRC_MU_PILOTS_TIME && layout != LSMRC_MU_PILOTS_COMB) return fail(h, LSMRC_ERR_INVALID, "unknown pilot layout");
+    h->mu_pilots = layout;
+    return LSMRC_OK;
+}
 
 int lsmrc_set_timing(lsmrc_handle h, int enabled)
 {

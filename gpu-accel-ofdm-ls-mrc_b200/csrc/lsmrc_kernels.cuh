@@ -2382,10 +2382,54 @@ __global__ void k_mu_soft_scale(const float* __restrict__ ginv_diag, float2* __r
     }
 }
 
+// Comb pilots (DESIGN.md 8h): symbol 0 carries user u's pilot on the ascending-frequency indices i = u (mod U) only.
+// From the LS estimate of that one symbol, ls [rows = F*A][K] = conj(Z0 / X) in bin order (the pilot kernel's export),
+// every user's conj(H) on every subcarrier, out [U][rows][K] (user_stride between users), bin order:
+//   own pilot (i = u mod U)               ls[i], copied;
+//   between u's pilots p0 < i < p1        ls[p0] + w (ls[p1] - ls[p0]),  w = (phi(i) - phi(p0)) / (phi(p1) - phi(p0));
+//   beyond u's outermost pilot            the nearest pilot's ls, held.
+// phi(i) = i - N/2 for i < N/2, i - N/2 + 1 above: the signed frequency, without DC.  Bin-order index k holds ascending
+// i = (k + N/2) mod K.  A CTA takes one (frame, antenna) row at a time, staged in shared memory (K float2); threads run
+// over the output index k, so each user's output row is one coalesced store.
+__global__ void k_mu_comb_interp(const float2* __restrict__ ls, float2* __restrict__ out, int N, int U, long long rows,
+                                 long long user_stride)
+{
+    extern __shared__ float2 s_row[];
+    const int K = N - 1, half = N / 2;
+    auto phi = [&](int i) { return i < half ? i - half : i - half + 1; };
+    auto bin = [&](int i) { return i < half ? i + half - 1 : i - half; };  // ascending index -> bin-order index
+    for (long long row = blockIdx.x; row < rows; row += gridDim.x) {
+        for (int k = threadIdx.x; k < K; k += blockDim.x) s_row[k] = ls[row * K + k];
+        __syncthreads();
+        for (int u = 0; u < U; ++u) {
+            float2* o = out + u * user_stride + row * K;
+            for (int k = threadIdx.x; k < K; k += blockDim.x) {
+                const int i = k + half < K ? k + half : k + half - K;
+                float2 v;
+                if (i <= u) {
+                    v = s_row[bin(u)];  // own first pilot, or below it: held
+                } else {
+                    const int p0 = i - (i - u) % U, p1 = p0 + U;
+                    if (p0 == i || p1 >= K) {
+                        v = s_row[bin(p0)];  // own pilot, or above the last one: held
+                    } else {
+                        const float w = (float)(phi(i) - phi(p0)) / (float)(phi(p1) - phi(p0));
+                        const float2 a = s_row[bin(p0)], b = s_row[bin(p1)];
+                        v = make_float2(fmaf(w, b.x - a.x, a.x), fmaf(w, b.y - a.y, a.y));
+                    }
+                }
+                o[k] = v;
+            }
+        }
+        __syncthreads();  // the row buffer is refilled next
+    }
+}
+
 // Teams take items (frame f, user group g, data symbol s), consecutive items sharing (f, g) so that the teams working
-// at the same time read the same detector rows (L1/L2).  Outputs: combined [F][S-U][U][K] ascending frequency, bits
-// [F][S-U][U][row].  p.first_sym = U, p.n_sym_work = S-U; n_users = U, UP = groups * UG.
-// SOFT: also p.llr [F][S-U][U][K][b] from soft_tab [F][U][K] (k_mu_soft_scale); the hard kernel ignores soft_tab.
+// at the same time read the same detector rows (L1/L2).  Outputs: combined [F][S-P][U][K] ascending frequency, bits
+// [F][S-P][U][row], P pilot symbols (U time-orthogonal, 1 comb).  p.first_sym = P, p.n_sym_work = S-P; n_users = U,
+// UP = groups * UG.
+// SOFT: also p.llr [F][S-P][U][K][b] from soft_tab [F][U][K] (k_mu_soft_scale); the hard kernel ignores soft_tab.
 template <class PL, int UG, bool SOFT = false>
 __global__ void __launch_bounds__(PL::THREADS, 1) lsmrc_mu_data(const KernelParams p, const float2* __restrict__ wd, int n_users, int n_groups,
                                                                 const float2* __restrict__ soft_tab)

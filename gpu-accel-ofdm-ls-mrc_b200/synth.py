@@ -130,24 +130,42 @@ def make_frames_torch(n_frames, cfg, device, seed=None, snr_db="cfg", chunk=64):
     return rx, pilot_asc, src
 
 
-def make_frames_mu(n_frames, n_ant, fft_size, cp_len, n_sym, qam_bits, n_users, snr_db=None, seed=0, h=None, pilot_asc=None):
-    """Multi-user uplink frames (include/ofdm_lsmrc.h, lsmrc_demod_frames_device_mu): symbol u < U carries user u's
-    pilot (the handle's pilot, the other users silent), symbols U..S-1 the data of all U users at once; i.i.d. Rayleigh
-    channel per user, antenna and subcarrier; AWGN at `snr_db` per user and antenna.  `h` [F,U,A,K] (bin order)
-    replaces the random channel.  With n_users=1 the random draws, their order and the arithmetic are those of
-    make_frames: rx is byte-identical.  Returns dict(rx [F,S,A,N+C] c64, pilot_asc [K] c64, src_idx [F,S-U,U,K] u8
-    (ascending frequency), h_true [F,U,A,K] c128 (bin order))."""
+def _pilot_rows(pilot_asc, U, pilots):
+    """(number of pilot symbols P, per-user pilot rows [U, K] ascending frequency) of a multi-user frame: time
+    pilots, P = U (row u is the whole pilot, sent on symbol u), or comb pilots, P = 1 (row u is the pilot on the
+    indices i = u mod U and zero elsewhere, all sent on symbol 0)"""
+    K = pilot_asc.shape[0]
+    rows = np.broadcast_to(pilot_asc.astype(np.complex128), (U, K)).copy()
+    if pilots == "time":
+        return U, rows
+    if pilots != "comb":
+        raise ValueError("pilots must be 'time' or 'comb'")
+    rows[np.arange(K)[None, :] % U != np.arange(U)[:, None]] = 0.0
+    return 1, rows
+
+
+def make_frames_mu(n_frames, n_ant, fft_size, cp_len, n_sym, qam_bits, n_users, snr_db=None, seed=0, h=None, pilot_asc=None,
+                   pilots="time"):
+    """Multi-user uplink frames (include/ofdm_lsmrc.h, lsmrc_demod_frames_device_mu).  pilots="time": symbol u < U
+    carries user u's pilot (the handle's pilot, the other users silent), symbols U..S-1 the data of all U users at once.
+    pilots="comb": symbol 0 carries user u's pilot on the ascending-frequency indices i = u mod U (nothing elsewhere),
+    symbols 1..S-1 the data.  i.i.d. Rayleigh channel per user, antenna and subcarrier; AWGN at `snr_db` per user and
+    antenna.  `h` [F,U,A,K] (bin order, e.g. multipath_channel) replaces the random channel.  With n_users=1 and time
+    pilots the random draws, their order and the arithmetic are those of make_frames: rx is byte-identical.  Returns
+    dict(rx [F,S,A,N+C] c64, pilot_asc [K] c64, src_idx [F,S-P,U,K] u8 (ascending frequency; P = U time, 1 comb),
+    h_true [F,U,A,K] c128 (bin order))."""
     F, A, N, C, S, U = n_frames, n_ant, fft_size, cp_len, n_sym, n_users
     K = N - 1
-    assert 1 <= U < S
     rng = np.random.default_rng(seed)
     pilot_asc = make_pilot(K, seed) if pilot_asc is None else np.asarray(pilot_asc, np.complex64)
-    src_idx = rng.integers(0, 1 << qam_bits, size=(F, S - U, U, K), dtype=np.uint8)
+    P, prow = _pilot_rows(pilot_asc, U, pilots)
+    assert 1 <= U and P < S
+    src_idx = rng.integers(0, 1 << qam_bits, size=(F, S - P, U, K), dtype=np.uint8)
     data_asc = qam_map_indices(src_idx, qam_bits)
     tx_bin = np.zeros((F, S, U, N), np.complex128)
     for u in range(U):
-        tx_bin[:, u, u, 1:] = asc_to_bin(pilot_asc.astype(np.complex128))
-    tx_bin[:, U:, :, 1:] = asc_to_bin(data_asc)
+        tx_bin[:, u if P == U else 0, u, 1:] = asc_to_bin(prow[u])
+    tx_bin[:, P:, :, 1:] = asc_to_bin(data_asc)
     if h is None:
         h = (rng.standard_normal((F, U, A, K)) + 1j * rng.standard_normal((F, U, A, K))) / np.sqrt(2.0)
     else:
@@ -169,9 +187,10 @@ def make_frames_mu(n_frames, n_ant, fft_size, cp_len, n_sym, qam_bits, n_users, 
 
 
 def make_frames_mu_torch(n_frames, n_ant, fft_size, cp_len, n_sym, qam_bits, n_users, device, seed=0, snr_db=30.0,
-                         chunk=16):
-    """make_frames_mu built directly on `device` with torch, for full-size batches (same frame format, its own random
-    stream).  Returns (rx [F,S,A,N+C] complex64 tensor, pilot_asc numpy [K], src_idx [F,S-U,U,K] uint8 tensor)."""
+                         chunk=16, pilots="time"):
+    """make_frames_mu built directly on `device` with torch, for full-size batches (same frame formats, its own random
+    stream).  Returns (rx [F,S,A,N+C] complex64 tensor, pilot_asc numpy [K], src_idx [F,S-P,U,K] uint8 tensor; P = U
+    with time pilots, 1 with comb pilots)."""
     import torch
 
     A, N, C, S, U, b = n_ant, fft_size, cp_len, n_sym, n_users, qam_bits
@@ -179,19 +198,21 @@ def make_frames_mu_torch(n_frames, n_ant, fft_size, cp_len, n_sym, qam_bits, n_u
     g = torch.Generator(device=device)
     g.manual_seed(seed)
     pilot_asc = make_pilot(K, seed)
-    pil_bin = torch.from_numpy(asc_to_bin(pilot_asc)).to(device)
+    P, prow = _pilot_rows(pilot_asc, U, pilots)
+    assert 1 <= U and P < S
+    pil_bin = torch.from_numpy(asc_to_bin(prow).astype(np.complex64)).to(device)   # [U,K]
     lut = torch.from_numpy(qam_map_indices(np.arange(1 << b), b).astype(np.complex64)).to(device)
     rx = torch.empty((n_frames, S, A, N + C), dtype=torch.complex64, device=device)
-    src = torch.empty((n_frames, S - U, U, K), dtype=torch.uint8, device=device)
+    src = torch.empty((n_frames, S - P, U, K), dtype=torch.uint8, device=device)
     shift = (K + 1) // 2
     for f0 in range(0, n_frames, chunk):
         nf = min(chunk, n_frames - f0)
-        idx = torch.randint(0, 1 << b, (nf, S - U, U, K), generator=g, device=device, dtype=torch.uint8)
+        idx = torch.randint(0, 1 << b, (nf, S - P, U, K), generator=g, device=device, dtype=torch.uint8)
         src[f0:f0 + nf] = idx
         tx = torch.zeros((nf, S, U, N), dtype=torch.complex64, device=device)
         for u in range(U):
-            tx[:, u, u, 1:] = pil_bin
-        tx[:, U:, :, 1:] = torch.roll(lut[idx.long()], -shift, dims=-1)
+            tx[:, u if P == U else 0, u, 1:] = pil_bin[u]
+        tx[:, P:, :, 1:] = torch.roll(lut[idx.long()], -shift, dims=-1)
         h = torch.zeros((nf, U, A, N), dtype=torch.complex64, device=device)
         h[..., 1:] = torch.view_as_complex(torch.randn((nf, U, A, K, 2), generator=g, device=device) * (0.5 ** 0.5))
         yf = torch.einsum("fsun,fuan->fsan", tx, h)
@@ -204,6 +225,18 @@ def make_frames_mu_torch(n_frames, n_ant, fft_size, cp_len, n_sym, qam_bits, n_u
             rx[f0:f0 + nf, :, :, :C] = yt[..., N - C:]
         del tx, h, yf, yt, idx
     return rx, pilot_asc, src
+
+
+def multipath_channel(n_frames, n_users, n_ant, fft_size, n_taps, seed=0):
+    """Frequency response of a tapped delay line per (frame, user, antenna): n_taps independent complex Gaussian taps at
+    the integer delays 0 .. n_taps-1, each of power 1 / n_taps (E|H|^2 = 1).  H[bin] = sum_l g_l exp(-2 pi j bin l / N)
+    on bins 1..N-1.  Unlike the i.i.d. Rayleigh draw of make_frames_mu it is smooth in frequency, so comb pilots can be
+    interpolated.  Returns [F,U,A,K] complex128, bin order (make_frames_mu's `h`)."""
+    rng = np.random.default_rng(seed)
+    shape = (n_frames, n_users, n_ant, n_taps)
+    g = (rng.standard_normal(shape) + 1j * rng.standard_normal(shape)) / np.sqrt(2.0 * n_taps)
+    ph = np.exp(-2j * np.pi * np.outer(np.arange(n_taps), np.arange(1, fft_size)) / fft_size)   # [L,K]
+    return g @ ph
 
 
 def make_pn(length=255, seed=0x1D):

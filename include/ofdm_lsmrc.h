@@ -239,13 +239,25 @@ int lsmrc_zf_create(lsmrc_handle h, const void *d_x, int n_ant, int n_sc, int n_
 int lsmrc_zf_apply(lsmrc_handle h, const void *d_hzf, const void *d_xd, int n_ant, int n_sc, int n_users, void *d_hx);
 
 /* ---- multi-user uplink: per-user LS channel estimates and linear detection fused with the row FFT (not in the
- *      reference; DESIGN.md 8e).  Frame format: the usual rx [F][S][A][N+C] (N+C per antenna row, CP first), with
- *      U = n_users:
+ *      reference; DESIGN.md 8e, 8h).  Frame format: the usual rx [F][S][A][N+C] (N+C per antenna row, CP first), with
+ *      U = n_users and P pilot symbols, in one of two pilot layouts chosen per handle with lsmrc_set_mu_pilots:
+ *      LSMRC_MU_PILOTS_TIME (default), P = U:
  *        symbols 0 .. U-1   time-orthogonal pilots: on symbol u user u sends the handle's pilot (lsmrc_set_pilot*),
  *                           the other users are silent;
  *        symbols U .. S-1   data of all U users on the same subcarriers at once.
- *      With U = 1 this is the single-user frame.  Per frame f and subcarrier k (FFT-bin order):
- *        H[u][a][k] = Z_u[a][k] / X[k]                       LS per user (Z_u: FFT of pilot symbol u)
+ *      LSMRC_MU_PILOTS_COMB, P = 1:
+ *        symbol 0           comb pilots: user u sends the handle's pilot X[i] on the ascending-frequency indices
+ *                           i = u (mod U) (i = 0 .. K-1, the lsmrc_set_pilot order) and nothing on the others;
+ *        symbols 1 .. S-1   data of all U users on the same subcarriers at once.
+ *      With U = 1 both are the single-user frame.  Per frame f and subcarrier k (FFT-bin order):
+ *        H[u][a][k] = Z_u[a][k] / X[k]                       time: LS per user (Z_u: FFT of pilot symbol u)
+ *        H[u][a][k] = interpolated LS of symbol 0            comb: LS[a][i] = conj(Z_0[a][i] / X[i]) (conj(H)) is
+ *                                                            copied on u's own pilots; between u's nearest pilots
+ *                                                            p0 < i < p1 it is LS[p0] + w (LS[p1] - LS[p0]) with
+ *                                                            w = (phi(i) - phi(p0)) / (phi(p1) - phi(p0)), fp32;
+ *                                                            beyond u's outermost pilot the nearest one is held.
+ *                                                            phi(i) = i - N/2 (i < N/2), i - N/2 + 1 (i >= N/2): the
+ *                                                            signed frequency, DC skipped.
  *        G_k = H_k^H H_k + lambda I,  W_k = inv(G_k) H_k^H    H_k the A x U matrix; W_k is U x A
  *        xhat[s][u][k] = sum_a W_k[u][a] Z_s[a][k]           every data symbol s
  *      ZF: lambda = 0.  MMSE: lambda = noise_var, the noise variance per antenna and subcarrier after the FFT (same
@@ -254,15 +266,21 @@ int lsmrc_zf_apply(lsmrc_handle h, const void *d_hzf, const void *d_xd, int n_an
  *      With U = 1 and ZF, W = conj(H) / sum_a |H|^2: MRC.
  *      Device pointers, complex64 unless noted; the handle's compute stream, as lsmrc_demod_frames_device:
  *        d_hconj    [F][U][A][K]        conj(H) per user in the reference layout (bin k+1 at index k); may be NULL
- *        d_combined [F][S-U][U][K]      xhat, ascending frequency
- *        d_bits     [F][S-U][U][row]    hard-demapped xhat, row = lsmrc_bits_row_bytes(N, b); may be NULL
+ *        d_combined [F][S-P][U][K]      xhat, ascending frequency ([F][S-U][U][K] time, [F][S-1][U][K] comb)
+ *        d_bits     [F][S-P][U][row]    hard-demapped xhat, row = lsmrc_bits_row_bytes(N, b); may be NULL
  *        n_singular (host, may be NULL; non-NULL makes the call synchronous): (frame, subcarrier) pairs whose Gram
  *                   matrix was singular.
- *      Any FFT size the handle supports, A <= 256, 1 <= U <= 16, U <= A, U < S.  LSMRC_ERR_INVALID for a bad U, an
- *      unknown detector, or MMSE with a noise_var that is not finite and > 0; LSMRC_ERR_NO_PILOT without a pilot.
+ *      Any FFT size the handle supports, A <= 256, 1 <= U <= 16, U <= A; time pilots need U < S, comb pilots S >= 2
+ *      (U >= S is valid there, e.g. 16 users in 14 symbols).  LSMRC_ERR_INVALID for a bad U or S, an unknown
+ *      detector, or MMSE with a noise_var that is not finite and > 0; LSMRC_ERR_NO_PILOT without a pilot.
  *      Nothing is mirrored on the host: with n_singular == NULL the call can be captured into a CUDA graph after one
  *      ordinary call of the same size (which allocates its scratch). */
 enum { LSMRC_DETECT_ZF = 0, LSMRC_DETECT_MMSE = 1 };
+enum { LSMRC_MU_PILOTS_TIME = 0, LSMRC_MU_PILOTS_COMB = 1 };
+/* pilot layout of lsmrc_demod_frames_device_mu and _mu_soft on this handle: LSMRC_MU_PILOTS_TIME (the default) or
+ * LSMRC_MU_PILOTS_COMB; any other value is LSMRC_ERR_INVALID.  A call reads it when it is enqueued, so a captured
+ * CUDA graph keeps the layout it was captured with. */
+int lsmrc_set_mu_pilots(lsmrc_handle h, int layout);
 int lsmrc_demod_frames_device_mu(lsmrc_handle h, const void *d_rx, int n_frames, int n_users, int detector,
                                  float noise_var, void *d_hconj, void *d_combined, void *d_bits, int *n_singular);
 
@@ -275,7 +293,8 @@ int lsmrc_demod_frames_device_mu(lsmrc_handle h, const void *d_rx, int n_frames,
  *      rho is the post-detection SINR of user u on subcarrier k; the LLRs are those of lsmrc_demod_frames_device_soft
  *      with sum|H|^2 / noise_var replaced by rho.  A singular subcarrier gets rho = 0 and all-zero LLRs.  With U = 1
  *      both detectors give lsmrc_demod_frames_device_soft's LLRs for the same noise_var.
- *        d_llr      [F][S-U][U][K][b] float, ascending frequency, bit order of the packed bits, LLR > 0 <=> bit 0
+ *        d_llr      [F][S-P][U][K][b] float, ascending frequency, bit order of the packed bits, LLR > 0 <=> bit 0
+ *                   (P pilot symbols: [F][S-U][U][K][b] with time pilots, [F][S-1][U][K][b] with comb pilots)
  *        d_sinr     [F][U][K] float, ascending frequency: rho; may be NULL
  *      Every other argument keeps its meaning and layout from lsmrc_demod_frames_device_mu, and d_combined and d_bits
  *      are byte-identical to what that call writes for the same input.  For MMSE they therefore stay the biased xhat:
