@@ -148,9 +148,10 @@ def _run_gpu(ofdm, r, rx, F, U, b, detector="zf", noise_var=0.0, want_hconj=True
     K = N - 1
     dev = torch.device("cuda:0")
     d_rx = torch.from_numpy(np.ascontiguousarray(rx)).to(dev) if isinstance(rx, np.ndarray) else rx
-    comb = torch.zeros((F, S - U, U, K), dtype=torch.complex64, device=dev)
-    bits = torch.zeros((F, S - U, U, (K * b + 7) // 8), dtype=torch.uint8, device=dev)
-    hc = torch.zeros((F, U, A, K), dtype=torch.complex64, device=dev) if want_hconj else None
+    nan = float("nan")                      # every output element is written: nothing may be left as filled
+    comb = torch.view_as_complex(torch.full((F, S - U, U, K, 2), nan, device=dev))
+    bits = torch.full((F, S - U, U, (K * b + 7) // 8), 0xA5, dtype=torch.uint8, device=dev)
+    hc = torch.view_as_complex(torch.full((F, U, A, K, 2), nan, device=dev)) if want_hconj else None
     torch.cuda.synchronize()
     bad = r.demod_frames_device_mu(d_rx, F, U, comb, bits, hc, detector=detector, noise_var=noise_var, count_singular=count)
     r.sync()

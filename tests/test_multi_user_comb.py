@@ -1,122 +1,14 @@
 """Multi-user uplink with comb pilots (lsmrc_set_mu_pilots(h, LSMRC_MU_PILOTS_COMB), DESIGN.md 8h): all users send
 their pilot in symbol 0, user u on the ascending-frequency indices i = u mod U, and the receiver interpolates each
-user's channel across its own comb.  comb_ref restates the whole chain in float64 numpy -- CP strip, np.fft.fft, LS on
+user's channel across its own comb.  comb_ref (mu_ref64.py) restates the whole chain in float64 numpy -- CP strip, np.fft.fft, LS on
 symbol 0, the interpolation rule, np.linalg.solve per subcarrier, hard decisions -- independently of the library and of
 the C oracles.  The CPU tests pin the rule and the generator and measure the interpolation error of the multipath
 settings the GPU tests decode; the GPU tests hold the library to comb_ref on every plan."""
 import numpy as np
 import pytest
 
+from mu_ref64 import _synth, comb_ref, demap, interp_comb, phi, soft_ref
 from util import assert_bits_match, assert_close
-
-SINGULAR_COND = 1e8  # a Gram matrix this badly conditioned in float64 is singular (the tests make such ones exactly)
-A_EXACT = {2: 1 / np.sqrt(2.0), 4: 1 / np.sqrt(10.0), 6: 1 / np.sqrt(42.0)}
-
-
-def _synth():
-    from gpu_accel_ofdm_ls_mrc_b200 import synth
-
-    return synth
-
-
-def phi(i, N):
-    """signed frequency of ascending index i (DC skipped)"""
-    i = np.asarray(i)
-    return np.where(i < N // 2, i - N // 2, i - N // 2 + 1)
-
-
-def interp_comb(ls_asc, U, N):
-    """The comb rule on ascending-frequency LS values ls_asc [..., K] (float64): [..., U, K], user u copied on its own
-    pilots i = u mod U, linear in phi between its two nearest pilots, the nearest pilot held beyond its outermost ones."""
-    ls_asc = np.asarray(ls_asc).astype(np.complex128)
-    K = ls_asc.shape[-1]
-    i = np.arange(K)
-    ph = phi(i, N).astype(np.float64)
-    out = np.empty(ls_asc.shape[:-1] + (U, K), np.complex128)
-    for u in range(U):
-        own = np.arange(u, K, U)
-        j = np.clip(np.searchsorted(own, i, side="right") - 1, 0, len(own) - 1)
-        p0 = own[j]
-        p1 = own[np.minimum(j + 1, len(own) - 1)]
-        inside = (i > p0) & (p1 > p0)
-        w = np.where(inside, (ph - ph[p0]) / np.where(inside, ph[p1] - ph[p0], 1.0), 0.0)
-        a, b = ls_asc[..., p0], ls_asc[..., p1]
-        out[..., u, :] = np.where(inside, a + w * (b - a), a)
-    return out
-
-
-def demap(y, b):
-    """nearest constellation point of the Gray-mapped QAM (synth.qam_map_indices) per axis -> symbol index"""
-    synth = _synth()
-    pts = synth.qam_map_indices(np.arange(1 << b), b)
-    lv = np.unique(np.round(pts.real, 12))
-    m = len(lv)
-    table = np.zeros((m, m), np.uint8)
-    table[np.searchsorted(lv, np.round(pts.real, 12)), np.searchsorted(lv, np.round(pts.imag, 12))] = np.arange(1 << b)
-    step = lv[1] - lv[0]
-    ri = np.clip(np.rint((y.real - lv[0]) / step), 0, m - 1).astype(np.int64)
-    ii = np.clip(np.rint((y.imag - lv[0]) / step), 0, m - 1).astype(np.int64)
-    return table[ri, ii]
-
-
-def comb_ref(rx, pilot_asc, C, U, lam, b=None):
-    """rx [F,S,A,N+C] comb frames -> dict(hconj [F,U,A,K] conj(H) bin order, combined [F,S-1,U,K] ascending frequency,
-    bits [F,S-1,U,row] (with b), ginv_diag [F,U,K] bin order, singular [F,K] bin order, gram_cond (over the regular
-    subcarriers)).  Singular subcarriers (cond > SINGULAR_COND) get W = 0."""
-    synth = _synth()
-    rx = np.asarray(rx)
-    N = rx.shape[-1] - C
-    z = np.fft.fft(rx[..., C:].astype(np.complex128), axis=-1)[..., 1:]          # [F,S,A,K] bin order
-    x_bin = synth.asc_to_bin(np.asarray(pilot_asc).astype(np.complex128))
-    ls = np.conj(z[:, 0] / x_bin)                                                # [F,A,K] as the pilot kernel exports it
-    hc = interp_comb(synth.bin_to_asc(ls), U, N)                                 # [F,A,U,K] ascending
-    hconj = synth.asc_to_bin(hc).transpose(0, 2, 1, 3)                           # [F,U,A,K] bin order
-    H = np.conj(hconj).transpose(0, 3, 2, 1)                                     # [F,K,A,U]
-    Hh = np.conj(np.swapaxes(H, -1, -2))
-    G = Hh @ H + lam * np.eye(U)
-    cond = np.linalg.cond(G)
-    singular = cond > SINGULAR_COND
-    Gs = np.where(singular[..., None, None], np.eye(U), G)
-    W = np.where(singular[..., None, None], 0.0, np.linalg.solve(Gs, Hh))        # [F,K,U,A]
-    M = np.where(singular[..., None, None], 0.0, np.linalg.inv(Gs))
-    x = (W @ z[:, 1:].transpose(0, 3, 2, 1)).transpose(0, 3, 2, 1)               # [F,S-1,U,K] bin order
-    out = {"hconj": hconj, "combined": synth.bin_to_asc(x), "singular": singular, "n_singular": int(singular.sum()),
-           "ginv_diag": np.diagonal(M, axis1=-2, axis2=-1).real.transpose(0, 2, 1),
-           "gram_cond": float(np.where(singular, 1.0, cond).max())}
-    if b is not None:
-        out["bits"] = synth.pack_bits_rows(demap(out["combined"], b), b)
-    return out
-
-
-def soft64(y, rho, b):
-    """max-log piecewise-linear LLRs (soft_symbol in csrc/lsmrc_kernels.cuh) in float64, exact constants: [..., K, b]"""
-    a = A_EXACT[b]
-    g = 4 * a * np.asarray(rho, np.float64)
-    re, im = y.real, y.imag
-    out = [g * re, g * im]
-    if b == 4:
-        out += [g * (2 * a - np.abs(re)), g * (2 * a - np.abs(im))]
-    elif b == 6:
-        out += [g * (4 * a - np.abs(re)), g * (4 * a - np.abs(im)),
-                g * (2 * a - np.abs(np.abs(re) - 4 * a)), g * (2 * a - np.abs(np.abs(im) - 4 * a))]
-    return np.stack(out, axis=-1)
-
-
-def soft_ref(ref, detector, noise_var, b):
-    """DESIGN.md 8f on comb_ref's interpolated H: sinr [F,U,K] and llr [F,S-1,U,K,b], ascending frequency"""
-    synth = _synth()
-    d = ref["ginv_diag"]
-    with np.errstate(divide="ignore", invalid="ignore"):
-        if detector == "mmse":
-            rho = np.where(d > 0, 1.0 / (noise_var * d) - 1.0, 0.0)
-            scale = np.where(rho > 0, 1.0 / (1.0 - noise_var * d), 0.0)
-            rho = np.maximum(rho, 0.0)
-        else:
-            rho = np.where(d > 0, 1.0 / (noise_var * d), 0.0)
-            scale = np.where(d > 0, 1.0, 0.0)
-    rho, scale = synth.bin_to_asc(rho), synth.bin_to_asc(scale)
-    y = ref["combined"] * scale[:, None]
-    return {"sinr": rho, "llr": soft64(y, rho[:, None, :, :], b)}
 
 
 def noise_var_of(snr_db, N):
@@ -304,11 +196,12 @@ def _run(r, rx, F, U, b, detector="zf", noise_var=0.0, soft=False, count=False, 
     A, N, S = r.cfg.n_ant, r.cfg.fft_size, r.cfg.n_sym
     K, D = N - 1, S - P
     dev = _dev()
-    comb = torch.zeros((F, D, U, K), dtype=torch.complex64, device=dev)
-    bits = torch.zeros((F, D, U, (K * b + 7) // 8), dtype=torch.uint8, device=dev)
-    hc = torch.zeros((F, U, A, K), dtype=torch.complex64, device=dev)
-    llr = torch.zeros((F, D, U, K, b), dtype=torch.float32, device=dev) if soft else None
-    sinr = torch.zeros((F, U, K), dtype=torch.float32, device=dev) if soft else None
+    nan = float("nan")                      # every output element is written: nothing may be left as filled
+    comb = torch.view_as_complex(torch.full((F, D, U, K, 2), nan, device=dev))
+    bits = torch.full((F, D, U, (K * b + 7) // 8), 0xA5, dtype=torch.uint8, device=dev)
+    hc = torch.view_as_complex(torch.full((F, U, A, K, 2), nan, device=dev))
+    llr = torch.full((F, D, U, K, b), nan, device=dev) if soft else None
+    sinr = torch.full((F, U, K), nan, device=dev) if soft else None
     d_rx = _to_dev(rx)
     torch.cuda.synchronize()
     if soft:

@@ -204,11 +204,12 @@ def _run_soft(ofdm, r, rx, F, U, b, detector, noise_var, want_hconj=True, want_s
     K = N - 1
     dev = torch.device("cuda:0")
     d_rx = torch.from_numpy(np.ascontiguousarray(rx)).to(dev) if isinstance(rx, np.ndarray) else rx
-    comb = torch.zeros((F, S - U, U, K), dtype=torch.complex64, device=dev)
-    bits = torch.zeros((F, S - U, U, (K * b + 7) // 8), dtype=torch.uint8, device=dev)
-    llr = torch.zeros((F, S - U, U, K, b), dtype=torch.float32, device=dev)
-    sinr = torch.zeros((F, U, K), dtype=torch.float32, device=dev) if want_sinr else None
-    hc = torch.zeros((F, U, A, K), dtype=torch.complex64, device=dev) if want_hconj else None
+    nan = float("nan")                      # every output element is written: nothing may be left as filled
+    comb = torch.view_as_complex(torch.full((F, S - U, U, K, 2), nan, device=dev))
+    bits = torch.full((F, S - U, U, (K * b + 7) // 8), 0xA5, dtype=torch.uint8, device=dev)
+    llr = torch.full((F, S - U, U, K, b), nan, device=dev)
+    sinr = torch.full((F, U, K), nan, device=dev) if want_sinr else None
+    hc = torch.view_as_complex(torch.full((F, U, A, K, 2), nan, device=dev)) if want_hconj else None
     torch.cuda.synchronize()
     bad = r.demod_frames_device_mu_soft(d_rx, F, U, comb, llr, bits, hc, sinr, detector=detector, noise_var=noise_var,
                                         count_singular=count)
@@ -225,8 +226,8 @@ def _run_hard(ofdm, r, rx, F, U, b, detector, noise_var):
     K = N - 1
     dev = torch.device("cuda:0")
     d_rx = torch.from_numpy(np.ascontiguousarray(rx)).to(dev) if isinstance(rx, np.ndarray) else rx
-    comb = torch.zeros((F, S - U, U, K), dtype=torch.complex64, device=dev)
-    bits = torch.zeros((F, S - U, U, (K * b + 7) // 8), dtype=torch.uint8, device=dev)
+    comb = torch.view_as_complex(torch.full((F, S - U, U, K, 2), float("nan"), device=dev))
+    bits = torch.full((F, S - U, U, (K * b + 7) // 8), 0xA5, dtype=torch.uint8, device=dev)
     torch.cuda.synchronize()
     r.demod_frames_device_mu(d_rx, F, U, comb, bits, detector=detector, noise_var=noise_var)
     r.sync()

@@ -38,7 +38,9 @@ def test_oracle_flags_singular_subcarriers(oracle):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("U,A,K", [(1, 1, 7), (2, 4, 63), (4, 64, 1023), (8, 32, 100), (16, 16, 31), (4, 256, 4095)])
+@pytest.mark.parametrize("U,A,K", [(1, 1, 7), (2, 4, 63), (4, 64, 1023), (8, 32, 100), (16, 16, 31), (4, 256, 4095),
+                                   (3, 8, 63), (5, 16, 255), (7, 32, 100), (9, 24, 1023),
+                                   (15, 256, 4095)])   # (15 users on 256 antennas: 4 subcarriers per CTA, the last CTA 3)
 def test_gpu_zero_forcing_matches_oracle(ofdm, oracle, U, A, K):
     import torch
 
